@@ -3,6 +3,9 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU algorithm (oracle port), host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + the outputs of the last timed step, DIR/<name>.npy
+
+Exactly K steps are timed (one block, CUDA events); W >= 3 untimed steps come first.
 
 One JSON line on stdout (rank 0).  metric/unit/config follow BASELINE.json:
   value      = propagated edges/s of the training step (steps * 2 * E / time), inputs resident in HBM,
@@ -57,6 +60,31 @@ def make_data(workload):
     u, i = hostdata.synth_bipartite(U, I, E, 0)
     (tu, ti), (su, si) = hostdata.split_per_user(u, i, U, 1)
     return U, I, u, i, tu, ti, su, si
+
+
+DUMP_ROWS = 65536       # --dump-outputs: larger arrays are cut to this many rows, so that the largest shapes stay under 64 MB
+
+
+def write_dump(out_dir, arrays):
+    """arrays: name -> numpy array, written as out_dir/<name>.npy in float32 (float64 for float64 and integer input, which holds
+    ids exactly).  An array with more than DUMP_ROWS rows is cut to a fixed, seeded sample of rows (sorted), whose indices are
+    written as <name>.rows.npy: the sample depends on the shape alone, so two runs with the same arguments store the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if a.ndim and a.shape[0] > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_ROWS, replace=False))
+            out[name + ".rows"] = rows.astype(np.float64)
+            a = a[rows]
+        out[name] = a
+    total = sum(a.nbytes for a in out.values())
+    if total > 64 * 2 ** 20:
+        raise SystemExit("--dump-outputs: %d bytes exceed the 64 MB budget" % total)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log("[bench] wrote %d arrays (%.1f MB) to %s" % (len(out), total / 2 ** 20, out_dir))
 
 
 def peaks():
@@ -189,7 +217,14 @@ def main():
     ap.add_argument("--dist", default="shard", choices=["replica", "shard"],
                     help="N>1: 'shard' = users range-partitioned, item rows all-gathered / reduce-scattered per stage (north star, strong "
                          "scaling); 'replica' = the reference's --parallel semantics (every GPU propagates the whole graph, weak scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (its loss and the updated parameters) and the last evaluation's "
+                         "results to DIR/<name>.npy, to compare two builds output for output (single GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.profile_only):
+        ap.error("--dump-outputs needs the timed run of this repo's CUDA path (--impl ours, no --profile-only)")
     # exactly ONE JSON line may reach stdout: anything native libraries print to fd 1 (e.g. NCCL's version banner) is
     # diverted to stderr; the JSON line is written to the saved descriptor at the end
     global _STDOUT
@@ -209,6 +244,8 @@ def main():
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs is a single-GPU option")
         dist.init_process_group("nccl", device_id=dev)
     from ngacf_b200 import _lib, roofline
     from ngacf_b200.data import Interactions
@@ -286,39 +323,37 @@ def main():
 
     clocks = ClockSampler(local) if rank == 0 else None
 
-    def timed_blocks(run_block, min_total_ms=500.0, max_blocks=64):
-        """K-step blocks, each bracketed by barrier + synchronize and timed with CUDA events (max over ranks), repeated until the
-        timed region adds up to >= 0.5 s (a single 100-step block is ~80 ms: too short for the clock sampler and for a stable
-        number); the reported time is the MEDIAN block."""
-        times = []
+    def timed_block(run_block):
+        """One block of exactly K steps (--steps), bracketed by barrier + synchronize and timed with CUDA events (max over ranks).
+        A block of ~0.1 s is noisier than a longer one: raise --steps for a steadier number."""
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        while True:
-            barrier()
-            e0.record()
-            run_block()
-            e1.record()
-            barrier()
-            ms = e0.elapsed_time(e1)
-            if world > 1:
-                t = torch.tensor([ms], device=dev)
-                dist.all_reduce(t, op=dist.ReduceOp.MAX)
-                ms = float(t.item())
-            times.append(ms)
-            if sum(times) >= min_total_ms or len(times) >= max_blocks:
-                return times
+        barrier()
+        e0.record()
+        run_block()
+        e1.record()
+        barrier()
+        ms = e0.elapsed_time(e1)
+        if world > 1:
+            t = torch.tensor([ms], device=dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            ms = float(t.item())
+        return ms
 
     # ---------------- device-resident timed region ----------------
     trainer.run_steps(W)
-    blocks = timed_blocks(lambda: trainer.run_steps(K))
-    ms_step = float(np.median(blocks)) / K
+    ms_block = timed_block(lambda: trainer.run_steps(K))
+    ms_step = ms_block / K
     units_per_step = trainer.units_per_step()          # propagated edges per step, all ranks
     value = units_per_step / (ms_step / 1000.0)
+    if args.dump_outputs:
+        # what the caller of the timed step holds after its last step: that step's loss and the updated parameters
+        dumped = {"train_loss": trainer.loss.detach().reshape(1).cpu().numpy()}
+        dumped.update({"param." + k: v.detach().cpu().numpy() for k, v in model.state_dict().items()})
 
     # ---------------- e2e: host rows in, loss out, every step ----------------
     rows_host = torch.from_numpy(np.ascontiguousarray(tu.astype(np.int32))).pin_memory()
     trainer.run_steps(2, host_rows=rows_host, read_loss=True)
-    blocks_e2e = timed_blocks(lambda: trainer.run_steps(K, host_rows=rows_host, read_loss=True))
-    ms_e2e = float(np.median(blocks_e2e))
+    ms_e2e = timed_block(lambda: trainer.run_steps(K, host_rows=rows_host, read_loss=True))
     e2e_value = units_per_step / (ms_e2e / K / 1000.0)
     clk = clocks.stop() if clocks else {}
 
@@ -332,8 +367,8 @@ def main():
             tr_f = FusedTrainer(model_f, inter, graph, B, FusedAdam(model_f.parameters(), lr=HYPER["lr"], weight_decay=HYPER["weight_decay"]),
                                 sample_seed=0, split_dense_backward=args.split_bwd)
             tr_f.run_steps(W)
-            bf = timed_blocks(lambda: tr_f.run_steps(K))
-            full_prop = dict(ms_per_step=float(np.median(bf)) / K, value=units_per_step / (float(np.median(bf)) / K / 1000.0), unit="edges/s",
+            bf = timed_block(lambda: tr_f.run_steps(K))
+            full_prop = dict(ms_per_step=bf / K, value=units_per_step / (bf / K / 1000.0), unit="edges/s",
                              note="NGACF_PRUNE=0: the output stage is computed for every row, as the reference does (results identical up to "
                                   "the order of additions, tests/test_gpu_parity.py::test_pruned_last_stage_equals_full)")
             del tr_f, model_f
@@ -434,6 +469,8 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         ms_eval = e0.elapsed_time(e1) / 5
+        if args.dump_outputs:
+            dumped.update(eval_hr=np.array([hr], np.float64), eval_ndcg=np.array([nd], np.float64))
         ev_out = dict(metric="sampledneg_eval_rows_per_s", value=inter.n_test_rows / (ms_eval / 1000.0), unit="rows/s", ms=ms_eval,
                       rows=inter.n_test_rows, candidates_per_row=100, hr_at_10=hr, ndcg_at_10=nd,
                       e2e=dict(value=inter.n_test_rows / (ms_eval / 1000.0), unit="rows/s", d2h_bytes=16))
@@ -465,10 +502,13 @@ def main():
         ms_eval = e0.elapsed_time(e1) / reps
         e0.record()
         for _ in range(reps):
-            res, _ = eval_once(True)
+            res, top_ids = eval_once(True)
         e1.record()
         barrier()
         ms_eval_e2e = e0.elapsed_time(e1) / reps
+        if args.dump_outputs:
+            dumped.update({"eval_" + k: np.asarray(res[k], np.float64) for k in ("precision", "recall", "ndcg", "hit_ratio")})
+            dumped["eval_top_ids"] = top_ids.numpy().astype(np.float64)
         fl = roofline.eval_flops(n_eval, I)
         # live duration of the scoring entry point alone (prep + tcgen05 kernel + exact re-score), CUDA events
         _lib.PROFILE = []
@@ -503,10 +543,11 @@ def main():
                    sample="%d full %s-shape %s training steps of the oracle port (closed form, torch CPU), 1 warm-up; %.2f s/step"
                           % (len(times), args.workload, "NegSampling" if args.train_mode == "neg" else "PairSampling", cpu_ms / 1000.0))
 
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, dumped)
     if rank == 0:
         line = dict(metric="spuigacf_train_propagated_edges_per_s", value=value, unit="edges/s", n_gpus=world, steps=K, warmup=W,
-                    ms_per_step=ms_step, timed_blocks=dict(n=len(blocks), steps_each=K, ms_per_step_min=min(blocks) / K, ms_per_step_max=max(blocks) / K,
-                                                          total_ms=sum(blocks), statistic="median block"),
+                    ms_per_step=ms_step, timed_ms=ms_block,
                     higher_is_better=True, scaling="strong" if (world > 1 and args.dist == "shard") else "weak",
                     vs_baseline=None, dtype="f32",
                     data="synthetic",
