@@ -13,7 +13,8 @@
  *     call, still async, and reports its data-dependent sizes through a device counter array);
  *   - `stream` is a cudaStream_t passed as void*;
  *   - return value: NGACF_OK or a negative NGACF_ERR_* code; ngacf_last_error() gives the text;
- *   - all float tensors are fp32 row-major with 64 columns (embedSize 64 of every BASELINE config);
+ *   - all float tensors are fp32 row-major with 64 columns (embedSize 64 of every BASELINE config); the `_w` variants at the
+ *     end take other row widths (embedSize 128);
  *   - node numbering: users 0..U-1 then items U..U+I-1 ("features" layout of SPUIGACF.py:38);
  *   - H = heads of a stage: 8 (eight 64->8 heads, SPUIGACF.py:191-198) or 1 (out_att 64->64, :200-205).
  */
@@ -343,6 +344,53 @@ int ngacf_spgat_bwd(const int32_t* tasks, int32_t T, const int32_t* adj_ptr, con
                     const float* norm, const float* h, const float* p, const float* q, int32_t H, const uint8_t* emask, float scale,
                     int32_t self_loops, int32_t n_adj, const float* const* wtab, float* Ghat, float* pairs, float* dP, float* dQ,
                     float* dh, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Row widths other than 64 (embedSize 128).  Every entry point above is the 64-wide case and keeps its signature; the `_w`
+ * variants carry the widths.  Width 64 in a `_w` call reaches exactly the kernels of the unsuffixed call (tensor-core dense
+ * transforms and NGACF_DENSE included).  The SPUIGACF stage shapes at embedSize d = 128: the first stage (8 heads) reads d-wide
+ * rows and writes 64, a middle stage (SPUIMultiGACF) is 64 -> 64, the last stage (1 head) writes d-wide rows; the scores read
+ * d-wide rows.  Built: width 128 for single-head rows, the dense shapes (H, d_in, d_out) = (8, 128, 64) and (1, 64, 128) (CUDA-core
+ * kernels), the 128-wide scores and the exact AllNeg top-K.  Anything else returns NGACF_ERR_UNSUPPORTED with a message (not
+ * built at 128: partial-row multi-GPU calls, the pruned output stage, the tcgen05 dense kernels and AllNeg scorer).
+ * Buffer sizes at width w: rows (N, w) fp32; feature masks w/64 uint64 words per row (word j = columns 64j .. 64j+63; row n draws
+ * Philox counters n*(w/8) + c, c = 0 .. w/8-1, eight columns each); long-row scratch S*(w+8) floats.
+ * ------------------------------------------------------------------------------------------- */
+/* widths: HOST array of S per-stage INPUT widths (NULL = all 64) */
+int ngacf_dropout_masks_w(uint64_t* const* feat, uint8_t* const* edge, const int32_t* heads, const int32_t* widths, int32_t S, int64_t N,
+                          int64_t E, uint64_t seed, uint32_t call, const int64_t* call_dev, float droprate, void* stream);
+int ngacf_transform_fwd_w(const float* Xu, const float* Xi, int32_t apply_elu, const uint64_t* featmask, float scale,
+                          const float* const* wtab, int32_t H, int32_t d_in, int32_t d_out, int32_t U, int32_t I, float* h, float* s,
+                          void* stream);
+/* workspace of ngacf_transform_bwd_w for that shape (one d_in*d_out + d_out float partial per block); 0 for a shape that is not built */
+size_t ngacf_transform_bwd_workspace_bytes_w(int32_t d_in, int32_t d_out, int32_t U, int32_t I);
+int ngacf_transform_bwd_w(const float* dh, const float* dS, const float* h, const float* Xu, const float* Xi, int32_t apply_elu,
+                          const uint64_t* featmask, float scale, const float* const* wtab, float* const* gtab, int32_t H, int32_t d_in,
+                          int32_t d_out, int32_t U, int32_t I, float* dXu, float* dXi, int32_t accumulate_dx, int32_t accumulate_dw,
+                          void* workspace, size_t workspace_bytes, void* stream);
+int ngacf_aggregate_fwd_w(const int32_t* tasks, int32_t T, const int32_t* adj_ptr, const int32_t* adj_idx, const int32_t* adj_eid,
+                          const int32_t* long_first_slot, int32_t* long_counter, float* scratch, const float* h, const float* s, int32_t H,
+                          int32_t width, const uint8_t* edgemask, float scale, float* Z, float* norm, int32_t partial_from, void* stream);
+int ngacf_stage_bwd_prep_w(const float* G, const float* Z, const float* h, const float* norm, int32_t H, int32_t width, int64_t N,
+                           float* Ghat, float* dN, void* stream);
+int ngacf_stage_bwd_edges_w(int32_t mode, const int32_t* tasks, int32_t T_begin, int32_t T_end, const int32_t* adj_ptr,
+                            const int32_t* adj_idx, const int32_t* adj_eid, const int32_t* long_first_slot, int32_t* long_counter,
+                            float* scratch, const float* G, const float* Ghat, const float* dN, const float* h, const float* s, int32_t H,
+                            int32_t width, const uint8_t* edgemask, float scale, const float* const* wtab, int32_t U, float* ds_store,
+                            float* dh, float* dS, int32_t partial, void* stream);
+int ngacf_score_pairs_w(const float* Z, int32_t width, int32_t U, const int64_t* users, const int64_t* items, int32_t B, float* scores,
+                        void* stream);
+int ngacf_score_pairs_bwd_w(const float* Z, int32_t width, int32_t U, const int64_t* users, const int64_t* items, const float* dscore,
+                            int32_t B, float* G, int32_t accumulate, void* stream);
+int ngacf_final_features_w(const float* Z, int64_t N, int32_t width, float* F, void* stream);
+/* scores of 128-wide rows: the same adjacent-pair tree over 128 products (7 levels); the split variant uses the workspace size of
+ * ngacf_score_topk_exact_split_workspace_bytes */
+int ngacf_score_topk_exact_w(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users,
+                             const int32_t* train_ptr, const int32_t* train_items, const uint8_t* in_pool, int32_t* top_ids,
+                             float* top_scores, void* stream);
+int ngacf_score_topk_exact_split_w(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users,
+                                   const int32_t* train_ptr, const int32_t* train_items, const uint8_t* in_pool, int32_t* top_ids,
+                                   float* top_scores, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -68,6 +68,21 @@ SIGNATURES = {
     "ngacf_score_topk_tc": (c_int32, [P, c_int32, c_int32, P, c_int32, P, P, P, P, P, P, c_int32, P, c_size_t, P]),
     "ngacf_eval_metrics_workspace_bytes": (c_size_t, [c_int32]),
     "ngacf_eval_metrics": (c_int32, [P, P, c_int32, P, P, P, P, P, c_size_t, P]),
+    # width-carrying variants (embedSize 128)
+    "ngacf_dropout_masks_w": (c_int32, [P, P, P, P, c_int32, c_int64, c_int64, c_uint64, c_uint32, P, c_float, P]),
+    "ngacf_transform_fwd_w": (c_int32, [P, P, c_int32, P, c_float, P, c_int32, c_int32, c_int32, c_int32, c_int32, P, P, P]),
+    "ngacf_transform_bwd_workspace_bytes_w": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "ngacf_transform_bwd_w": (c_int32, [P, P, P, P, P, c_int32, P, c_float, P, P, c_int32, c_int32, c_int32, c_int32, c_int32, P, P, c_int32,
+                                        c_int32, P, c_size_t, P]),
+    "ngacf_aggregate_fwd_w": (c_int32, [P, c_int32, P, P, P, P, P, P, P, P, c_int32, c_int32, P, c_float, P, P, c_int32, P]),
+    "ngacf_stage_bwd_prep_w": (c_int32, [P, P, P, P, c_int32, c_int32, c_int64, P, P, P]),
+    "ngacf_stage_bwd_edges_w": (c_int32, [c_int32, P, c_int32, c_int32, P, P, P, P, P, P, P, P, P, P, P, c_int32, c_int32, P, c_float, P,
+                                          c_int32, P, P, P, c_int32, P]),
+    "ngacf_score_pairs_w": (c_int32, [P, c_int32, c_int32, P, P, c_int32, P, P]),
+    "ngacf_score_pairs_bwd_w": (c_int32, [P, c_int32, c_int32, P, P, P, c_int32, P, c_int32, P]),
+    "ngacf_final_features_w": (c_int32, [P, c_int64, c_int32, P, P]),
+    "ngacf_score_topk_exact_w": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, P, P, P, P, P, P]),
+    "ngacf_score_topk_exact_split_w": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, P, P, P, P, P, P, c_size_t, P]),
 }
 
 _lib = None

@@ -250,6 +250,57 @@ __device__ __forceinline__ bool long_row_combine(int lid, int chunk, const int* 
     return true;
 }
 
+// the same hand-over for W-wide single-head rows (W = 128: lane l owns columns W/16*l .. W/16*(l+1)-1, V float4 each); the slot
+// stride is W + 8 floats.  The 64-wide kernels keep long_row_combine above.
+template <int W, int NSUM>
+__device__ __forceinline__ bool long_row_combine_wide(int lid, int chunk, const int* __restrict__ long_first_slot, int* long_counter,
+                                                      float* scratch, int lane16, unsigned gm, float4 (&acc)[W / 64], float (&sums)[NSUM]) {
+    constexpr int V = W / 64, STRIDE = W + 8;
+    static_assert(NSUM <= 8, "per-slot room for 8 scalars");
+    const int first = long_first_slot[lid];
+    const int nslots = long_first_slot[lid + 1] - first;
+    float* slot = scratch + (size_t)(first + chunk) * STRIDE;
+#pragma unroll
+    for (int v = 0; v < V; ++v) *reinterpret_cast<float4*>(slot + lane16 * 4 * V + 4 * v) = acc[v];
+    if (lane16 == 0) {
+#pragma unroll
+        for (int j = 0; j < NSUM; ++j) slot[W + j] = sums[j];
+    }
+    fence_acq_rel_gpu();
+    __syncwarp(gm);
+    int old = 0;
+    if (lane16 == 0) old = atomicAdd(long_counter + lid, 1);
+    old = __shfl_sync(gm, old, 0, 16);
+    if (old != nslots - 1) return false;
+    fence_acq_rel_gpu();
+    float4 t[V];
+    float ts[NSUM];
+#pragma unroll
+    for (int v = 0; v < V; ++v) t[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+    for (int j = 0; j < NSUM; ++j) ts[j] = 0.f;
+    for (int c = 0; c < nslots; ++c) {
+        const float* sl = scratch + (size_t)(first + c) * STRIDE;
+#pragma unroll
+        for (int v = 0; v < V; ++v) {
+            const float4 x = ld_cg4(sl + lane16 * 4 * V + 4 * v);
+            t[v].x += x.x; t[v].y += x.y; t[v].z += x.z; t[v].w += x.w;
+        }
+#pragma unroll
+        for (int j = 0; j < NSUM; ++j) ts[j] += __ldcg(sl + W + j);
+    }
+#pragma unroll
+    for (int v = 0; v < V; ++v) acc[v] = t[v];
+#pragma unroll
+    for (int j = 0; j < NSUM; ++j) sums[j] = ts[j];
+    if (lane16 == 0) long_counter[lid] = 0;
+    return true;
+}
+
+// row widths of the width-generic (`_w`) entry points: 64 (every stage of the 64-wide models) and 128 (embedSize 128: the input
+// of the first stage and the output of the single-head last stage)
+static inline bool width_supported(int w) { return w == 64 || w == 128; }
+
 // "active" rows of a pruned last stage (ngacf_mark_active): node n is active iff stamp[n] == value of this propagation
 __device__ __forceinline__ int active_value(int val, const int64_t* __restrict__ val_dev) {
     return val_dev ? val + (int)*val_dev : val;

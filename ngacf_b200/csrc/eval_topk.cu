@@ -12,24 +12,30 @@ constexpr int K = NGACF_TOPK;
 constexpr int EX_USERS = 16;          // users per CTA
 constexpr int EX_ITEMS = 64;          // items per tile
 constexpr int EX_THREADS = 256;       // 16 users x 16 item lanes, 4 items per thread per tile
-constexpr size_t EX_SMEM = (size_t)(64 * EX_ITEMS + EX_USERS * 64) * 4 + (size_t)EX_THREADS * K * 8 + EX_USERS * 8 + EX_ITEMS + 64;
+template <int W> __host__ __device__ constexpr size_t ex_smem() {
+    return (size_t)(W * EX_ITEMS + EX_USERS * W) * 4 + (size_t)EX_THREADS * K * 8 + EX_USERS * 8 + EX_ITEMS + 64;
+}
+constexpr size_t EX_SMEM = ex_smem<64>();
 
 // order: score descending, item id ascending
 __device__ __forceinline__ bool better(float s1, int i1, float s2, int i2) { return s1 > s2 || (s1 == s2 && i1 < i2); }
 
-// 64-term adjacent-pair tree evaluated incrementally: `add(d, v)` with d compile-time after unrolling
-struct Tree64 {
-    float st[6];
+// 2^L-term adjacent-pair tree evaluated incrementally: `add(d, v)` with d compile-time after unrolling (L = 6: 64-wide rows,
+// L = 7: 128-wide rows); the total ends in st[L-1]
+template <int L>
+struct TreeN {
+    float st[L];
     __device__ __forceinline__ void add(int d, float v) {
 #pragma unroll
-        for (int l = 0; l < 6; ++l) {
+        for (int l = 0; l < L; ++l) {
             if (((d >> l) & 1) == 0) { st[l] = v; return; }
             v = __fadd_rn(st[l], v);
         }
-        st[5] = v;   // d == 63: v is the total (kept in st[5])
+        st[L - 1] = v;   // d == 2^L - 1: v is the total (kept in st[L-1])
     }
 };
 
+template <int W = 64>
 __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const float* __restrict__ F, int U, int I, const int* __restrict__ users,
                                                                       int n_users, const int* __restrict__ train_ptr,
                                                                       const int* __restrict__ train_items, const uint8_t* __restrict__ in_pool,
@@ -37,9 +43,10 @@ __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const floa
     // gridDim.y > 1 (few users, ngacf_score_topk_exact_split): CTA (x, y) ranks its 16 users on item slice y only and writes the
     // slice's top-K to row (uslot * gridDim.y + y) of the outputs, which then are partial lists merged by merge_partial_topk_kernel
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    float* It = reinterpret_cast<float*>(smem_raw);                 // [64 d][64 items]
-    float* Us = It + 64 * EX_ITEMS;                                 // [16 users][64]
-    float* Ls = Us + EX_USERS * 64;                                 // [K][256] scores (thread-interleaved)
+    constexpr int L = W == 64 ? 6 : 7;
+    float* It = reinterpret_cast<float*>(smem_raw);                 // [W d][64 items]
+    float* Us = It + W * EX_ITEMS;                                  // [16 users][W]
+    float* Ls = Us + EX_USERS * W;                                  // [K][256] scores (thread-interleaved)
     int* Li = reinterpret_cast<int*>(Ls + EX_THREADS * K);          // [K][256] ids
     unsigned long long* Mk = reinterpret_cast<unsigned long long*>(Li + EX_THREADS * K);   // [16] train-positive bits of the tile
     uint8_t* Pool = reinterpret_cast<uint8_t*>(Mk + EX_USERS);      // [64]
@@ -48,9 +55,9 @@ __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const floa
     const int tid = threadIdx.x, ul = tid >> 4, il = tid & 15;
     const int uslot = blockIdx.x * EX_USERS + ul;
     const int user = uslot < n_users ? users[uslot] : -1;
-    for (int idx = tid; idx < EX_USERS * 64; idx += EX_THREADS) {
-        int us = blockIdx.x * EX_USERS + (idx >> 6);
-        Us[idx] = us < n_users ? F[(int64_t)users[us] * D + (idx & 63)] : 0.f;
+    for (int idx = tid; idx < EX_USERS * W; idx += EX_THREADS) {
+        int us = blockIdx.x * EX_USERS + idx / W;
+        Us[idx] = us < n_users ? F[(int64_t)users[us] * W + (idx % W)] : 0.f;
     }
     for (int k = 0; k < K; ++k) { Ls[k * EX_THREADS + tid] = -INFINITY; Li[k * EX_THREADS + tid] = -1; }
     const int tiles_all = (I + EX_ITEMS - 1) / EX_ITEMS;
@@ -72,10 +79,10 @@ __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const floa
     for (int i0 = i_begin; i0 < i_end; i0 += EX_ITEMS) {
         __syncthreads();
         // item tile, transposed: It[d][j] = F[U+i0+j][d]
-        for (int idx = tid; idx < EX_ITEMS * 16; idx += EX_THREADS) {
-            int j = idx >> 4, q = idx & 15;
+        for (int idx = tid; idx < EX_ITEMS * (W / 4); idx += EX_THREADS) {
+            int j = idx / (W / 4), q = idx % (W / 4);
             float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (i0 + j < I) v = ld_gather4(F + (int64_t)(U + i0 + j) * D + q * 4);
+            if (i0 + j < I) v = ld_gather4(F + (int64_t)(U + i0 + j) * W + q * 4);
             It[(q * 4 + 0) * EX_ITEMS + j] = v.x; It[(q * 4 + 1) * EX_ITEMS + j] = v.y;
             It[(q * 4 + 2) * EX_ITEMS + j] = v.z; It[(q * 4 + 3) * EX_ITEMS + j] = v.w;
         }
@@ -93,10 +100,10 @@ __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const floa
             Mk[ul] = m;
         }
         __syncthreads();
-        Tree64 t0, t1, t2, t3;
-        const float* up = Us + ul * 64;
+        TreeN<L> t0, t1, t2, t3;
+        const float* up = Us + ul * W;
 #pragma unroll
-        for (int d = 0; d < 64; ++d) {
+        for (int d = 0; d < W; ++d) {
             const float u = up[d];
             const float* row = It + d * EX_ITEMS + il;
             t0.add(d, __fmul_rn(u, row[0]));
@@ -105,7 +112,7 @@ __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const floa
             t3.add(d, __fmul_rn(u, row[48]));
         }
         const unsigned long long mk = Mk[ul];
-        const float sc[4] = {t0.st[5], t1.st[5], t2.st[5], t3.st[5]};
+        const float sc[4] = {t0.st[L - 1], t1.st[L - 1], t2.st[L - 1], t3.st[L - 1]};
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int jj = il + 16 * j;
@@ -273,9 +280,9 @@ extern "C" int ngacf_score_topk_exact(const float* F, int32_t U, int32_t I, cons
     if (n_users == 0) return NGACF_OK;
     static PerDeviceOnce once;
     once.run([] {
-        cudaFuncSetAttribute(score_topk_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EX_SMEM);
+        cudaFuncSetAttribute(score_topk_exact_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EX_SMEM);
     });
-    score_topk_exact_kernel<<<ceil_div(n_users, EX_USERS), EX_THREADS, EX_SMEM, (cudaStream_t)stream>>>(F, U, I, users, n_users, train_ptr,
+    score_topk_exact_kernel<64><<<ceil_div(n_users, EX_USERS), EX_THREADS, EX_SMEM, (cudaStream_t)stream>>>(F, U, I, users, n_users, train_ptr,
                                                                                                          train_items, in_pool, top_ids, top_scores);
     return check_launch("score_topk_exact");
 }
@@ -307,16 +314,61 @@ extern "C" int ngacf_score_topk_exact_split(const float* F, int32_t U, int32_t I
     if (P == 1) return ngacf_score_topk_exact(F, U, I, users, n_users, train_ptr, train_items, in_pool, top_ids, top_scores, stream);
     static PerDeviceOnce once;
     once.run([] {
-        cudaFuncSetAttribute(score_topk_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EX_SMEM);
+        cudaFuncSetAttribute(score_topk_exact_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)EX_SMEM);
     });
     cudaStream_t st = (cudaStream_t)stream;
     char* w = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     int* part_ids = (int*)w;
     float* part_scores = (float*)(w + (size_t)n_users * P * K * 4);
-    score_topk_exact_kernel<<<dim3(ceil_div(n_users, EX_USERS), P), EX_THREADS, EX_SMEM, st>>>(F, U, I, users, n_users, train_ptr, train_items, in_pool,
+    score_topk_exact_kernel<64><<<dim3(ceil_div(n_users, EX_USERS), P), EX_THREADS, EX_SMEM, st>>>(F, U, I, users, n_users, train_ptr, train_items, in_pool,
                                                                                               part_ids, part_scores);
     merge_partial_topk_kernel<<<n_users, 256, 0, st>>>(part_ids, part_scores, n_users, P, top_ids, top_scores);
     return check_launch("score_topk_exact_split");
+}
+
+// width-carrying entry points: width 64 reaches the calls above (the same kernel); 128-wide features run the W = 128 instantiation
+// (seven-level tree, twice the user / item tiles in shared memory)
+static int launch_topk_exact128(const float* F, int U, int I, const int* users, int n_users, const int* train_ptr, const int* train_items,
+                                const uint8_t* in_pool, int* top_ids, float* top_scores, int P, cudaStream_t st) {
+    static PerDeviceOnce once;
+    once.run([] { cudaFuncSetAttribute(score_topk_exact_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ex_smem<128>()); });
+    score_topk_exact_kernel<128><<<dim3(ceil_div(n_users, EX_USERS), P), EX_THREADS, ex_smem<128>(), st>>>(F, U, I, users, n_users, train_ptr,
+                                                                                                           train_items, in_pool, top_ids, top_scores);
+    return check_launch("score_topk_exact_w");
+}
+
+extern "C" int ngacf_score_topk_exact_w(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users,
+                                        const int32_t* train_ptr, const int32_t* train_items, const uint8_t* in_pool, int32_t* top_ids,
+                                        float* top_scores, void* stream) {
+    if (width == 64) return ngacf_score_topk_exact(F, U, I, users, n_users, train_ptr, train_items, in_pool, top_ids, top_scores, stream);
+    if (width != 128) { set_error("score_topk_exact_w: width %d is not built (supported: 64, 128)", width); return NGACF_ERR_UNSUPPORTED; }
+    NGACF_REQUIRE(F && users && train_ptr && train_items && in_pool && top_ids && top_scores && U > 0 && I > 0 && n_users >= 0,
+                  "score_topk_exact_w: null/empty argument");
+    if (n_users == 0) return NGACF_OK;
+    return launch_topk_exact128(F, U, I, users, n_users, train_ptr, train_items, in_pool, top_ids, top_scores, 1, (cudaStream_t)stream);
+}
+
+extern "C" int ngacf_score_topk_exact_split_w(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users,
+                                              const int32_t* train_ptr, const int32_t* train_items, const uint8_t* in_pool, int32_t* top_ids,
+                                              float* top_scores, void* workspace, size_t workspace_bytes, void* stream) {
+    if (width == 64)
+        return ngacf_score_topk_exact_split(F, U, I, users, n_users, train_ptr, train_items, in_pool, top_ids, top_scores, workspace,
+                                            workspace_bytes, stream);
+    if (width != 128) { set_error("score_topk_exact_split_w: width %d is not built (supported: 64, 128)", width); return NGACF_ERR_UNSUPPORTED; }
+    NGACF_REQUIRE(F && users && train_ptr && train_items && in_pool && top_ids && top_scores && workspace && U > 0 && I > 0 && n_users >= 0,
+                  "score_topk_exact_split_w: null/empty argument");
+    if (workspace_bytes < ngacf_score_topk_exact_split_workspace_bytes(I, n_users)) { set_error("score_topk_exact_split_w: workspace too small"); return NGACF_ERR_WORKSPACE; }
+    if (n_users == 0) return NGACF_OK;
+    const int P = exact_split_parts(n_users, I);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (P == 1) return launch_topk_exact128(F, U, I, users, n_users, train_ptr, train_items, in_pool, top_ids, top_scores, 1, st);
+    char* w = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    int* part_ids = (int*)w;
+    float* part_scores = (float*)(w + (size_t)n_users * P * K * 4);
+    const int rc = launch_topk_exact128(F, U, I, users, n_users, train_ptr, train_items, in_pool, part_ids, part_scores, P, st);
+    if (rc != NGACF_OK) return rc;
+    merge_partial_topk_kernel<<<n_users, 256, 0, st>>>(part_ids, part_scores, n_users, P, top_ids, top_scores);
+    return check_launch("score_topk_exact_split_w");
 }
 
 extern "C" size_t ngacf_eval_metrics_workspace_bytes(int32_t n_users) { return (size_t)(n_users > 0 ? n_users : 1) * 16 * sizeof(double); }

@@ -60,6 +60,7 @@ struct MaskPlan {
     uint64_t* feat[MASK_MAX_STAGES];
     uint8_t* edge[MASK_MAX_STAGES];
     int heads[MASK_MAX_STAGES];
+    int wshift[MASK_MAX_STAGES];    // log2(input width / 64): a row has 8 << wshift Philox counters and 1 << wshift words
     int S;
     int feat_blocks, edge_blocks;   // per stage
 };
@@ -73,12 +74,14 @@ __global__ void __launch_bounds__(256) dropout_masks_kernel(MaskPlan plan, int64
     b -= site * per_stage;
     uint32_t w[4];
     if (b < plan.feat_blocks) {
+        // thread t = Philox counter t = (row n, 8-column group c) with t = n * (8 << wshift) + c; word t/8 of the mask holds the
+        // decisions of counters 8*(t/8) .. 8*(t/8)+7 (a 64-wide row: word n, counters 8n .. 8n+7)
         const int64_t t = (int64_t)b * 256 + threadIdx.x;
-        const int64_t n = t >> 3;
+        const bool in = t < (N << (3 + plan.wshift[site]));
         const int c = (int)(t & 7);
         uint32_t bits = 0;
-        if (n < N) {
-            const uint64_t idx = (uint64_t)n * 8u + (uint64_t)c;
+        if (in) {
+            const uint64_t idx = (uint64_t)t;
             philox4x32_10((uint32_t)idx, (uint32_t)(idx >> 32), (uint32_t)site * 2u, call, k0, k1, w);
             bits = decisions8(w, thr);
         }
@@ -86,7 +89,7 @@ __global__ void __launch_bounds__(256) dropout_masks_kernel(MaskPlan plan, int64
         word |= __shfl_xor_sync(0xffffffffu, word, 1);
         word |= __shfl_xor_sync(0xffffffffu, word, 2);
         word |= __shfl_xor_sync(0xffffffffu, word, 4);
-        if (n < N && c == 0) plan.feat[site][n] = word;
+        if (in && c == 0) plan.feat[site][t >> 3] = word;
     } else {
         const int64_t e = (int64_t)(b - plan.feat_blocks) * 256 + threadIdx.x;
         if (e >= E) return;
@@ -134,31 +137,34 @@ __global__ void __launch_bounds__(256) dropout_masks_ranges_kernel(MaskPlan plan
 
 // ------------------------------------------------------------------------------------------------
 // dense transform: h = Xd @ Wcat, s = per-head a . h
-// block = 256 threads, tile = 128 rows of one side; thread = 8 rows x 4 columns
+// block = 256 threads, tile = TF_TM(DOUT) rows of one side; thread = TF_TM/16 rows x 4 columns of every 64-column group.
+// (DIN, DOUT) = (64, 64) for every stage of the 64-wide models; embedSize 128 adds (128, 64) (first stage) and (64, 128) (last).
 // ------------------------------------------------------------------------------------------------
+template <int DOUT> __host__ __device__ constexpr int tf_tm() { return 128 * 64 / DOUT; }          // 8 rows x 4 columns per thread at DOUT = 64
+template <int DIN, int DOUT> __host__ __device__ constexpr size_t tf_smem() { return (size_t)(DIN * DOUT + tf_tm<DOUT>() * (DIN + 4) + DOUT) * sizeof(float); }
 constexpr int TF_TM = 128;
-constexpr int TF_XS = 68;   // padded smem row stride (floats)
-constexpr size_t TF_SMEM = (size_t)(64 * 64 + TF_TM * TF_XS + 64) * sizeof(float);
+constexpr size_t TF_SMEM = tf_smem<64, 64>();
 
-// load the H per-head (64,DH) matrices of one side into Ws[k][c], c = head*DH + j
-__device__ __forceinline__ void load_wcat(float* Ws, const float* const* wptr, int H, bool transpose) {
-    const int DH = D / H;
-    // 16-byte loads: every (64,DH) head matrix is contiguous and DH is a multiple of 4
-    for (int idx = threadIdx.x; idx < 64 * 16; idx += blockDim.x) {
-        const int k = idx >> 4, c = (idx & 15) * 4;
+// load the H per-head (DIN,DH) matrices of one side into Ws[k][c], c = head*DH + j
+template <int DIN, int DOUT>
+__device__ __forceinline__ void load_wcat(float* Ws, const float* const* wptr, int H) {
+    const int DH = DOUT / H;
+    // 16-byte loads: every (DIN,DH) head matrix is contiguous and DH is a multiple of 4
+    for (int idx = threadIdx.x; idx < DIN * DOUT / 4; idx += blockDim.x) {
+        const int k = idx / (DOUT / 4), c = (idx % (DOUT / 4)) * 4;
         const float4 v = __ldg(reinterpret_cast<const float4*>(wptr[c / DH] + k * DH + (c % DH)));
-        if (transpose) { Ws[(c + 0) * 64 + k] = v.x; Ws[(c + 1) * 64 + k] = v.y; Ws[(c + 2) * 64 + k] = v.z; Ws[(c + 3) * 64 + k] = v.w; }
-        else *reinterpret_cast<float4*>(Ws + k * 64 + c) = v;
+        *reinterpret_cast<float4*>(Ws + k * DOUT + c) = v;
     }
 }
 
-// stage-input element: ELU on load for stage > 0, then dropout keep-bit and 1/(1-p)
+// stage-input element: ELU on load for stage > 0, then dropout keep-bit and 1/(1-p); the mask has DIN/64 words per row
+template <int DIN>
 __device__ __forceinline__ float4 load_input4(const float* __restrict__ X, int64_t row, int q, bool apply_elu,
                                               const uint64_t* __restrict__ featmask, int64_t node, float scale) {
-    float4 v = ld_stream4(X + row * D + q * 4);
+    float4 v = ld_stream4(X + row * DIN + q * 4);
     if (apply_elu) { v.x = elu(v.x); v.y = elu(v.y); v.z = elu(v.z); v.w = elu(v.w); }
     if (featmask) {
-        uint32_t m = (uint32_t)(featmask[node] >> (q * 4)) & 0xFu;
+        uint32_t m = (uint32_t)(featmask[node * (DIN / 64) + (q >> 4)] >> ((q & 15) * 4)) & 0xFu;
         v.x = (m & 1u) ? v.x * scale : 0.f;
         v.y = (m & 2u) ? v.y * scale : 0.f;
         v.z = (m & 4u) ? v.z * scale : 0.f;
@@ -167,70 +173,88 @@ __device__ __forceinline__ float4 load_input4(const float* __restrict__ X, int64
     return v;
 }
 
-template <int H>
+template <int H, int DIN, int DOUT>
 __global__ void __launch_bounds__(256, 4) transform_fwd_kernel(const float* __restrict__ Xu, const float* __restrict__ Xi, int apply_elu,
                                                             const uint64_t* __restrict__ featmask, float scale,
                                                             const float* const* __restrict__ wtab, int U, int I, int tiles_u,
                                                             float* __restrict__ h, float* __restrict__ s) {
+    constexpr int TM = tf_tm<DOUT>(), XS = DIN + 4, RI = TM / 16, NC = DOUT / 64;
     extern __shared__ __align__(16) float smem[];
-    float* Ws = smem;                    // [64][64]
-    float* Xs = smem + 64 * 64;          // [128][68]
-    float* av = Xs + TF_TM * TF_XS;      // [64]
-    constexpr int DH = D / H;
+    float* Ws = smem;                    // [DIN][DOUT]
+    float* Xs = smem + DIN * DOUT;       // [TM][DIN+4]
+    float* av = Xs + TM * XS;            // [DOUT]
+    constexpr int DH = DOUT / H;
     const bool item_side = (int)blockIdx.x >= tiles_u;
     const int tile = item_side ? blockIdx.x - tiles_u : blockIdx.x;
     const int rows_side = item_side ? I : U;
     const float* X = item_side ? Xi : Xu;
-    const int64_t node0 = (item_side ? (int64_t)U : 0) + (int64_t)tile * TF_TM;
-    const int row0 = tile * TF_TM;
-    const int nrows = min(TF_TM, rows_side - row0);
+    const int64_t node0 = (item_side ? (int64_t)U : 0) + (int64_t)tile * TM;
+    const int row0 = tile * TM;
+    const int nrows = min(TM, rows_side - row0);
 
-    load_wcat(Ws, wtab + (item_side ? H : 0), H, false);
-    if (threadIdx.x < 64) {
-        int k = threadIdx.x / DH, j = threadIdx.x % DH;
-        av[threadIdx.x] = __ldg(wtab[2 * H + k] + (item_side ? DH : 0) + j);
+    load_wcat<DIN, DOUT>(Ws, wtab + (item_side ? H : 0), H);
+    for (int c = threadIdx.x; c < DOUT; c += 256) {
+        int k = c / DH, j = c % DH;
+        av[c] = __ldg(wtab[2 * H + k] + (item_side ? DH : 0) + j);
     }
-    for (int idx = threadIdx.x; idx < TF_TM * 16; idx += 256) {
-        int r = idx >> 4, q = idx & 15;
+    for (int idx = threadIdx.x; idx < TM * (DIN / 4); idx += 256) {
+        int r = idx / (DIN / 4), q = idx % (DIN / 4);
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (r < nrows) v = load_input4(X, row0 + r, q, apply_elu != 0, featmask, node0 + r, scale);
-        *reinterpret_cast<float4*>(Xs + r * TF_XS + q * 4) = v;
+        if (r < nrows) v = load_input4<DIN>(X, row0 + r, q, apply_elu != 0, featmask, node0 + r, scale);
+        *reinterpret_cast<float4*>(Xs + r * XS + q * 4) = v;
     }
     __syncthreads();
 
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    float acc[8][4];
+    float acc[RI][NC][4];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) { acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.f; }
+    for (int i = 0; i < RI; ++i)
+#pragma unroll
+        for (int n = 0; n < NC; ++n) { acc[i][n][0] = acc[i][n][1] = acc[i][n][2] = acc[i][n][3] = 0.f; }
 #pragma unroll 4
-    for (int k4 = 0; k4 < 16; ++k4) {
-        float4 w0 = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 0) * 64 + tx * 4);
-        float4 w1 = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 1) * 64 + tx * 4);
-        float4 w2 = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 2) * 64 + tx * 4);
-        float4 w3 = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 3) * 64 + tx * 4);
+    for (int k4 = 0; k4 < DIN / 4; ++k4) {
+        float4 w0[NC], w1[NC], w2[NC], w3[NC];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            float4 x = *reinterpret_cast<const float4*>(Xs + (ty + 16 * i) * TF_XS + k4 * 4);
-            acc[i][0] = fmaf(x.x, w0.x, acc[i][0]); acc[i][1] = fmaf(x.x, w0.y, acc[i][1]);
-            acc[i][2] = fmaf(x.x, w0.z, acc[i][2]); acc[i][3] = fmaf(x.x, w0.w, acc[i][3]);
-            acc[i][0] = fmaf(x.y, w1.x, acc[i][0]); acc[i][1] = fmaf(x.y, w1.y, acc[i][1]);
-            acc[i][2] = fmaf(x.y, w1.z, acc[i][2]); acc[i][3] = fmaf(x.y, w1.w, acc[i][3]);
-            acc[i][0] = fmaf(x.z, w2.x, acc[i][0]); acc[i][1] = fmaf(x.z, w2.y, acc[i][1]);
-            acc[i][2] = fmaf(x.z, w2.z, acc[i][2]); acc[i][3] = fmaf(x.z, w2.w, acc[i][3]);
-            acc[i][0] = fmaf(x.w, w3.x, acc[i][0]); acc[i][1] = fmaf(x.w, w3.y, acc[i][1]);
-            acc[i][2] = fmaf(x.w, w3.z, acc[i][2]); acc[i][3] = fmaf(x.w, w3.w, acc[i][3]);
+        for (int n = 0; n < NC; ++n) {
+            w0[n] = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 0) * DOUT + 64 * n + tx * 4);
+            w1[n] = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 1) * DOUT + 64 * n + tx * 4);
+            w2[n] = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 2) * DOUT + 64 * n + tx * 4);
+            w3[n] = *reinterpret_cast<const float4*>(Ws + (k4 * 4 + 3) * DOUT + 64 * n + tx * 4);
+        }
+#pragma unroll
+        for (int i = 0; i < RI; ++i) {
+            float4 x = *reinterpret_cast<const float4*>(Xs + (ty + 16 * i) * XS + k4 * 4);
+#pragma unroll
+            for (int n = 0; n < NC; ++n) {
+                float* a = acc[i][n];
+                a[0] = fmaf(x.x, w0[n].x, a[0]); a[1] = fmaf(x.x, w0[n].y, a[1]);
+                a[2] = fmaf(x.x, w0[n].z, a[2]); a[3] = fmaf(x.x, w0[n].w, a[3]);
+                a[0] = fmaf(x.y, w1[n].x, a[0]); a[1] = fmaf(x.y, w1[n].y, a[1]);
+                a[2] = fmaf(x.y, w1[n].z, a[2]); a[3] = fmaf(x.y, w1[n].w, a[3]);
+                a[0] = fmaf(x.z, w2[n].x, a[0]); a[1] = fmaf(x.z, w2[n].y, a[1]);
+                a[2] = fmaf(x.z, w2[n].z, a[2]); a[3] = fmaf(x.z, w2[n].w, a[3]);
+                a[0] = fmaf(x.w, w3[n].x, a[0]); a[1] = fmaf(x.w, w3[n].y, a[1]);
+                a[2] = fmaf(x.w, w3[n].z, a[2]); a[3] = fmaf(x.w, w3[n].w, a[3]);
+            }
         }
     }
-    const float4 a4 = *reinterpret_cast<const float4*>(av + tx * 4);
+    float4 a4[NC];
+#pragma unroll
+    for (int n = 0; n < NC; ++n) a4[n] = *reinterpret_cast<const float4*>(av + 64 * n + tx * 4);
     const unsigned gm = group_mask();
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
+    for (int i = 0; i < RI; ++i) {
         int r = ty + 16 * i;
-        float part = acc[i][0] * a4.x + acc[i][1] * a4.y + acc[i][2] * a4.z + acc[i][3] * a4.w;
+        float part = acc[i][0][0] * a4[0].x + acc[i][0][1] * a4[0].y + acc[i][0][2] * a4[0].z + acc[i][0][3] * a4[0].w;
+#pragma unroll
+        for (int n = 1; n < NC; ++n)
+            part += acc[i][n][0] * a4[n].x + acc[i][n][1] * a4[n].y + acc[i][n][2] * a4[n].z + acc[i][n][3] * a4[n].w;
         part = head_reduce<H>(part, gm);     // every thread of the warp executes the shuffles
         if (r < nrows) {
             int64_t node = node0 + r;
-            st_stream4(h + node * D + tx * 4, make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]));
+#pragma unroll
+            for (int n = 0; n < NC; ++n)
+                st_stream4(h + node * DOUT + 64 * n + tx * 4, make_float4(acc[i][n][0], acc[i][n][1], acc[i][n][2], acc[i][n][3]));
             if (H == 8) { if ((tx & 1) == 0) s[node * 8 + (tx >> 1)] = part; }
             else        { if (tx == 0) s[node] = part; }
         }
@@ -398,6 +422,93 @@ __global__ void __launch_bounds__(256) aggregate_fwd_kernel(const int4* __restri
                                      partial_from);
 }
 
+// the single-head aggregation on W-wide rows (W = 128: the last stage at embedSize 128): the algorithm of aggregate_task<1, DROP,
+// false> (three-stage adjacency / logit / mask pipeline, one weight per lane and batch); lane l owns the W/16 columns W/16*l ..
+template <bool DROP, int W>
+__global__ void __launch_bounds__(256) aggregate_fwd_wide_kernel(const int4* __restrict__ tasks, int T, const int* __restrict__ adj_ptr,
+                                                                 const int* __restrict__ adj_idx, const int* __restrict__ adj_eid,
+                                                                 const int* __restrict__ long_first_slot, int* long_counter, float* scratch,
+                                                                 const float* __restrict__ h, const float* __restrict__ s,
+                                                                 const uint8_t* __restrict__ edgemask, float scale,
+                                                                 float* __restrict__ Z, float* __restrict__ norm) {
+    constexpr int V = W / 64;
+    const int t = (blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+    if (t >= T) return;                                  // whole 16-lane groups exit together
+    const int lane16 = threadIdx.x & 15;
+    const unsigned gm = group_mask();
+    const int col0 = lane16 * 4 * V;
+    const int4 tk = __ldg(tasks + t);
+    const int node = tk.x, beg = tk.y, end = tk.z, lid = tk.w;
+    const float sn = __ldg(s + node);
+    float4 acc[V];
+#pragma unroll
+    for (int v = 0; v < V; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
+    float rs_l = 0.f, s_c = 0.f;
+    int m_c = 0, m_1 = 0, eid_1 = 0;
+    unsigned mk_c = 1u;
+    if (beg + lane16 < end) {
+        m_c = ld_stream_i32(adj_idx + beg + lane16);
+        if (DROP) mk_c = edgemask[ld_stream_i32(adj_eid + beg + lane16)];
+    }
+    if (beg + 16 + lane16 < end) {
+        m_1 = ld_stream_i32(adj_idx + beg + 16 + lane16);
+        if (DROP) eid_1 = ld_stream_i32(adj_eid + beg + 16 + lane16);
+    }
+    if (beg + lane16 < end) s_c = __ldg(s + m_c);
+    for (int base = beg; base < end; base += 16) {
+        const int i1x = base + 16 + lane16, i2x = base + 32 + lane16;
+        int m_2 = 0, eid_2 = 0;
+        float s_1 = 0.f;
+        unsigned mk_1 = 1u;
+        if (i2x < end) {
+            m_2 = ld_stream_i32(adj_idx + i2x);
+            if (DROP) eid_2 = ld_stream_i32(adj_eid + i2x);
+        }
+        if (i1x < end) {
+            s_1 = __ldg(s + m_1);
+            if (DROP) mk_1 = edgemask[eid_1];
+        }
+        const float w_l = base + lane16 < end ? edge_weight(sn + s_c) : 0.f;
+        rs_l += w_l;
+        const float wd_l = DROP ? ((mk_c & 1u) ? w_l * scale : 0.f) : w_l;
+        const int cnt = min(16, end - base);
+#pragma unroll 8
+        for (int j = 0; j < cnt; ++j) {
+            const int m = __shfl_sync(gm, m_c, j, 16);
+            const float wd = __shfl_sync(gm, wd_l, j, 16);
+            float4 hm[V];
+#pragma unroll
+            for (int v = 0; v < V; ++v) hm[v] = ld_gather4(h + (int64_t)m * W + col0 + 4 * v);
+#pragma unroll
+            for (int v = 0; v < V; ++v) {
+                acc[v].x = fmaf(wd, hm[v].x, acc[v].x); acc[v].y = fmaf(wd, hm[v].y, acc[v].y);
+                acc[v].z = fmaf(wd, hm[v].z, acc[v].z); acc[v].w = fmaf(wd, hm[v].w, acc[v].w);
+            }
+        }
+        m_c = m_1; m_1 = m_2; eid_1 = eid_2; s_c = s_1; mk_c = mk_1;
+    }
+    rs_l += __shfl_xor_sync(gm, rs_l, 1, 16);
+    rs_l += __shfl_xor_sync(gm, rs_l, 2, 16);
+    rs_l += __shfl_xor_sync(gm, rs_l, 4, 16);
+    rs_l += __shfl_xor_sync(gm, rs_l, 8, 16);
+    float rs = rs_l;
+    if (lid >= 0) {
+        float sums[1] = {rs};
+        const int chunk = (beg - __ldg(adj_ptr + node)) / CHUNK;
+        if (!long_row_combine_wide<W, 1>(lid, chunk, long_first_slot, long_counter, scratch, lane16, gm, acc, sums)) return;
+        rs = sums[0];
+    }
+    // epilogue: Z = h + agg / norm, NaN -> 0 for isolated nodes (SPUIGACF.py:383,388-390)
+    const float inv = rs != 0.f ? 1.0f / rs : 0.f;
+#pragma unroll
+    for (int v = 0; v < V; ++v) {
+        const int64_t off = (int64_t)node * W + col0 + 4 * v;
+        const float4 hn = ld_stream4(h + off);
+        st_stream4(Z + off, make_float4(fmaf(acc[v].x, inv, hn.x), fmaf(acc[v].y, inv, hn.y), fmaf(acc[v].z, inv, hn.z), fmaf(acc[v].w, inv, hn.w)));
+    }
+    if (lane16 == 0) norm[node] = rs;
+}
+
 // Pruned last stage (FusedTrainer): only the tasks of the rows marked active are run (list built by ngacf_active_plan) -- the
 // step reads nothing else of the last stage's output (the pair scores gather the batch rows, every other row has a zero
 // gradient).  Persistent grid over the compacted list: the working groups are dense however few rows are active.
@@ -464,22 +575,36 @@ extern "C" int ngacf_edge_mask(uint8_t* edge, int64_t E, int32_t H, uint64_t see
     return check_launch("edge_mask");
 }
 
-extern "C" int ngacf_dropout_masks(uint64_t* const* feat, uint8_t* const* edge, const int32_t* heads, int32_t S, int64_t N, int64_t E,
-                                   uint64_t seed, uint32_t call, const int64_t* call_dev, float droprate, void* stream) {
+extern "C" int ngacf_dropout_masks_w(uint64_t* const* feat, uint8_t* const* edge, const int32_t* heads, const int32_t* widths, int32_t S,
+                                     int64_t N, int64_t E, uint64_t seed, uint32_t call, const int64_t* call_dev, float droprate,
+                                     void* stream) {
     NGACF_REQUIRE(feat && edge && heads && S >= 1 && S <= MASK_MAX_STAGES && N >= 0 && E >= 0, "dropout_masks: bad args");
     MaskPlan plan;
+    int max_shift = 0;
     for (int k = 0; k < S; ++k) {
         NGACF_REQUIRE(feat[k] && (edge[k] || E == 0) && (heads[k] == 1 || heads[k] == 8), "dropout_masks: bad stage %d", k);
+        const int wd = widths ? widths[k] : 64;
+        if (!width_supported(wd)) {
+            set_error("dropout_masks_w: stage %d input width %d is not built (supported: 64, 128)", k, wd);
+            return NGACF_ERR_UNSUPPORTED;
+        }
         plan.feat[k] = feat[k]; plan.edge[k] = edge[k]; plan.heads[k] = heads[k];
+        plan.wshift[k] = wd == 128 ? 1 : 0;
+        if (plan.wshift[k] > max_shift) max_shift = plan.wshift[k];
     }
     plan.S = S;
-    plan.feat_blocks = ceil_div(N * 8, 256);
+    plan.feat_blocks = ceil_div((N * 8) << max_shift, 256);
     plan.edge_blocks = ceil_div(E, 256);
     const int64_t blocks = (int64_t)S * (plan.feat_blocks + plan.edge_blocks);
     if (blocks == 0) return NGACF_OK;
     dropout_masks_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(plan, N, E, (uint32_t)seed, (uint32_t)(seed >> 32), call,
                                                                              call_dev, keep_threshold(droprate));
     return check_launch("dropout_masks");
+}
+
+extern "C" int ngacf_dropout_masks(uint64_t* const* feat, uint8_t* const* edge, const int32_t* heads, int32_t S, int64_t N, int64_t E,
+                                   uint64_t seed, uint32_t call, const int64_t* call_dev, float droprate, void* stream) {
+    return ngacf_dropout_masks_w(feat, edge, heads, nullptr, S, N, E, seed, call, call_dev, droprate, stream);
 }
 
 extern "C" int ngacf_dropout_masks_ranges(uint64_t* const* feat, uint8_t* const* edge, const int32_t* heads, int32_t S, int64_t fa0, int64_t fb0,
@@ -490,7 +615,7 @@ extern "C" int ngacf_dropout_masks_ranges(uint64_t* const* feat, uint8_t* const*
     MaskPlan plan;
     for (int k = 0; k < S; ++k) {
         NGACF_REQUIRE(feat[k] && (edge[k] || e1 == e0) && (heads[k] == 1 || heads[k] == 8), "dropout_masks_ranges: bad stage %d", k);
-        plan.feat[k] = feat[k]; plan.edge[k] = edge[k]; plan.heads[k] = heads[k];
+        plan.feat[k] = feat[k]; plan.edge[k] = edge[k]; plan.heads[k] = heads[k]; plan.wshift[k] = 0;
     }
     plan.S = S;
     plan.feat_blocks = plan.edge_blocks = 0;
@@ -518,14 +643,44 @@ extern "C" int ngacf_transform_fwd(const float* Xu, const float* Xi, int32_t app
     const int tiles_u = ceil_div(U, TF_TM), tiles_i = ceil_div(I, TF_TM);
     static PerDeviceOnce once;
     once.run([] {
-        cudaFuncSetAttribute(transform_fwd_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TF_SMEM);
-        cudaFuncSetAttribute(transform_fwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TF_SMEM);
+        cudaFuncSetAttribute(transform_fwd_kernel<8, 64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TF_SMEM);
+        cudaFuncSetAttribute(transform_fwd_kernel<1, 64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TF_SMEM);
     });
     if (H == 8)
-        transform_fwd_kernel<8><<<tiles_u + tiles_i, 256, TF_SMEM, (cudaStream_t)stream>>>(Xu, Xi, apply_elu, featmask, scale, wtab, U, I, tiles_u, h, s);
+        transform_fwd_kernel<8, 64, 64><<<tiles_u + tiles_i, 256, TF_SMEM, (cudaStream_t)stream>>>(Xu, Xi, apply_elu, featmask, scale, wtab, U, I, tiles_u, h, s);
     else
-        transform_fwd_kernel<1><<<tiles_u + tiles_i, 256, TF_SMEM, (cudaStream_t)stream>>>(Xu, Xi, apply_elu, featmask, scale, wtab, U, I, tiles_u, h, s);
+        transform_fwd_kernel<1, 64, 64><<<tiles_u + tiles_i, 256, TF_SMEM, (cudaStream_t)stream>>>(Xu, Xi, apply_elu, featmask, scale, wtab, U, I, tiles_u, h, s);
     return check_launch("transform_fwd");
+}
+
+// (d_in, d_out) = (64, 64): ngacf_transform_fwd (tensor cores or NGACF_DENSE=ffma).  The embedSize-128 shapes run on the CUDA-core
+// kernel: (128, 64) with 8 heads (first stage) and (64, 128) with one head (last stage).
+template <int H, int DIN, int DOUT>
+static int launch_transform_fwd_wide(const float* Xu, const float* Xi, int apply_elu, const uint64_t* featmask, float scale,
+                                     const float* const* wtab, int U, int I, float* h, float* s, cudaStream_t st) {
+    constexpr int TM = tf_tm<DOUT>();
+    constexpr size_t SMEM = tf_smem<DIN, DOUT>();
+    static PerDeviceOnce once;
+    once.run([] { cudaFuncSetAttribute(transform_fwd_kernel<H, DIN, DOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM); });
+    const int tiles_u = ceil_div(U, TM), tiles_i = ceil_div(I, TM);
+    transform_fwd_kernel<H, DIN, DOUT><<<tiles_u + tiles_i, 256, SMEM, st>>>(Xu, Xi, apply_elu, featmask, scale, wtab, U, I, tiles_u, h, s);
+    return check_launch("transform_fwd_w");
+}
+
+extern "C" int ngacf_transform_fwd_w(const float* Xu, const float* Xi, int32_t apply_elu, const uint64_t* featmask, float scale,
+                                     const float* const* wtab, int32_t H, int32_t d_in, int32_t d_out, int32_t U, int32_t I, float* h,
+                                     float* s, void* stream) {
+    if (d_in == 64 && d_out == 64) return ngacf_transform_fwd(Xu, Xi, apply_elu, featmask, scale, wtab, H, U, I, h, s, stream);
+    const bool first = H == 8 && d_in == 128 && d_out == 64, last = H == 1 && d_in == 64 && d_out == 128;
+    if (!first && !last) {
+        set_error("transform_fwd_w: (H, d_in, d_out) = (%d, %d, %d) is not built; supported: (1|8, 64, 64), (8, 128, 64), (1, 64, 128)", H,
+                  d_in, d_out);
+        return NGACF_ERR_UNSUPPORTED;
+    }
+    NGACF_REQUIRE(wtab && h && s && U >= 0 && I >= 0 && (U == 0 || Xu) && (I == 0 || Xi), "transform_fwd_w: null argument");
+    if (U + I == 0) return NGACF_OK;
+    if (first) return launch_transform_fwd_wide<8, 128, 64>(Xu, Xi, apply_elu, featmask, scale, wtab, U, I, h, s, (cudaStream_t)stream);
+    return launch_transform_fwd_wide<1, 64, 128>(Xu, Xi, apply_elu, featmask, scale, wtab, U, I, h, s, (cudaStream_t)stream);
 }
 
 extern "C" int ngacf_aggregate_fwd(const int32_t* tasks, int32_t T, const int32_t* adj_ptr, const int32_t* adj_idx, const int32_t* adj_eid,
@@ -555,6 +710,37 @@ extern "C" int ngacf_aggregate_fwd(const int32_t* tasks, int32_t T, const int32_
     }
 #undef LAUNCH
     return check_launch("aggregate_fwd");
+}
+
+extern "C" int ngacf_aggregate_fwd_w(const int32_t* tasks, int32_t T, const int32_t* adj_ptr, const int32_t* adj_idx, const int32_t* adj_eid,
+                                     const int32_t* long_first_slot, int32_t* long_counter, float* scratch, const float* h, const float* s,
+                                     int32_t H, int32_t width, const uint8_t* edgemask, float scale, float* Z, float* norm,
+                                     int32_t partial_from, void* stream) {
+    if (width == 64)
+        return ngacf_aggregate_fwd(tasks, T, adj_ptr, adj_idx, adj_eid, long_first_slot, long_counter, scratch, h, s, H, edgemask, scale, Z,
+                                   norm, partial_from, stream);
+    if (width != 128 || H != 1 || (partial_from >= 0 && partial_from < T)) {
+        set_error("aggregate_fwd_w: (H, width) = (%d, %d)%s is not built; 128-wide rows: H = 1, full rows", H, width,
+                  (partial_from >= 0 && partial_from < T) ? " with partial rows" : "");
+        return NGACF_ERR_UNSUPPORTED;
+    }
+    NGACF_REQUIRE(tasks && adj_ptr && adj_idx && h && s && Z && norm && T > 0, "aggregate_fwd_w: null/empty argument");
+    NGACF_REQUIRE(!edgemask || adj_eid, "aggregate_fwd_w: edge dropout needs adj_eid");
+    const int blocks = ceil_div((int64_t)T * 16, 256);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int4* tk = reinterpret_cast<const int4*>(tasks);
+    static PerDeviceOnce once;
+    once.run([] {
+        cudaFuncSetAttribute(aggregate_fwd_wide_kernel<true, 128>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
+        cudaFuncSetAttribute(aggregate_fwd_wide_kernel<false, 128>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
+    });
+    if (edgemask)
+        aggregate_fwd_wide_kernel<true, 128><<<blocks, 256, 0, st>>>(tk, T, adj_ptr, adj_idx, adj_eid, long_first_slot, long_counter, scratch, h,
+                                                                     s, edgemask, scale, Z, norm);
+    else
+        aggregate_fwd_wide_kernel<false, 128><<<blocks, 256, 0, st>>>(tk, T, adj_ptr, adj_idx, adj_eid, long_first_slot, long_counter, scratch, h,
+                                                                      s, edgemask, scale, Z, norm);
+    return check_launch("aggregate_fwd_w");
 }
 
 int ngacf_launch_aggregate_fwd_cta(const int32_t* tasks, int32_t T, const int32_t* task_list, const int32_t* task_count, const int32_t* adj_ptr,

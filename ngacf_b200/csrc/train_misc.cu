@@ -17,6 +17,23 @@ __device__ __forceinline__ float dot64_tree(float4 a, float4 b, unsigned gm) {
     return v;
 }
 
+// the same adjacent-pair tree over 128 products (oracle/port.py:dot64_tree, whose tree is generic over the length): lane l holds
+// columns 8l .. 8l+7 as two float4, levels 1-3 in the lane, levels 4-7 across the lanes
+__device__ __forceinline__ float dot128_tree(const float4 (&a)[2], const float4 (&b)[2], unsigned gm) {
+    float q[2];
+#pragma unroll
+    for (int v = 0; v < 2; ++v) {
+        const float p0 = __fmul_rn(a[v].x, b[v].x), p1 = __fmul_rn(a[v].y, b[v].y), p2 = __fmul_rn(a[v].z, b[v].z), p3 = __fmul_rn(a[v].w, b[v].w);
+        q[v] = __fadd_rn(__fadd_rn(p0, p1), __fadd_rn(p2, p3));
+    }
+    float v = __fadd_rn(q[0], q[1]);
+    v = __fadd_rn(v, __shfl_xor_sync(gm, v, 1, 16));
+    v = __fadd_rn(v, __shfl_xor_sync(gm, v, 2, 16));
+    v = __fadd_rn(v, __shfl_xor_sync(gm, v, 4, 16));
+    v = __fadd_rn(v, __shfl_xor_sync(gm, v, 8, 16));
+    return v;
+}
+
 __device__ __forceinline__ float4 elu4(float4 z) { return make_float4(elu(z.x), elu(z.y), elu(z.z), elu(z.w)); }
 
 __global__ void __launch_bounds__(256) score_pairs_kernel(const float* __restrict__ Z, int U, const int64_t* __restrict__ users,
@@ -29,6 +46,23 @@ __global__ void __launch_bounds__(256) score_pairs_kernel(const float* __restric
     const float4 fu = elu4(ld_gather4(Z + u * D + lane16 * 4));
     const float4 fi = elu4(ld_gather4(Z + it * D + lane16 * 4));
     const float sc = dot64_tree(fu, fi, gm);
+    if (lane16 == 0) scores[b] = sc;
+}
+
+__global__ void __launch_bounds__(256) score_pairs128_kernel(const float* __restrict__ Z, int U, const int64_t* __restrict__ users,
+                                                             const int64_t* __restrict__ items, int B, float* __restrict__ scores) {
+    const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+    if (b >= B) return;
+    const int lane16 = threadIdx.x & 15;
+    const unsigned gm = group_mask();
+    const int64_t u = users[b], it = items[b] + U;
+    float4 fu[2], fi[2];
+#pragma unroll
+    for (int v = 0; v < 2; ++v) {
+        fu[v] = elu4(ld_gather4(Z + u * 128 + lane16 * 8 + 4 * v));
+        fi[v] = elu4(ld_gather4(Z + it * 128 + lane16 * 8 + 4 * v));
+    }
+    const float sc = dot128_tree(fu, fi, gm);
     if (lane16 == 0) scores[b] = sc;
 }
 
@@ -45,13 +79,16 @@ __global__ void final_features_kernel(const float* __restrict__ Z, int64_t n4, f
 // entries in batch order, and its 16 lane-groups gather the matching rows in parallel (4 loads in flight each); the 16 partial
 // sums are combined in a fixed order.  A PairSampling batch is user-sorted, so a heavy user can own a whole batch: this keeps
 // that case parallel.
+// W: row width (64, or 128 at embedSize 128: lane l owns columns 8l .. 8l+7)
 constexpr int SPB_SUPER = 2048;
+template <int W = 64>
 __global__ void __launch_bounds__(256) score_pairs_bwd_kernel(const float* __restrict__ Z, int U, const int64_t* __restrict__ users,
                                                               const int64_t* __restrict__ items, const float* __restrict__ dscore, int B,
                                                               float* __restrict__ G, int accumulate) {
     __shared__ int list[SPB_SUPER];
     __shared__ int warp_cnt[8][8];
-    __shared__ float part[16][D];
+    constexpr int V = W / 64;
+    __shared__ float part[16][W];
     const int e = blockIdx.x;
     const bool user_row = e < B;
     const int eb = user_row ? e : e - B;
@@ -60,7 +97,9 @@ __global__ void __launch_bounds__(256) score_pairs_bwd_kernel(const float* __res
     const int64_t key = keys[eb];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int grp = tid >> 4, lane16 = tid & 15;
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 acc[V];
+#pragma unroll
+    for (int v = 0; v < V; ++v) acc[v] = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int sbase = 0; sbase < B; sbase += SPB_SUPER) {
         int64_t kreg[8];
 #pragma unroll
@@ -95,7 +134,7 @@ __global__ void __launch_bounds__(256) score_pairs_bwd_kernel(const float* __res
         }
         __syncthreads();
         for (int q0 = grp; q0 < total; q0 += 64) {           // group g takes matches g, g+16, g+32, g+48 per round
-            int jj[4]; float c[4]; float4 f[4];
+            int jj[4]; float c[4]; float4 f[4][V];
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 const int qi = q0 + 16 * q;
@@ -106,26 +145,36 @@ __global__ void __launch_bounds__(256) score_pairs_bwd_kernel(const float* __res
                 if (jj[q] >= 0) {
                     const int64_t other = others[jj[q]] + (user_row ? U : 0);
                     c[q] = dscore[jj[q]];
-                    f[q] = ld_gather4(Z + other * D + lane16 * 4);
-                } else { c[q] = 0.f; f[q] = make_float4(0.f, 0.f, 0.f, 0.f); }
+#pragma unroll
+                    for (int v = 0; v < V; ++v) f[q][v] = ld_gather4(Z + other * W + lane16 * 4 * V + 4 * v);
+                } else {
+                    c[q] = 0.f;
+#pragma unroll
+                    for (int v = 0; v < V; ++v) f[q][v] = make_float4(0.f, 0.f, 0.f, 0.f);
+                }
             }
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
-                const float4 fo = elu4(f[q]);
-                acc.x = fmaf(c[q], fo.x, acc.x); acc.y = fmaf(c[q], fo.y, acc.y); acc.z = fmaf(c[q], fo.z, acc.z); acc.w = fmaf(c[q], fo.w, acc.w);
+#pragma unroll
+                for (int v = 0; v < V; ++v) {
+                    const float4 fo = elu4(f[q][v]);
+                    float4& a = acc[v];
+                    a.x = fmaf(c[q], fo.x, a.x); a.y = fmaf(c[q], fo.y, a.y); a.z = fmaf(c[q], fo.z, a.z); a.w = fmaf(c[q], fo.w, a.w);
+                }
             }
         }
         __syncthreads();                                      // list is rewritten by the next 2048 keys
     }
-    *reinterpret_cast<float4*>(&part[grp][lane16 * 4]) = acc;
+#pragma unroll
+    for (int v = 0; v < V; ++v) *reinterpret_cast<float4*>(&part[grp][lane16 * 4 * V + 4 * v]) = acc[v];
     __syncthreads();
-    if (tid < D) {
+    if (tid < W) {
         float sum = 0.f;
 #pragma unroll
         for (int g = 0; g < 16; ++g) sum += part[g][tid];
         const int64_t row = user_row ? key : key + U;
-        const float gnew = sum * elu_grad(Z[row * D + tid]);
-        G[row * D + tid] = accumulate ? G[row * D + tid] + gnew : gnew;
+        const float gnew = sum * elu_grad(Z[row * W + tid]);
+        G[row * W + tid] = accumulate ? G[row * W + tid] + gnew : gnew;
     }
 }
 
@@ -415,4 +464,34 @@ extern "C" int ngacf_sample_pairs(const int32_t* train_rows_user, const int32_t*
                                                                              row_begin, n, row_dev, (uint32_t)seed, (uint32_t)(seed >> 32), epoch,
                                                                              users, pos, neg);
     return check_launch("sample_pairs");
+}
+
+// width-carrying entry points: width 64 reaches the calls above (the same kernels)
+extern "C" int ngacf_score_pairs_w(const float* Z, int32_t width, int32_t U, const int64_t* users, const int64_t* items, int32_t B, float* scores,
+                                   void* stream) {
+    if (width == 64) return ngacf_score_pairs(Z, U, users, items, B, scores, stream);
+    if (width != 128) { set_error("score_pairs_w: width %d is not built (supported: 64, 128)", width); return NGACF_ERR_UNSUPPORTED; }
+    NGACF_REQUIRE(Z && users && items && scores && B >= 0, "score_pairs_w: null argument");
+    if (B == 0) return NGACF_OK;
+    score_pairs128_kernel<<<ceil_div((int64_t)B * 16, 256), 256, 0, (cudaStream_t)stream>>>(Z, U, users, items, B, scores);
+    return check_launch("score_pairs_w");
+}
+
+extern "C" int ngacf_score_pairs_bwd_w(const float* Z, int32_t width, int32_t U, const int64_t* users, const int64_t* items, const float* dscore,
+                                       int32_t B, float* G, int32_t accumulate, void* stream) {
+    if (width == 64) return ngacf_score_pairs_bwd(Z, U, users, items, dscore, B, G, accumulate, stream);
+    if (width != 128) { set_error("score_pairs_bwd_w: width %d is not built (supported: 64, 128)", width); return NGACF_ERR_UNSUPPORTED; }
+    NGACF_REQUIRE(Z && users && items && dscore && G && B >= 0, "score_pairs_bwd_w: null argument");
+    if (B == 0) return NGACF_OK;
+    score_pairs_bwd_kernel<128><<<2 * B, 256, 0, (cudaStream_t)stream>>>(Z, U, users, items, dscore, B, G, accumulate);
+    return check_launch("score_pairs_bwd_w");
+}
+
+extern "C" int ngacf_final_features_w(const float* Z, int64_t N, int32_t width, float* F, void* stream) {
+    if (width == 64) return ngacf_final_features(Z, N, F, stream);
+    if (width != 128) { set_error("final_features_w: width %d is not built (supported: 64, 128)", width); return NGACF_ERR_UNSUPPORTED; }
+    NGACF_REQUIRE(Z && F && N >= 0, "final_features_w: null argument");
+    if (N == 0) return NGACF_OK;
+    final_features_kernel<<<ceil_div(N * 32, 256), 256, 0, (cudaStream_t)stream>>>(Z, N * 32, F);    // elementwise: N*128/4 float4
+    return check_launch("final_features_w");
 }

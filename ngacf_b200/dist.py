@@ -68,10 +68,18 @@ def shard_eval_users(eval_users: torch.Tensor, rank: int, world: int) -> torch.T
     return eval_users[lo:hi].contiguous()
 
 
+def require_width_64(model):
+    """The multi-GPU trainers (partial-row kernels, batch-row exchange) are built for embedSize 64 only."""
+    if getattr(model, "embedSize", 64) != 64:
+        raise ValueError("multi-GPU training is built for embedSize 64 only (got %d); train embedSize %d on one GPU"
+                         % (model.embedSize, model.embedSize))
+
+
 class ReplicaTrainer(FusedTrainer):
     """Data-parallel replicas of the fused step (see module docstring)."""
 
     def __init__(self, model, inter, graph, batch_size, optim, sample_seed, use_cuda_graph=True, two_streams=True):
+        require_width_64(model)
         self.rank, self.world = world_info()
         super().__init__(model, inter, graph, batch_size, optim, sample_seed, use_cuda_graph, two_streams)
         self.weak = True
@@ -393,6 +401,7 @@ class ShardedTrainer:
                  plan=None, prop_parallel=None):
         from .graph import BipartiteGraph
         from .propagation import Propagation
+        require_width_64(model)
         if transport is None:
             r0, w0 = world_info()
             self.topo = Topology(r0, w0, prop_parallel)

@@ -32,9 +32,14 @@ class AllNegEvaluator:
         self.fallback = torch.zeros(max(n, 1) + 1, dtype=torch.int32, device=dev)      # flag per user + number of flagged users
         self._pending_fallback = False
 
-    def _use_tc(self):
+    def _use_tc(self, width: int = 64):
         from . import _lib
         if self.mode == "exact":
+            return False
+        if width != 64:
+            # the tcgen05 scorer is built for 64-wide features; 'auto' ranks wider ones on the exact path
+            if self.mode == "tc":
+                raise _lib.NgacfError("ngacf_score_topk_tc is built for 64-wide features (got %d); use mode='exact' or 'auto'" % width)
             return False
         have = hasattr(_lib.load(), "ngacf_score_topk_tc")
         if self.mode == "tc" and not have:
@@ -42,7 +47,7 @@ class AllNegEvaluator:
         return have
 
     def rank(self, Z: torch.Tensor):
-        """Z: pre-ELU last-stage output (N,64).  Fills top_ids/top_scores for inter.eval_users."""
+        """Z: pre-ELU last-stage output (N,64) or (N,128).  Fills top_ids/top_scores for inter.eval_users."""
         it = self.inter
         if self.F is None or self.F.shape != Z.shape:
             self.F = torch.empty_like(Z)
@@ -50,7 +55,7 @@ class AllNegEvaluator:
         n = self.users.numel()
         if n == 0:
             return
-        if self._use_tc():
+        if self._use_tc(Z.shape[-1]):
             # the workspace also carries the allowed-column matrix of (users, train set, pool): built by the first call, reused while
             # this evaluator's users tensor and the interactions' arrays are the same objects at the same version
             key = (self.users.data_ptr(), self.users._version, it.train_ptr.data_ptr(), it.train_ptr._version, it.train_items.data_ptr(),

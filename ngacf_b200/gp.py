@@ -112,6 +112,8 @@ class GPLayer(nn.Module):
 
 class SPUIGAGPCF(SPUIGACF):
     def __init__(self, userNum, itemNum, adj, embedSize, layers, droprate, useCuda=True):
+        if embedSize != 64:
+            raise ValueError("SPUIGAGPCF is built for embedSize 64 only (its GP layers and stage kernels are 64 wide)")
         super().__init__(userNum, itemNum, embedSize, list(layers), droprate, useCuda)
         self.LaplacianMat = adj
         self._lap_key, self._lap = None, None

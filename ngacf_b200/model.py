@@ -40,7 +40,7 @@ class SpUIGraphAttentionLayer(nn.Module):
 
 
 class SpUIGAT(nn.Module):
-    """attention_0..7 (64->8, concat) + out_att (64->64)  (SPUIGACF.py:187-205)."""
+    """attention_0..7 (embedSize->8, concat) + out_att (64->embedSize)  (SPUIGACF.py:187-205)."""
 
     def __init__(self, nfeat, nhid, nclass, dropout, alpha, nheads):
         super().__init__()
@@ -62,7 +62,8 @@ class SpUIGAT(nn.Module):
 
 
 class SPUIMultiGAT(nn.Module):
-    """attention1_0..7, attention2_0..7 (64->8, concat) + out_att (64->64): the 3-stage variant (SPUIGACF.py:217-256)."""
+    """attention1_0..7 (embedSize->8), attention2_0..7 (64->8, concat) + out_att (64->embedSize): the 3-stage variant
+    (SPUIGACF.py:217-256).  attention2 reads the 64-wide concatenation of attention1; at embedSize 64 its in_dim is nfeat."""
 
     def __init__(self, nfeat, nhid, nclass, dropout, alpha, nheads):
         super().__init__()
@@ -70,7 +71,7 @@ class SPUIMultiGAT(nn.Module):
         self.nheads = nheads
         # the reference constructs all attentions1 layers, then all attentions2 layers, then registers them (same RNG order)
         a1 = [SpUIGraphAttentionLayer(nfeat, nhid, dropout, alpha, True) for _ in range(nheads)]
-        a2 = [SpUIGraphAttentionLayer(nfeat, nhid, dropout, alpha, True) for _ in range(nheads)]
+        a2 = [SpUIGraphAttentionLayer(nhid * nheads, nhid, dropout, alpha, True) for _ in range(nheads)]
         for k, l in enumerate(a1):
             self.add_module("attention1_{}".format(k), l)
         for k, l in enumerate(a2):
@@ -87,16 +88,17 @@ class SPUIMultiGAT(nn.Module):
 
 
 class SPUIGACF(nn.Module):
+    """embedSize 64 or 128 (ops.WIDTHS); anything else raises ValueError."""
     GAT = SpUIGAT
-    STAGES = ((8, 8), (1, 64))
+    HEAD_STAGES = 1               # 8-head stages in front of out_att
 
     def __init__(self, userNum, itemNum, embedSize, layers, droprate, useCuda=True):
         super().__init__()
-        if embedSize != 64:
-            raise ValueError("the sm_100a kernels are specialised for embedSize 64 (every BASELINE config)")
+        ops.check_width(embedSize)
         self.useCuda = useCuda
+        self.embedSize = int(embedSize)
         self.userNum, self.itemNum, self.droprate = int(userNum), int(itemNum), float(droprate)
-        self.stages = tuple(self.STAGES)
+        self.stages = ops.spuigacf_stages(embedSize, self.HEAD_STAGES)
         self.uEmbd = nn.Embedding(userNum, embedSize)
         self.iEmbd = nn.Embedding(itemNum, embedSize)
         # `layers` is accepted and ignored exactly as in the reference (SPUIGACF.py:7 is its only use)
@@ -134,7 +136,7 @@ class SPUIGACF(nn.Module):
         return self.drop_seed
 
     def propagate(self, mask) -> torch.Tensor:
-        """Pre-ELU output Z (N,64) of the last stage; final features are ELU(Z)."""
+        """Pre-ELU output Z (N,embedSize) of the last stage; final features are ELU(Z)."""
         dev = self.uEmbd.weight.device
         if dev.type != "cuda":
             raise _lib.NgacfError("SPUIGACF runs on CUDA only (sm_100a kernels, no CPU fallback); call .cuda() first")
@@ -171,4 +173,4 @@ class SPUIGACF(nn.Module):
 class SPUIMultiGACF(SPUIGACF):
     """3-stage variant (SPUIGACF.py:54-101): two 8-head stages, then out_att.  Same kernels, one more entry in the stage list."""
     GAT = SPUIMultiGAT
-    STAGES = ((8, 8), (8, 8), (1, 64))
+    HEAD_STAGES = 2

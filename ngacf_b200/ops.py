@@ -12,6 +12,20 @@ from .graph import BipartiteGraph
 
 STAGES = ((8, 8), (1, 64))   # SPUIGACF: eight 64->8 heads, then out_att 64->64 (SPUIGACF.py:17-22,191-205)
 D = 64
+WIDTHS = (64, 128)           # embedSize values the kernels are built for; the `_w` entry points carry widths other than 64
+
+
+def spuigacf_stages(embed: int, n_head_stages: int = 1):
+    """Stage list (heads, width per head) of SPUIGACF (n_head_stages = 1) / SPUIMultiGACF (2) at embedSize `embed`: every head
+    stage writes 8 x 8 = 64 columns, out_att writes `embed`.  The input width of the first stage is `embed` (the embedding tables)."""
+    check_width(embed)
+    return ((8, 8),) * n_head_stages + ((1, int(embed)),)
+
+
+def check_width(embed: int):
+    if int(embed) not in WIDTHS:
+        raise ValueError("embedSize %r is not supported: the sm_100a kernels are built for embedSize %s"
+                         % (embed, " and ".join(str(w) for w in WIDTHS)))
 
 
 def _p(t):
@@ -48,13 +62,18 @@ def counter_add(counter, delta):
     _lib.call("ngacf_counter_add", _p(counter), int(delta), _s())
 
 
-def dropout_masks(feats, edges, heads, N, E, seed, call, droprate, call_dev=None):
-    """every stage's feature + edge mask of one propagation in a single launch (same bits as feature_mask/edge_mask per stage)"""
+def dropout_masks(feats, edges, heads, N, E, seed, call, droprate, call_dev=None, widths=None):
+    """every stage's feature + edge mask of one propagation in a single launch (same bits as feature_mask/edge_mask per stage);
+    widths: per-stage input widths (feature masks of width/64 words per row), None = all 64"""
     S = len(heads)
     fa = (ctypes.c_void_p * S)(*[f.data_ptr() for f in feats])
     ea = (ctypes.c_void_p * S)(*[e.data_ptr() for e in edges])
     ha = (ctypes.c_int32 * S)(*[int(h) for h in heads])
-    _lib.call("ngacf_dropout_masks", fa, ea, ha, S, int(N), int(E), int(seed), int(call) & 0xFFFFFFFF, _p(call_dev), float(droprate), _s())
+    if widths is None or all(int(w) == 64 for w in widths):
+        _lib.call("ngacf_dropout_masks", fa, ea, ha, S, int(N), int(E), int(seed), int(call) & 0xFFFFFFFF, _p(call_dev), float(droprate), _s())
+        return
+    wa = (ctypes.c_int32 * S)(*[int(w) for w in widths])
+    _lib.call("ngacf_dropout_masks_w", fa, ea, ha, wa, S, int(N), int(E), int(seed), int(call) & 0xFFFFFFFF, _p(call_dev), float(droprate), _s())
 
 
 def dropout_masks_ranges(feats, edges, heads, node_ranges, edge_range, seed, call, droprate, call_dev=None):
@@ -81,13 +100,21 @@ def memset_zero(t):
     _lib.call("ngacf_memset_zero", _p(t), t.numel() * t.element_size(), _s())
 
 
-def transform_fwd(Xu, Xi, apply_elu, featmask, scale, wtab, H, U, I, h, s):
-    _lib.call("ngacf_transform_fwd", _p(Xu), _p(Xi), int(apply_elu), _p(featmask), float(scale), _p(wtab), H, U, I, _p(h), _p(s), _s())
+def transform_fwd(Xu, Xi, apply_elu, featmask, scale, wtab, H, U, I, h, s, d_in=64, d_out=64):
+    if d_in == 64 and d_out == 64:
+        _lib.call("ngacf_transform_fwd", _p(Xu), _p(Xi), int(apply_elu), _p(featmask), float(scale), _p(wtab), H, U, I, _p(h), _p(s), _s())
+    else:
+        _lib.call("ngacf_transform_fwd_w", _p(Xu), _p(Xi), int(apply_elu), _p(featmask), float(scale), _p(wtab), H, int(d_in), int(d_out), U, I,
+                  _p(h), _p(s), _s())
 
 
-def aggregate_fwd(g: BipartiteGraph, scratch, counter, h, s, H, edgemask, scale, Z, norm, partial_from=-1):
-    _lib.call("ngacf_aggregate_fwd", _p(g.tasks), g.T, _p(g.adj_ptr), _p(g.adj_idx), _p(g.adj_eid), _p(g.long_first_slot),
-              _p(counter), _p(scratch), _p(h), _p(s), H, _p(edgemask), float(scale), _p(Z), _p(norm), int(partial_from), _s())
+def aggregate_fwd(g: BipartiteGraph, scratch, counter, h, s, H, edgemask, scale, Z, norm, partial_from=-1, width=64):
+    if width == 64:
+        _lib.call("ngacf_aggregate_fwd", _p(g.tasks), g.T, _p(g.adj_ptr), _p(g.adj_idx), _p(g.adj_eid), _p(g.long_first_slot),
+                  _p(counter), _p(scratch), _p(h), _p(s), H, _p(edgemask), float(scale), _p(Z), _p(norm), int(partial_from), _s())
+    else:
+        _lib.call("ngacf_aggregate_fwd_w", _p(g.tasks), g.T, _p(g.adj_ptr), _p(g.adj_idx), _p(g.adj_eid), _p(g.long_first_slot),
+                  _p(counter), _p(scratch), _p(h), _p(s), H, int(width), _p(edgemask), float(scale), _p(Z), _p(norm), int(partial_from), _s())
 
 
 class ActiveRows:
@@ -152,39 +179,67 @@ def bpr_loss_owned(pos, neg, gscale, loss, dpos, dneg, users, u_lo, u_hi):
 
 
 def score_pairs(Z, U, users, items, out):
-    _lib.call("ngacf_score_pairs", _p(Z), U, _p(users), _p(items), users.numel(), _p(out), _s())
+    """the row width is Z's (64 or 128)"""
+    if Z.shape[-1] == 64:
+        _lib.call("ngacf_score_pairs", _p(Z), U, _p(users), _p(items), users.numel(), _p(out), _s())
+    else:
+        _lib.call("ngacf_score_pairs_w", _p(Z), int(Z.shape[-1]), U, _p(users), _p(items), users.numel(), _p(out), _s())
 
 
 def score_pairs_bwd(Z, U, users, items, dscore, G, accumulate=False):
-    _lib.call("ngacf_score_pairs_bwd", _p(Z), U, _p(users), _p(items), _p(dscore), users.numel(), _p(G), int(accumulate), _s())
+    if Z.shape[-1] == 64:
+        _lib.call("ngacf_score_pairs_bwd", _p(Z), U, _p(users), _p(items), _p(dscore), users.numel(), _p(G), int(accumulate), _s())
+    else:
+        _lib.call("ngacf_score_pairs_bwd_w", _p(Z), int(Z.shape[-1]), U, _p(users), _p(items), _p(dscore), users.numel(), _p(G),
+                  int(accumulate), _s())
 
 
 def final_features(Z, F):
-    _lib.call("ngacf_final_features", _p(Z), Z.shape[0], _p(F), _s())
+    if Z.shape[-1] == 64:
+        _lib.call("ngacf_final_features", _p(Z), Z.shape[0], _p(F), _s())
+    else:
+        _lib.call("ngacf_final_features_w", _p(Z), Z.shape[0], int(Z.shape[-1]), _p(F), _s())
 
 
 def bpr_loss(pos, neg, gscale, loss, dpos, dneg):
     _lib.call("ngacf_bpr_loss", _p(pos), _p(neg), pos.numel(), float(gscale), _p(loss), _p(dpos), _p(dneg), _s())
 
 
-def stage_bwd_prep(G, Z, h, norm, H, Ghat, dN):
-    _lib.call("ngacf_stage_bwd_prep", _p(G), _p(Z), _p(h), _p(norm), H, G.shape[0], _p(Ghat), _p(dN), _s())
+def stage_bwd_prep(G, Z, h, norm, H, Ghat, dN, width=64):
+    if width == 64:
+        _lib.call("ngacf_stage_bwd_prep", _p(G), _p(Z), _p(h), _p(norm), H, G.shape[0], _p(Ghat), _p(dN), _s())
+    else:
+        _lib.call("ngacf_stage_bwd_prep_w", _p(G), _p(Z), _p(h), _p(norm), H, int(width), G.shape[0], _p(Ghat), _p(dN), _s())
 
 
-def stage_bwd_edges(mode, g: BipartiteGraph, scratch, counter, G, Ghat, dN, h, s, H, edgemask, scale, wtab, ds_store, dh, dS, partial=0):
+def stage_bwd_edges(mode, g: BipartiteGraph, scratch, counter, G, Ghat, dN, h, s, H, edgemask, scale, wtab, ds_store, dh, dS, partial=0,
+                    width=64):
     t0, t1 = (0, g.T_users) if mode == 0 else (g.T_users, g.T)
-    _lib.call("ngacf_stage_bwd_edges", mode, _p(g.tasks), t0, t1, _p(g.adj_ptr), _p(g.adj_idx), _p(g.adj_eid),
-              _p(g.long_first_slot), _p(counter), _p(scratch), _p(G), _p(Ghat), _p(dN), _p(h), _p(s), H, _p(edgemask),
-              float(scale), _p(wtab), g.U, _p(ds_store), _p(dh), _p(dS), int(partial), _s())
+    if width == 64:
+        _lib.call("ngacf_stage_bwd_edges", mode, _p(g.tasks), t0, t1, _p(g.adj_ptr), _p(g.adj_idx), _p(g.adj_eid),
+                  _p(g.long_first_slot), _p(counter), _p(scratch), _p(G), _p(Ghat), _p(dN), _p(h), _p(s), H, _p(edgemask),
+                  float(scale), _p(wtab), g.U, _p(ds_store), _p(dh), _p(dS), int(partial), _s())
+    else:
+        _lib.call("ngacf_stage_bwd_edges_w", mode, _p(g.tasks), t0, t1, _p(g.adj_ptr), _p(g.adj_idx), _p(g.adj_eid),
+                  _p(g.long_first_slot), _p(counter), _p(scratch), _p(G), _p(Ghat), _p(dN), _p(h), _p(s), H, int(width), _p(edgemask),
+                  float(scale), _p(wtab), g.U, _p(ds_store), _p(dh), _p(dS), int(partial), _s())
 
 
-def transform_bwd_workspace_bytes(U, I):
-    return int(_lib.load().ngacf_transform_bwd_workspace_bytes(U, I))
+def transform_bwd_workspace_bytes(U, I, d_in=64, d_out=64):
+    if d_in == 64 and d_out == 64:
+        return int(_lib.load().ngacf_transform_bwd_workspace_bytes(U, I))
+    return int(_lib.load().ngacf_transform_bwd_workspace_bytes_w(int(d_in), int(d_out), U, I))
 
 
-def transform_bwd(dh, dS, h, Xu, Xi, apply_elu, featmask, scale, wtab, gtab, H, U, I, dXu, dXi, accumulate_dx, accumulate_dw, ws):
-    _lib.call("ngacf_transform_bwd", _p(dh), _p(dS), _p(h), _p(Xu), _p(Xi), int(apply_elu), _p(featmask), float(scale), _p(wtab),
-              _p(gtab), H, U, I, _p(dXu), _p(dXi), int(accumulate_dx), int(accumulate_dw), _p(ws), ws.numel() * ws.element_size(), _s())
+def transform_bwd(dh, dS, h, Xu, Xi, apply_elu, featmask, scale, wtab, gtab, H, U, I, dXu, dXi, accumulate_dx, accumulate_dw, ws,
+                  d_in=64, d_out=64):
+    if d_in == 64 and d_out == 64:
+        _lib.call("ngacf_transform_bwd", _p(dh), _p(dS), _p(h), _p(Xu), _p(Xi), int(apply_elu), _p(featmask), float(scale), _p(wtab),
+                  _p(gtab), H, U, I, _p(dXu), _p(dXi), int(accumulate_dx), int(accumulate_dw), _p(ws), ws.numel() * ws.element_size(), _s())
+    else:
+        _lib.call("ngacf_transform_bwd_w", _p(dh), _p(dS), _p(h), _p(Xu), _p(Xi), int(apply_elu), _p(featmask), float(scale), _p(wtab),
+                  _p(gtab), H, int(d_in), int(d_out), U, I, _p(dXu), _p(dXi), int(accumulate_dx), int(accumulate_dw), _p(ws),
+                  ws.numel() * ws.element_size(), _s())
 
 
 def transform_bwd_dx(dh, Xu, Xi, apply_elu, featmask, scale, wtab, H, U, I, dXu, dXi, accumulate):
@@ -216,16 +271,25 @@ def sample_pairs(inter, row_begin, row_end, seed, epoch, users, pos, neg, row_de
 
 
 def score_topk_exact(F, U, I, users, inter, top_ids, top_scores):
-    _lib.call("ngacf_score_topk_exact", _p(F), U, I, _p(users), users.numel(), _p(inter.train_ptr), _p(inter.train_items),
-              _p(inter.in_pool), _p(top_ids), _p(top_scores), _s())
+    """the row width is F's (64 or 128)"""
+    if F.shape[-1] == 64:
+        _lib.call("ngacf_score_topk_exact", _p(F), U, I, _p(users), users.numel(), _p(inter.train_ptr), _p(inter.train_items),
+                  _p(inter.in_pool), _p(top_ids), _p(top_scores), _s())
+    else:
+        _lib.call("ngacf_score_topk_exact_w", _p(F), int(F.shape[-1]), U, I, _p(users), users.numel(), _p(inter.train_ptr),
+                  _p(inter.train_items), _p(inter.in_pool), _p(top_ids), _p(top_scores), _s())
 
 
 def score_topk_exact_split(F, U, I, users, inter, top_ids, top_scores):
     """score_topk_exact for few users: item range split over CTAs (workspace allocated here: this is the rare fallback path)"""
     n = users.numel()
     ws = torch.empty(int(_lib.load().ngacf_score_topk_exact_split_workspace_bytes(I, n)), dtype=torch.uint8, device=F.device)
-    _lib.call("ngacf_score_topk_exact_split", _p(F), U, I, _p(users), n, _p(inter.train_ptr), _p(inter.train_items),
-              _p(inter.in_pool), _p(top_ids), _p(top_scores), _p(ws), ws.numel(), _s())
+    if F.shape[-1] == 64:
+        _lib.call("ngacf_score_topk_exact_split", _p(F), U, I, _p(users), n, _p(inter.train_ptr), _p(inter.train_items),
+                  _p(inter.in_pool), _p(top_ids), _p(top_scores), _p(ws), ws.numel(), _s())
+    else:
+        _lib.call("ngacf_score_topk_exact_split_w", _p(F), int(F.shape[-1]), U, I, _p(users), n, _p(inter.train_ptr), _p(inter.train_items),
+                  _p(inter.in_pool), _p(top_ids), _p(top_scores), _p(ws), ws.numel(), _s())
 
 
 def score_topk_tc_workspace_bytes(I, n_users):

@@ -2,7 +2,8 @@
 closed-form backward (SURVEY.md 3.4) over persistent HBM buffers, plus the autograd bridge used by the
 drop-in ``SPUIGACF.forward``.
 
-Layout in HBM per propagation (N = U+I nodes, users first; every row is 64 fp32 = 256 B):
+Layout in HBM per propagation (N = U+I nodes, users first; a row is 64 fp32 = 256 B at embedSize 64; at embedSize 128 the
+embedding tables, the last stage's h/Z and the backward buffers of that stage are 128 wide, masks of the first stage 2 words):
   stage k:  h_k (N,64)  transformed features      s_k (N,H)  rank-1 logit scalars (p|q)
             Z_k (N,64)  pre-ELU stage output       norm_k (N,H) attention row/col sums (R|C)
             featmask_k uint64[N], edgemask_k uint8[E]   dropout keep bits (only when dropout is on)
@@ -18,24 +19,31 @@ import torch
 
 from . import ops
 from .graph import BipartiteGraph
-from .ops import D, STAGES
+from .ops import STAGES
 
 
 class Propagation:
     def __init__(self, graph: BipartiteGraph, stages=STAGES):
+        """stages: (heads, width per head) per stage.  Stage k writes H*DH columns; the first stage reads the embedding tables, whose
+        width is the last stage's output width (SPUIGACF's out_att maps back to embedSize), every later stage the previous output."""
         self.g = graph
         self.stages = tuple(stages)
+        self.w_out = [H * DH for H, DH in self.stages]
+        self.w_in = [self.w_out[-1]] + self.w_out[:-1]
+        for w in self.w_out + self.w_in:
+            ops.check_width(w)
+        self.w_max = max(self.w_out)
         dev, N, E = graph.device, graph.N, graph.E
         f32 = dict(dtype=torch.float32, device=dev)
-        self.h = [torch.empty((N, D), **f32) for _ in self.stages]
-        self.Z = [torch.zeros((N, D), **f32) for _ in self.stages]        # zeros: rows a pruned last stage skips stay finite
+        self.h = [torch.empty((N, w), **f32) for w in self.w_out]
+        self.Z = [torch.zeros((N, w), **f32) for w in self.w_out]        # zeros: rows a pruned last stage skips stay finite
         self.s = [torch.empty((N, H), **f32) for H, _ in self.stages]
         self.norm = [torch.zeros((N, H), **f32) for H, _ in self.stages]
         self.featmask: List[Optional[torch.Tensor]] = [None] * len(self.stages)
         self.edgemask: List[Optional[torch.Tensor]] = [None] * len(self.stages)
         self._own_masks = None
         self.scale = 1.0
-        self.scratch, self.counter = (torch.empty(max(graph.S, 1) * 72, **f32),
+        self.scratch, self.counter = (torch.empty(max(graph.S, 1) * (self.w_max + 8), **f32),
                                       torch.zeros(max(graph.L, 1), dtype=torch.int32, device=dev))
         self._bwd = None
 
@@ -43,7 +51,7 @@ class Propagation:
     def _mask_buffers(self):
         if self._own_masks is None:
             dev = self.g.device
-            self._own_masks = ([torch.empty(self.g.N, dtype=torch.int64, device=dev) for _ in self.stages],
+            self._own_masks = ([torch.empty(self.g.N * (w // 64), dtype=torch.int64, device=dev) for w in self.w_in],
                                [torch.empty(max(self.g.E, 1), dtype=torch.uint8, device=dev) for _ in self.stages])
         return self._own_masks
 
@@ -60,7 +68,7 @@ class Propagation:
             self.edgemask = [m.contiguous() for m in injected["edge"]]
             return
         fm, em = self._mask_buffers()
-        ops.dropout_masks(fm, em, [H for H, _ in self.stages], self.g.N, self.g.E, seed, call, droprate, call_dev)
+        ops.dropout_masks(fm, em, [H for H, _ in self.stages], self.g.N, self.g.E, seed, call, droprate, call_dev, widths=self.w_in)
         self.featmask, self.edgemask = list(fm), [m[:self.g.E] for m in em]
 
     def use_dropout_buffers(self, droprate: float):
@@ -76,8 +84,9 @@ class Propagation:
 
     # ------------------------------------------------------------------------------------------
     def can_prune(self) -> bool:
-        """The pruned last stage (ops.ActiveRows) exists for a single-head output stage, which every model of the family has."""
-        return self.stages[-1][0] == 1
+        """The pruned last stage (ops.ActiveRows) exists for a single-head, 64-wide output stage, which every model of the family
+        has at embedSize 64 (at 128 the full last stage runs)."""
+        return self.stages[-1][0] == 1 and self.w_out[-1] == 64
 
     def forward(self, uEmbd: torch.Tensor, iEmbd: torch.Tensor, wtabs: Sequence[torch.Tensor], after_first_kernel=None,
                 active=None) -> torch.Tensor:
@@ -90,7 +99,8 @@ class Propagation:
         Xu, Xi, act = uEmbd, iEmbd, 0
         last = len(self.stages) - 1
         for k, (H, _) in enumerate(self.stages):
-            ops.transform_fwd(Xu, Xi, act, self.featmask[k], self.scale, wtabs[k], H, g.U, g.I, self.h[k], self.s[k])
+            ops.transform_fwd(Xu, Xi, act, self.featmask[k], self.scale, wtabs[k], H, g.U, g.I, self.h[k], self.s[k],
+                              d_in=self.w_in[k], d_out=self.w_out[k])
             if k == 0 and after_first_kernel is not None:
                 after_first_kernel()
             if active is not None and k == last:
@@ -98,7 +108,7 @@ class Propagation:
                                          self.Z[k], self.norm[k], active)
             else:
                 ops.aggregate_fwd(g, self.scratch, self.counter, self.h[k], self.s[k], H, self.edgemask[k], self.scale,
-                                  self.Z[k], self.norm[k])
+                                  self.Z[k], self.norm[k], width=self.w_out[k])
             Xu, Xi, act = self.Z[k], self.Z[k][g.U:], 1
         return self.Z[-1]
 
@@ -108,19 +118,25 @@ class Propagation:
             dev, N, E = self.g.device, self.g.N, self.g.E
             f32 = dict(dtype=torch.float32, device=dev)
             S = len(self.stages)
+            D = self.w_max        # G / Ghat / dh hold the widest stage; narrower stages use the leading N*w floats (_rows)
+            ws = max(ops.transform_bwd_workspace_bytes(self.g.U, self.g.I, a, b) for a, b in zip(self.w_in, self.w_out))
             # G / Ghat / dN start as zeros: the pruned output stage leaves the rows of inactive nodes untouched (stale, finite)
             self._bwd = dict(G=[torch.zeros((N, D), **f32), torch.zeros((N, D), **f32)], Ghat=torch.zeros((N, D), **f32),
                              dh=torch.empty((N, D), **f32), dN=torch.zeros((N, 8), **f32), dS=torch.empty((N, 8), **f32),
                              ds=torch.empty(max(E, 1) * 8, **f32),
-                             ws=torch.empty(ops.transform_bwd_workspace_bytes(self.g.U, self.g.I) // 4, **f32),
+                             ws=torch.empty(ws // 4, **f32),
                              # split mode: per-stage dh/dS (the deferred dW kernel of stage k reads them while stage k-1 is running)
                              dh_k=[torch.empty((N, D), **f32) for _ in range(S)], dS_k=[torch.empty((N, 8), **f32) for _ in range(S)],
                              ws_k=[torch.empty(ops.transform_bwd_dw_workspace_bytes(self.g.U, self.g.I) // 4 + 16, **f32) for _ in range(S)])
         return self._bwd
 
+    def _rows(self, buf, w):
+        """(N, w) view of the leading N*w floats of a (N, w_max) buffer (the buffer itself when w == w_max)"""
+        return buf if w == buf.shape[1] else buf.view(-1)[:self.g.N * w].view(self.g.N, w)
+
     def grad_in(self) -> torch.Tensor:
-        """(N,64) buffer the caller fills with dL/dZ_last (zero-filled by the caller as needed)."""
-        return self._bwd_buffers()["G"][0]
+        """(N, width of the last stage) buffer the caller fills with dL/dZ_last (zero-filled by the caller as needed)."""
+        return self._rows(self._bwd_buffers()["G"][0], self.w_out[-1])
 
     def backward(self, G_last: torch.Tensor, uEmbd, iEmbd, wtabs, gtabs, dU, dI, accumulate: bool, after_first_kernel=None,
                  before_grads=None, after_grads=None, dw_launcher=None, active=None):
@@ -136,13 +152,18 @@ class Propagation:
         b = self._bwd_buffers()
         G = G_last
         last = len(self.stages) - 1
+        wide = self.w_max != 64
+        if wide and (dw_launcher is not None or active is not None):
+            raise NotImplementedError("the split dense backward and the pruned output stage are built for 64-wide stages only")
         for k in range(last, -1, -1):
             H, _ = self.stages[k]
+            w, w_in = self.w_out[k], self.w_in[k]
             pruned = active is not None and k == last
             if pruned:
                 ops.stage_bwd_prep_active(g, G, self.Z[k], self.h[k], self.norm[k], H, b["Ghat"], b["dN"], active)
             else:
-                ops.stage_bwd_prep(G, self.Z[k], self.h[k], self.norm[k], H, b["Ghat"], b["dN"])
+                Ghat = self._rows(b["Ghat"], w)
+                ops.stage_bwd_prep(G, self.Z[k], self.h[k], self.norm[k], H, Ghat, b["dN"], width=w)
             if k == last and after_first_kernel is not None:
                 after_first_kernel()
             dh, dS = (b["dh_k"][k], b["dS_k"][k]) if dw_launcher is not None else (b["dh"], b["dS"])
@@ -151,8 +172,9 @@ class Propagation:
                     ops.stage_bwd_edges_active(mode, g, self.scratch, self.counter, G, b["Ghat"], b["dN"], self.h[k], self.s[k], H,
                                                self.edgemask[k], self.scale, wtabs[k], b["ds"], dh, dS, active)
                 else:
-                    ops.stage_bwd_edges(mode, g, self.scratch, self.counter, G, b["Ghat"], b["dN"], self.h[k], self.s[k], H,
-                                        self.edgemask[k], self.scale, wtabs[k], b["ds"], dh, dS)
+                    dh = self._rows(dh, w)
+                    ops.stage_bwd_edges(mode, g, self.scratch, self.counter, G, self._rows(b["Ghat"], w), b["dN"], self.h[k], self.s[k], H,
+                                        self.edgemask[k], self.scale, wtabs[k], b["ds"], dh, dS, width=w)
             if dw_launcher is not None:
                 Xu, Xi, act = (self.Z[k - 1], self.Z[k - 1][g.U:], 1) if k > 0 else (uEmbd, iEmbd, 0)
                 dw_launcher(k, lambda k=k, H=H, dh=dh, dS=dS, Xu=Xu, Xi=Xi, act=act: ops.transform_bwd_dw(
@@ -170,14 +192,16 @@ class Propagation:
                 continue
             if before_grads is not None:
                 before_grads(k)
+            dh = self._rows(b["dh"], w)
             if k > 0:
-                Gprev = b["G"][1] if G is not b["G"][1] else b["G"][0]
-                ops.transform_bwd(b["dh"], b["dS"], self.h[k], self.Z[k - 1], self.Z[k - 1][g.U:], 1, self.featmask[k], self.scale,
-                                  wtabs[k], gtabs[k], H, g.U, g.I, Gprev, Gprev[g.U:], 0, int(accumulate), b["ws"])
+                Gprev = b["G"][1] if G.data_ptr() != b["G"][1].data_ptr() else b["G"][0]
+                Gprev = self._rows(Gprev, w_in)
+                ops.transform_bwd(dh, b["dS"], self.h[k], self.Z[k - 1], self.Z[k - 1][g.U:], 1, self.featmask[k], self.scale,
+                                  wtabs[k], gtabs[k], H, g.U, g.I, Gprev, Gprev[g.U:], 0, int(accumulate), b["ws"], d_in=w_in, d_out=w)
                 G = Gprev
             else:
-                ops.transform_bwd(b["dh"], b["dS"], self.h[k], uEmbd, iEmbd, 0, self.featmask[k], self.scale, wtabs[k], gtabs[k],
-                                  H, g.U, g.I, dU, dI, int(accumulate), int(accumulate), b["ws"])
+                ops.transform_bwd(dh, b["dS"], self.h[k], uEmbd, iEmbd, 0, self.featmask[k], self.scale, wtabs[k], gtabs[k],
+                                  H, g.U, g.I, dU, dI, int(accumulate), int(accumulate), b["ws"], d_in=w_in, d_out=w)
             if after_grads is not None:
                 after_grads(k)
 

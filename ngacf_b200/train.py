@@ -34,6 +34,8 @@ class FusedTrainer:
         # False: one fused dX+dW+da kernel per stage (shares the tile loads; measured best: 1.22 ms/step at Gowalla shape).
         # True: dX on the chain, dW/da deferred to a third stream (1.24 ms/step: ~40% more dense work for a shorter chain).
         self.split_dense_backward = split_dense_backward
+        if split_dense_backward and getattr(model, "embedSize", 64) != 64:
+            raise NotImplementedError("the split dense backward (NGACF_SPLIT_DENSE_BWD=1) is built for embedSize 64 only")
         # captured steps: masks of step t+1 are generated next to Adam of step t (NGACF_PREFETCH_MASKS=0: at the head of the step)
         self.prefetch_masks = os.environ.get("NGACF_PREFETCH_MASKS", "1") != "0"
         # NGACF_STAGGER=1: the neg propagation starts one kernel after the pos one.  That paid while the dense kernels were long

@@ -135,6 +135,19 @@ def build_parser():
     return p
 
 
+def parse_args(argv=None):
+    """Parses the flags and refuses unsupported combinations (ValueError) before anything is initialised -- in particular before
+    --parallel True creates a process group."""
+    from ngacf_b200.ops import WIDTHS
+    args = build_parser().parse_args(argv)
+    if args.embedSize not in WIDTHS:
+        raise ValueError("--embedSize %d is not supported: the sm_100a kernels are built for embedSize %s"
+                         % (args.embedSize, " and ".join(map(str, WIDTHS))))
+    if args.parallel and args.embedSize != 64:
+        raise ValueError("--parallel True is built for --embedSize 64 only; train --embedSize %d on one GPU (--parallel False)" % args.embedSize)
+    return args
+
+
 def init_parallel(args):
     """--parallel True under torchrun: one process per GPU over NCCL (replaces the thread-per-GPU DataParallelModel of
     parallel.py:94-130; run_Gowalla.py:104-112).  Launch: torchrun --nproc_per_node=N run_Gowalla.py --parallel True ..."""
@@ -150,7 +163,7 @@ def init_parallel(args):
 
 
 if __name__ == "__main__":
-    args = build_parser().parse_args()
+    args = parse_args()
     print("----------------Parallel Mode is %s----------------" % ("enabled" if args.parallel else "disabled."))
     multi = init_parallel(args)
     torch.manual_seed(args.seed)
