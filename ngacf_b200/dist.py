@@ -9,9 +9,13 @@ Two multi-GPU modes, both replacing the reference's single-process thread-per-GP
   gradient is the SUM of the per-GPU mean-loss gradients (``loss.backward(ones(ndev))``).  Instead of
   broadcasting 18 MB of parameters before every forward and reduce-adding gradients to GPU 0
   (parallel.py:19,127-130), the replicas stay bit-identical: one NCCL all-reduce of the flat 18 MB gradient
-  buffer per step and the same Adam update everywhere.  Weak scaling.
+  buffer per step and the same Adam update everywhere.  Weak scaling.  ``NegSamplingReplicaTrainer`` does the
+  same for the NegSampling step (one propagation per GPU, the 1 + K items of its own rows).
+* ``ShardedTrainer`` / ``ShardedNegSamplingTrainer`` -- the propagation(s) of one step partitioned by user range
+  over the GPUs (below): the single-GPU step on the same batch.  Strong scaling.
 * ``shard_eval_users`` / ``allreduce_sums`` -- AllNeg evaluation shards the test users over the ranks;
-  only 16 metric sums (and optionally the top-20 lists) are merged.
+  only 16 metric sums (and optionally the top-20 lists) are merged; SampledNeg evaluation shards the test
+  rows and merges its two sums.
 
 The host-side pieces (row slicing, user sharding, flat-gradient all-reduce, metric merge) are plain
 functions so that the world_size-2 gloo tests in tests/test_dist_cpu.py exercise them without a GPU.
@@ -22,6 +26,7 @@ import torch
 import torch.distributed as dist
 
 from . import ops
+from .negsampling import NegSamplingTrainer
 from .train import FusedTrainer
 
 
@@ -75,14 +80,10 @@ def require_width_64(model):
                          % (model.embedSize, model.embedSize))
 
 
-class ReplicaTrainer(FusedTrainer):
-    """Data-parallel replicas of the fused step (see module docstring)."""
-
-    def __init__(self, model, inter, graph, batch_size, optim, sample_seed, use_cuda_graph=True, two_streams=True):
-        require_width_64(model)
-        self.rank, self.world = world_info()
-        super().__init__(model, inter, graph, batch_size, optim, sample_seed, use_cuda_graph, two_streams)
-        self.weak = True
+class _ReplicaHooks:
+    """The hooks of FusedTrainer._step_body / train_epoch that make a trainer one data-parallel replica: rank r scores the rows
+    [r*B, (r+1)*B) of every step of batch*world rows with its own dropout stream, and the flat gradient is summed over the ranks
+    between the two captured graphs.  Mixed in before a FusedTrainer subclass; self.rank / self.world are set before its __init__."""
 
     def _setup_params(self):
         m = self.model
@@ -114,11 +115,40 @@ class ReplicaTrainer(FusedTrainer):
         allreduce_sums(t)          # the reference adds the per-GPU losses (loss.sum(), train_eval_Gowalla.py:139)
         return float(t.item()) / n
 
+
+class ReplicaTrainer(_ReplicaHooks, FusedTrainer):
+    """Data-parallel replicas of the fused PairSampling step (see module docstring)."""
+
+    def __init__(self, model, inter, graph, batch_size, optim, sample_seed, use_cuda_graph=True, two_streams=True):
+        require_width_64(model)
+        self.rank, self.world = world_info()
+        super().__init__(model, inter, graph, batch_size, optim, sample_seed, use_cuda_graph, two_streams)
+        self.weak = True
+
     def units_per_step(self):
         return 2 * self.g.E * self.world
 
     def parallelism(self):
         return "dp%d replicas (reference --parallel semantics): batch %d x %d rows/step, one NCCL all-reduce of %.1f MB grads" % (
+            self.world, self.B, self.world, self.flat_grad.numel() * 4 / 2 ** 20)
+
+
+class NegSamplingReplicaTrainer(_ReplicaHooks, NegSamplingTrainer):
+    """Data-parallel replicas of the NegSampling step: every GPU propagates the whole graph once with its own dropout stream and
+    scores the 1 + K items of its own batch_size train rows; the gradients are summed (the reference's --parallel True in
+    train_neg_sample).  The tail step of len % (batch*world) rows is trained, a rank without rows joins with a zero gradient."""
+
+    def __init__(self, model, inter, graph, batch_size, optim, sample_seed, K=4, use_cuda_graph=True):
+        require_width_64(model)
+        self.rank, self.world = world_info()
+        super().__init__(model, inter, graph, batch_size, optim, sample_seed, K=K, use_cuda_graph=use_cuda_graph)
+        self.weak = True
+
+    def units_per_step(self):
+        return self.g.E * self.world
+
+    def parallelism(self):
+        return "dp%d NegSampling replicas (reference --parallel semantics): batch %d x %d rows/step, one NCCL all-reduce of %.1f MB grads" % (
             self.world, self.B, self.world, self.flat_grad.numel() * 4 / 2 ** 20)
 
 
@@ -354,7 +384,7 @@ class LocalCluster:
             if read_loss:
                 losses.append(float(self.trainers[0].loss.item()))
         for tr in self.trainers:
-            tr.model._call += 2 * n_steps
+            tr.model._call += tr.CALLS_PER_STEP * n_steps
         return losses
 
     def gather_state(self):
@@ -397,11 +427,17 @@ class ShardedTrainer:
     step -- kernels and NCCL calls -- is captured in ONE CUDA graph; if the capture of the collectives is refused, the compute
     phases are captured separately and the collectives run eagerly between them (the round-1 structure)."""
 
+    CALLS_PER_STEP = 2          # dropout call indices per step = propagations per step (pos, neg)
+    PRUNABLE = True             # the output stage may be pruned to the batch rows when a rank holds a whole propagation (G == 1)
+    PROP_PARALLEL = None        # layout of Topology (None: NGACF_DIST_PROP_PARALLEL decides)
+
     def __init__(self, model, inter, edge_u, edge_i, batch_size, optim, sample_seed, use_cuda_graph=True, transport=None, rank=None, world=None,
                  plan=None, prop_parallel=None):
         from .graph import BipartiteGraph
         from .propagation import Propagation
         require_width_64(model)
+        if prop_parallel is None:
+            prop_parallel = self.PROP_PARALLEL
         if transport is None:
             r0, w0 = world_info()
             self.topo = Topology(r0, w0, prop_parallel)
@@ -439,7 +475,7 @@ class ShardedTrainer:
         def rows(w):
             return torch.zeros((N_alloc, w), **f32)
         self.props = []
-        for _ in range(2):       # pos / neg
+        for _ in range(self.CALLS_PER_STEP):       # one propagation per dropout call: pos / neg
             p = Propagation.__new__(Propagation)
             p.g, p.stages = g, self.stages
             p.h = [rows(ops.D) for _ in self.stages]
@@ -459,11 +495,7 @@ class ShardedTrainer:
             p.em = [torch.zeros(max(P.E, 1), dtype=torch.uint8, device=dev) for _ in self.stages]      # indexed by GLOBAL edge id
             p.featmask, p.edgemask, p.scale = [None] * S, [None] * S, 1.0
             self.props.append(p)
-        self.Zb = torch.zeros((2, 2 * self.B, ops.D), **f32)           # compact batch rows of both propagations (one all-reduce)
-        self.users, self.pos, self.neg = torch.zeros(self.B, **i64), torch.zeros(self.B, **i64), torch.zeros(self.B, **i64)
-        self.sc_all = torch.zeros((2, self.B), **f32)          # pair scores of both propagations (exchanged as scores when G == 1)
-        self.sc = [self.sc_all[0], self.sc_all[1]]
-        self.dsc = [torch.zeros(self.B, **f32), torch.zeros(self.B, **f32)]
+        self._batch_buffers(f32, i64)
         self.loss = torch.zeros((), **f32)
         self.total = torch.zeros((), dtype=torch.float64, device=dev)
         self.row_dev = torch.zeros(2, **i64)
@@ -473,7 +505,7 @@ class ShardedTrainer:
         # pruned to the batch rows exactly as in the single-GPU trainer (csrc/pruned_stage.cu)
         import os
         self.complete = self.topo.G == 1
-        self.prune = self.complete and os.environ.get("NGACF_PRUNE", "1") != "0" and self.stages[-1][0] == 1
+        self.prune = self.complete and self.PRUNABLE and os.environ.get("NGACF_PRUNE", "1") != "0" and self.stages[-1][0] == 1
         self.active = {q: ops.ActiveRows(g) for q in self.topo.props} if self.prune else {}
         # parameters: embedding gradients stay with the owner of the row; the attention parameters are replicated and their
         # gradients (partial sums over the own rows) are summed by one small all-reduce
@@ -520,6 +552,70 @@ class ShardedTrainer:
         self.capture_mode = None
 
     # ------------------------------------------------------------------------------------------
+    # the PairSampling-specific parts of the step (ShardedNegSamplingTrainer overrides them)
+    def _batch_buffers(self, f32, i64):
+        self.Zb = torch.zeros((2, 2 * self.B, ops.D), **f32)           # compact batch rows of both propagations (one all-reduce)
+        self.users, self.pos, self.neg = torch.zeros(self.B, **i64), torch.zeros(self.B, **i64), torch.zeros(self.B, **i64)
+        self.sc_all = torch.zeros((2, self.B), **f32)          # pair scores of both propagations (exchanged as scores when G == 1)
+        self.sc = [self.sc_all[0], self.sc_all[1]]
+        self.dsc = [torch.zeros(self.B, **f32), torch.zeros(self.B, **f32)]
+
+    def _mine(self):
+        """the propagations this rank runs: [0, 1], or [q] in the propagation-parallel layout"""
+        return list(self.topo.props)
+
+    def _sample(self):
+        ops.sample_pairs(self.inter, 0, self.B, self.sample_seed, 0, self.users, self.pos, self.neg, self.row_dev)
+        if self.prune:      # active rows of propagation q: stamped with its dropout call index (as in train.FusedTrainer)
+            for q in self._mine():
+                self.active[q].at(q, self.call_dev).mark(self.users, (self.pos, self.neg)[q])
+
+    def _output_rows(self, q, Z):
+        """end of the last stage of propagation q (Z: its output rows, complete for the own rows)"""
+        item = (self.pos, self.neg)[q]
+        if self.complete:      # every row is local: score the own propagation's pairs here, exchange SCORES instead of rows
+            ops.score_pairs(Z, self.U, self.users, item, self.sc[q])
+        else:
+            ops.batch_rows_gather(Z, self.U, self.users, item, (self.u_lo, self.u_hi), (self.i_lo, self.i_hi), self.Zb[q])
+
+    def _loss_phases(self, both, zero_own):
+        """the phases from the exchange of the batch rows (or scores) to the gradient rows G of the last stage"""
+        U, S, mine = self.U, len(self.stages), self._mine()
+        items = (self.pos, self.neg)
+        plan = []
+        if self.complete:
+            other = 1 - mine[0]
+            plan.append(("k", "zero the other propagation's scores", lambda: ops.memset_zero(self.sc[other])))
+            plan.append(("c", "all-reduce pair scores", "ar", [self.sc_all], "world"))
+        else:
+            if len(mine) == 1:
+                other = 1 - mine[0]
+                plan.append(("k", "zero the other propagation's batch rows", lambda: ops.memset_zero(self.Zb[other])))
+            plan.append(("c", "all-reduce batch rows", "ar", [self.Zb], "world"))
+
+        def score(q):
+            p = self.props[q]
+            ops.batch_rows_scatter(self.Zb[q], U, self.users, items[q], p.ZS)
+            ops.score_pairs(p.ZS, U, self.users, items[q], self.sc[q])
+
+        def loss_and_scatter():
+            if not self.complete:
+                both(score, [0, 1])()           # every rank scores both propagations' pairs (the loss needs both)
+            ops.bpr_loss(self.sc[0], self.sc[1], 1.0, self.loss, self.dsc[0], self.dsc[1])
+
+            def scatter(q):
+                p = self.props[q]
+                G = p.G[0]
+                if not self.prune:      # pruned: the scatter writes exactly the active rows, nothing else of G is read
+                    zero_own(G)
+                # rows of other owners are written and never read
+                ops.score_pairs_bwd(p.Z[S - 1] if self.complete else p.ZS, U, self.users, items[q], self.dsc[q], G)
+            both(scatter)()
+            ops.memset_zero(self.flat_small)        # attention-parameter gradients are accumulated by every dense backward
+        plan.append(("k", "scores+loss+scatter", loss_and_scatter))
+        return plan
+
+    # ------------------------------------------------------------------------------------------
     def _items_view(self, t):
         return t[self.U:]                        # (I_pad, w): the item rows of a per-node buffer
 
@@ -536,14 +632,13 @@ class ShardedTrainer:
         nu, ni = uhi - ulo, ihi - ilo
         uE, iE = m.uEmbd.weight.detach(), m.iEmbd.weight.detach()
         dU, dI = m.uEmbd.weight.grad, m.iEmbd.weight.grad
-        items = (self.pos, self.neg)
         side = self.side
         S = len(self.stages)
         heads = [H for H, _ in self.stages]
         scale = 1.0 / (1.0 - droprate) if droprate > 0 else 1.0
         plan = []
 
-        mine = list(self.topo.props)            # the propagations this rank runs: [0, 1], or [q] in the propagation-parallel layout
+        mine = self._mine()
 
         def both(fn, props=None):
             """fn(q) for each propagation of this rank: the first on the current stream, the second on the side stream"""
@@ -562,13 +657,7 @@ class ShardedTrainer:
             return run
 
         complete, prune = self.complete, self.prune
-
-        def head():
-            ops.sample_pairs(self.inter, 0, B, self.sample_seed, 0, self.users, self.pos, self.neg, self.row_dev)
-            for q in mine:
-                if prune:      # active rows of propagation q: stamped with its dropout call index (as in train.FusedTrainer)
-                    self.active[q].at(q, self.call_dev).mark(self.users, items[q])
-        plan.append(("k", "sample", head))
+        plan.append(("k", "sample", self._sample))
 
         def masks(k):
             p = self.props[k]
@@ -579,7 +668,7 @@ class ShardedTrainer:
             ops.dropout_masks_ranges(p.fm, p.em, heads, ((ulo, uhi), (U + ilo, U + ihi)), (self.e_lo, self.e_hi), seed, k, droprate, self.call_dev)
             p.featmask = list(p.fm)
             p.edgemask = [e[self.e_lo:] for e in p.em]          # local edge id + e_lo = global edge id
-        for k in (0, 1):
+        for k in range(len(self.props)):
             masks(k) if droprate <= 0 else None
         if droprate > 0:
             plan.append(("k", "masks", both(masks)))
@@ -618,45 +707,15 @@ class ShardedTrainer:
                 if ni and not complete:
                     ops.aggregate_finalize(p.Z[k][U + ilo:U + ihi], p.h[k][U + ilo:U + ihi], p.norm[k][U + ilo:U + ihi], H)
                 if k == S - 1:
-                    if complete:      # every row is local: score the own propagation's pairs here, exchange SCORES instead of rows
-                        ops.score_pairs(p.Z[k], U, self.users, items[q], self.sc[q])
-                    else:
-                        ops.batch_rows_gather(p.Z[k], U, self.users, items[q], (ulo, uhi), (ilo, ihi), self.Zb[q])
+                    self._output_rows(q, p.Z[k])
             plan.append(("k", "finalize%d" % k, both(finalize)))
 
-        if complete:
-            other = 1 - mine[0]
-            plan.append(("k", "zero the other propagation's scores", lambda: ops.memset_zero(self.sc[other])))
-            plan.append(("c", "all-reduce pair scores", "ar", [self.sc_all], "world"))
-        else:
-            if len(mine) == 1:
-                other = 1 - mine[0]
-                plan.append(("k", "zero the other propagation's batch rows", lambda: ops.memset_zero(self.Zb[other])))
-            plan.append(("c", "all-reduce batch rows", "ar", [self.Zb], "world"))
-
-        def score(q):
-            p = self.props[q]
-            ops.batch_rows_scatter(self.Zb[q], U, self.users, items[q], p.ZS)
-            ops.score_pairs(p.ZS, U, self.users, items[q], self.sc[q])
-
-        def loss_and_scatter():
-            if not complete:
-                both(score, [0, 1])()           # every rank scores both propagations' pairs (the loss needs both)
-            ops.bpr_loss(self.sc[0], self.sc[1], 1.0, self.loss, self.dsc[0], self.dsc[1])
-
-            def scatter(q):
-                p = self.props[q]
-                G = p.G[0]
-                if not prune:      # pruned: the scatter writes exactly the active rows, nothing else of G is read
-                    if nu:
-                        ops.memset_zero(G[ulo:uhi])
-                    if ni:
-                        ops.memset_zero(G[U + ilo:U + ihi])
-                # rows of other owners are written and never read
-                ops.score_pairs_bwd(p.Z[S - 1] if complete else p.ZS, U, self.users, items[q], self.dsc[q], G)
-            both(scatter)()
-            ops.memset_zero(self.flat_small)        # attention-parameter gradients are accumulated by every dense backward
-        plan.append(("k", "scores+loss+scatter", loss_and_scatter))
+        def zero_own(G):
+            if nu:
+                ops.memset_zero(G[ulo:uhi])
+            if ni:
+                ops.memset_zero(G[U + ilo:U + ihi])
+        plan += self._loss_phases(both, zero_own)
 
         evs = [torch.cuda.Event() for _ in range(S)]
         for k in range(S - 1, -1, -1):
@@ -748,7 +807,7 @@ class ShardedTrainer:
             h = self.hyper
             ops.adam_step_dev(self.adam_tab, len(self._adam_entries), self.adam_total, h["lr"], h["b1"], h["b2"], h["eps"], h["wd"], self.adam_state)
             ops.step_counters(self.total, self.loss, self.row_dev, B)
-            ops.counter_add(self.call_dev, 2)
+            ops.counter_add(self.call_dev, self.CALLS_PER_STEP)
         plan.append(("k", "adam", update))
         return plan
 
@@ -878,7 +937,7 @@ class ShardedTrainer:
             self._end_step()
             if read_loss:
                 losses.append(float(self.loss.item()))
-        m._call += 2 * n_steps
+        m._call += self.CALLS_PER_STEP * n_steps
         return losses
 
     def train_epoch(self, epoch: int = 0, max_steps=None) -> float:
@@ -950,18 +1009,91 @@ class ShardedTrainer:
         return 1 + 2 * per_prop + 1 + 2 + 2
 
     def units_per_step(self):
-        return 2 * self.plan.E           # strong scaling: the same global step on every world size
+        return len(self.props) * self.plan.E           # strong scaling: the same global step on every world size
+
+    def _layout(self):
+        return ("2 groups of %d GPUs (group q runs propagation q)" % self.topo.G) if self.topo.prop_parallel else "both propagations on every GPU"
 
     def parallelism(self):
-        lay = ("2 groups of %d GPUs (group q runs propagation q)" % self.topo.G) if self.topo.prop_parallel else "both propagations on every GPU"
         return ("%d GPUs: %s; users range-partitioned over %d ranks by edge count (rank %d: users [%d,%d), %d of %d edges), item rows owned by "
                 "range (%d per rank); per stage: all-gather of the item rows, reduce-scatter of the item partials; %s" % (
-                    self.world, lay, self.topo.G, self.rank, self.u_lo, self.u_hi, self.e_hi - self.e_lo, self.plan.E, self.plan.chunk,
+                    self.world, self._layout(), self.topo.G, self.rank, self.u_lo, self.u_hi, self.e_hi - self.e_lo, self.plan.E, self.plan.chunk,
                     self.capture_mode))
 
     def working_set_bytes(self):
         N = self.U + self.plan.I_pad
-        return 2 * (9 * N * 256 + 8 * (self.e_hi - self.e_lo) * 4) + 7 * self.adam_total * 4
+        return len(self.props) * (9 * N * 256 + 8 * (self.e_hi - self.e_lo) * 4) + 7 * self.adam_total * 4
 
     def profile_kernels(self, n_steps=3):
         return []
+
+
+class ShardedNegSamplingTrainer(ShardedTrainer):
+    """NegSampling step (negsampling.NegSamplingTrainer) with its ONE propagation partitioned by user range over all `world` ranks
+    (one group, G = world: no propagation-parallel layout, no sub-groups).  Same maths as the single-GPU step on the same batch:
+
+      batch         : every rank samples the same b train rows x (1 positive + K negatives), column-major (column j = pairs
+                      [j*b, (j+1)*b));
+      stages        : as in ShardedTrainer, for one propagation (dropout call offset 0, one call index per step);
+      pair scores   : the (K+1)*b pairs' rows are gathered into a compact table (a user row appears K+1 times; every copy is
+                      the same row) and summed by one all-reduce; scores, BCE and dscore are computed redundantly, and the
+                      gradient rows are scattered one column at a time (accumulating), as on one GPU;
+      backward and update as in ShardedTrainer.
+
+    As in the PairSampling partition, the tail batch of len % batch rows is dropped."""
+
+    CALLS_PER_STEP = 1
+    PRUNABLE = False            # a pruned NegSampling output stage is not built
+    PROP_PARALLEL = False       # one propagation: one group of `world` ranks
+
+    def __init__(self, model, inter, edge_u, edge_i, batch_size, optim, sample_seed, K=4, use_cuda_graph=True, transport=None, rank=None,
+                 world=None, plan=None):
+        self.K = int(K)
+        if inter.min_negatives() < self.K:      # random.sample(negative_items, K) raises in the reference (loadGowalla.py:82)
+            raise ValueError("a user has fewer than K=%d negatives (item pool minus the user's positives)" % self.K)
+        super().__init__(model, inter, edge_u, edge_i, batch_size, optim, sample_seed, use_cuda_graph=use_cuda_graph, transport=transport,
+                         rank=rank, world=world, plan=plan)
+
+    def _batch_buffers(self, f32, i64):
+        n = self.B * (self.K + 1)
+        self.pu, self.pi = torch.zeros(n, **i64), torch.zeros(n, **i64)
+        self.Zb = torch.zeros((2 * n, ops.D), **f32)          # compact rows of the n users, then of the n items
+        self.sc, self.dsc = torch.zeros(n, **f32), torch.zeros(n, **f32)
+
+    def _mine(self):
+        return [0]
+
+    def _sample(self):
+        it = self.inter
+        ops.sample_negs(it, it.train_rows_user, it.train_rows_item, 0, self.B, self.sample_seed, 0, self.K, ops.NEG_TAG_TRAIN, self.pu, self.pi,
+                        self.row_dev, col_stride=self.B)
+
+    def _output_rows(self, q, Z):
+        ops.batch_rows_gather(Z, self.U, self.pu, self.pi, (self.u_lo, self.u_hi), (self.i_lo, self.i_hi), self.Zb)
+
+    def _loss_phases(self, both, zero_own):
+        U, b, p = self.U, self.B, self.props[0]
+
+        def loss_and_scatter():
+            ops.batch_rows_scatter(self.Zb, U, self.pu, self.pi, p.ZS)
+            ops.score_pairs(p.ZS, U, self.pu, self.pi, self.sc)
+            ops.bce_logits_loss(self.sc, -b, self.loss, self.dsc)
+            G = p.G[0]
+            zero_own(G)
+            # one column of b pairs at a time, accumulating (negsampling.NegSamplingTrainer._step_body); rows of other owners are
+            # written and never read
+            for j in range(self.K + 1):
+                sl = slice(j * b, (j + 1) * b)
+                ops.score_pairs_bwd(p.ZS, U, self.pu[sl], self.pi[sl], self.dsc[sl], G, accumulate=j > 0)
+            ops.memset_zero(self.flat_small)        # attention-parameter gradients are accumulated by every dense backward
+        return [("c", "all-reduce batch rows", "ar", [self.Zb], "world"),
+                ("k", "scores+loss+scatter", loss_and_scatter)]
+
+    def launches_per_step(self, droprate):
+        S = len(self.stages)
+        fwd = (1 if droprate > 0 else 0) + S * (2 + 1 + 1) + 1            # masks, per stage transform x2 + aggregate + finalize, gather
+        loss = 2 + 1 + 2 + (self.K + 1) + 1                                # rows scatter + scores, BCE, zero G x2, scatter per column, zero grads
+        return 1 + fwd + loss + S * (2 + 2 + 1 + 4) + 2 + 2               # sampler, ..., backward per stage, adam(2), counters(2)
+
+    def _layout(self):
+        return "one propagation over all GPUs"

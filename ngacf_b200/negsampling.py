@@ -83,28 +83,41 @@ class NegSamplingTrainer(FusedTrainer):
 
 class SampledNegEvaluator:
     """eval_neg_sample (train_eval_Gowalla.py:193-257): HR@top_k / NDCG@top_k over 1 positive + K sampled negatives per test row,
-    all rows scored against ONE propagation (the reference re-propagates for every batch of batch_size//8 rows)."""
+    all rows scored against ONE propagation (the reference re-propagates for every batch of batch_size//8 rows).
 
-    def __init__(self, inter: Interactions, top_k: int = 10, K: int = 99, seed: int = 0):
+    rows = (lo, hi) evaluates the test rows [lo, hi) only (one rank's shard): the sampler is keyed by the test row, so a shard draws
+    exactly the negatives of the whole evaluation, and the metric sums of the shards add up to those of the whole."""
+
+    def __init__(self, inter: Interactions, top_k: int = 10, K: int = 99, seed: int = 0, rows=None):
         self.inter, self.top_k, self.K, self.seed = inter, int(top_k), int(K), int(seed)
         if inter.n_test_rows and inter.min_negatives() < self.K:      # loadGowalla.py:103
             raise ValueError("a user has fewer than K=%d negatives (item pool minus the user's positives)" % self.K)
-        n = inter.n_test_rows * (self.K + 1)
+        self.rows = (0, inter.n_test_rows) if rows is None else (int(rows[0]), int(rows[1]))
+        if not 0 <= self.rows[0] <= self.rows[1] <= inter.n_test_rows:
+            raise ValueError("test rows [%d, %d) outside [0, %d)" % (self.rows + (inter.n_test_rows,)))
+        n = (self.rows[1] - self.rows[0]) * (self.K + 1)
         dev = inter.device
         self.pu = torch.zeros(n, dtype=torch.int64, device=dev)
         self.pi = torch.zeros(n, dtype=torch.int64, device=dev)
         self.sc = torch.zeros(n, dtype=torch.float32, device=dev)
         self.sums = torch.zeros(2, dtype=torch.float64, device=dev)
 
-    def __call__(self, Z: torch.Tensor):
-        """Z: pre-ELU output of the last stage (model.propagate in eval mode).  Returns (HR, NDCG) as python floats."""
+    def metric_sums(self, Z: torch.Tensor) -> torch.Tensor:
+        """float64[2] on the device: the sums of HR@top_k and NDCG@top_k over the evaluated rows"""
         it = self.inter
-        rows = it.n_test_rows
+        lo, hi = self.rows
+        self.sums.zero_()
+        if hi > lo:
+            ops.sample_negs(it, it.test_rows_user, it.test_rows_item, lo, hi, self.seed, 0, self.K, ops.NEG_TAG_EVAL, self.pu, self.pi)
+            ops.score_pairs(Z, it.U, self.pu, self.pi, self.sc)
+            ops.rank_metrics(self.sc, self.K + 1, self.top_k, self.sums)
+        return self.sums
+
+    def __call__(self, Z: torch.Tensor):
+        """Z: pre-ELU output of the last stage (model.propagate in eval mode).  Returns (HR, NDCG) as python floats, averaged over
+        all test rows (a shard's sums divided by the total count: add the shards' results to get the whole)."""
+        rows = self.inter.n_test_rows
         if rows == 0:
             return 0.0, 0.0
-        ops.sample_negs(it, it.test_rows_user, it.test_rows_item, 0, rows, self.seed, 0, self.K, ops.NEG_TAG_EVAL, self.pu, self.pi)
-        ops.score_pairs(Z, it.U, self.pu, self.pi, self.sc)
-        self.sums.zero_()
-        ops.rank_metrics(self.sc, self.K + 1, self.top_k, self.sums)
-        hr, nd = (self.sums / rows).tolist()
+        hr, nd = (self.metric_sums(Z) / rows).tolist()
         return hr, nd

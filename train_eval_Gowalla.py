@@ -218,15 +218,16 @@ def train_neg_sample(model, batch_size, train_df, train_pos_neg, adj, optim, los
     """One epoch of train_neg_sample (train_eval_Gowalla.py:36-88): per train row 1 positive + 4 sampled negatives, ONE propagation per
     batch, BCEWithLogitsLoss on the B*5 scores, backward, optimizer step.  Returns sum(batch-mean loss) / len(train_df) (:84,88).
     train_pos_neg = positives_negtives(rt) (or an ngacf_b200.data.Interactions); `epoch`/`sample_seed` select the sampler's stream."""
-    if is_parallel:
-        raise NotImplementedError("--parallel True is replaced by one process per GPU (ngacf_b200/dist.py)")
     m = _unwrap(model)
     model.train()
     inter = _neg_interactions(model, train_pos_neg, train_df=train_df)
     dev = m.uEmbd.weight.device
-    graph = m.graph_for(_device_adj(model, adj))
     if sample_seed is None:
         sample_seed = int(torch.initial_seed()) & 0xFFFFFFFFFFFFFFFF
+    if is_parallel and _world() > 1:
+        return _train_neg_parallel(m, batch_size, inter, adj, optim, lossfn, epoch, sample_seed, max_steps)
+    # a lone --parallel True process runs the one-GPU step (see train_bpr)
+    graph = m.graph_for(_device_adj(model, adj))
     if fused is None:
         fused = os.environ.get("NGACF_FUSED", "1") != "0"
     K = 4
@@ -263,19 +264,56 @@ def train_neg_sample(model, batch_size, train_df, train_pos_neg, adj, optim, los
     return float(total.item()) / n
 
 
+def _train_neg_parallel(m, batch_size, inter, adj, optim, lossfn, epoch, sample_seed, max_steps):
+    """--parallel True under torchrun for NegSampling, NGACF_PARALLEL_MODE as in _train_bpr_parallel:
+      shard   (default) the one propagation user-range partitioned over all GPUs (ngacf_b200.dist.ShardedNegSamplingTrainer): the SAME
+              step as one GPU on the same batch, split over the GPUs (the tail batch of len % batch rows is dropped);
+      replica the reference's semantics: every GPU propagates the whole graph and scores the 1 + 4 items of its own batch_size rows,
+              gradients are summed (ngacf_b200.dist.NegSamplingReplicaTrainer)."""
+    from ngacf_b200.dist import NegSamplingReplicaTrainer, ShardedNegSamplingTrainer
+    if not _fused_ok(m, optim, lossfn, loss_type=torch.nn.BCEWithLogitsLoss):
+        raise NotImplementedError("--parallel True needs the fused step: SPUIGACF + BCEWithLogitsLoss (mean) + a single-group Adam over "
+                                  "model.parameters()")
+    mode = os.environ.get("NGACF_PARALLEL_MODE", "shard")
+    tr = getattr(m, "_neg_parallel_trainer", None)
+    key = (mode, id(inter), id(adj), int(batch_size), id(optim), int(sample_seed))
+    if tr is None or tr.key != key:
+        if mode == "replica":
+            tr = NegSamplingReplicaTrainer(m, inter, m.graph_for(_device_adj(m, adj)), batch_size, optim, sample_seed)
+        else:
+            idx = np.asarray(adj.cpu() if torch.is_tensor(adj) else adj).reshape(2, -1)
+            tr = ShardedNegSamplingTrainer(m, inter, idx[0], idx[1], batch_size, optim, sample_seed)
+        tr.key = key
+        m._neg_parallel_trainer = tr
+    return tr.train_epoch(epoch, max_steps)
+
+
 def eval_neg_sample(model, batch_size, test_df, test_pos_neg, adj, top_k, is_parallel, seed=0):
     """eval_neg_sample (train_eval_Gowalla.py:193-257): per test row 1 positive + 99 sampled negatives, HR@top_k and NDCG@top_k
-    averaged over the test rows.  All rows are scored against one propagation.  Returns (HR, NDCG)."""
+    averaged over the test rows.  All rows are scored against one propagation.  Returns (HR, NDCG).
+    is_parallel under torchrun: every rank evaluates its shard of the test rows, the two metric sums are merged, and every rank
+    returns the same (HR, NDCG)."""
     m = _unwrap(model)
     model.eval()
     _require_plain(m, "eval_neg_sample")
     inter = _neg_interactions(model, test_pos_neg, test_df=test_df)
     adj_t = _device_adj(model, adj)
     from ngacf_b200.negsampling import SampledNegEvaluator
+    world = _world() if is_parallel else 1
+    rows = None
+    if world > 1:
+        import torch.distributed as dist
+        from ngacf_b200.dist import shard_range
+        rows = shard_range(inter.n_test_rows, dist.get_rank(), world)
     with torch.no_grad():
         Z = m.propagate(adj_t)
         ev = getattr(m, "_neg_evaluator", None)
-        if ev is None or ev.inter is not inter or ev.top_k != int(top_k) or ev.seed != int(seed):
-            ev = SampledNegEvaluator(inter, top_k, 99, seed)
+        if ev is None or ev.inter is not inter or ev.top_k != int(top_k) or ev.seed != int(seed) or ev.rows != (rows or (0, inter.n_test_rows)):
+            ev = SampledNegEvaluator(inter, top_k, 99, seed, rows=rows)
             m._neg_evaluator = ev
-        return ev(Z)
+        if world == 1:
+            return ev(Z)
+        from ngacf_b200.dist import allreduce_sums
+        sums = allreduce_sums(ev.metric_sums(Z))
+        hr, nd = (sums / max(inter.n_test_rows, 1)).tolist()
+        return hr, nd
