@@ -392,6 +392,27 @@ int ngacf_score_topk_exact_split_w(const float* F, int32_t width, int32_t U, int
                                    const int32_t* train_ptr, const int32_t* train_items, const uint8_t* in_pool, int32_t* top_ids,
                                    float* top_scores, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Top-K recommendation lists for any users (K = 1 .. NGACF_RECOMMEND_MAX_K).  F: (U+I, width) final features (ELU applied, as
+ * ngacf_final_features(_w) writes them), width 64 or 128.  The score of (u, i) is F[u] . F[U+i] with products rounded to fp32 and
+ * summed by the adjacent-pair tree of ngacf_score_topk_exact(_w), so the scores are the bits of the AllNeg ranking.
+ *   candidates: items with in_pool[i] != 0 (in_pool NULL: every item) minus the user's excluded items, given as a CSR over users
+ *               (excl_ptr[U+1], excl_items ascending per user; both NULL: nothing is excluded).
+ *   order:      score descending, then item id ascending.  Row r of top_ids / top_scores ([n_users][K]) is users[r]'s list; a row
+ *               with fewer than K candidates is padded with id -1 / score 0.0, and so is the whole row of a user id outside [0, U)
+ *               (nothing of it is read).  Duplicated users get identical rows; a row does not depend on the other users of the call.
+ *   workspace:  ngacf_recommend_topk_workspace_bytes(width, I, n_users, K) bytes (0 when there are enough users to rank every item
+ *               range in one pass; few users split the item range and merge partial lists there).  A smaller workspace returns
+ *               NGACF_ERR_WORKSPACE; nothing beyond the reported size is written.
+ * Width other than 64 / 128 or K outside 1 .. NGACF_RECOMMEND_MAX_K returns NGACF_ERR_UNSUPPORTED.  Deterministic; no allocation, no
+ * synchronisation (CUDA-graph capturable).  n_users == 0 is a no-op.
+ * ------------------------------------------------------------------------------------------- */
+#define NGACF_RECOMMEND_MAX_K 100
+size_t ngacf_recommend_topk_workspace_bytes(int32_t width, int32_t I, int32_t n_users, int32_t K);
+int ngacf_recommend_topk(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users, int32_t K,
+                         const int32_t* excl_ptr, const int32_t* excl_items, const uint8_t* in_pool, int32_t* top_ids,
+                         float* top_scores, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

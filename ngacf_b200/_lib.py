@@ -83,6 +83,9 @@ SIGNATURES = {
     "ngacf_final_features_w": (c_int32, [P, c_int64, c_int32, P, P]),
     "ngacf_score_topk_exact_w": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, P, P, P, P, P, P]),
     "ngacf_score_topk_exact_split_w": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, P, P, P, P, P, P, c_size_t, P]),
+    # top-K recommendation lists
+    "ngacf_recommend_topk_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "ngacf_recommend_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, P, P, c_size_t, P]),
 }
 
 _lib = None

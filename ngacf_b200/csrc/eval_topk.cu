@@ -4,7 +4,7 @@
 // Replaces train_eval_Gowalla.py:300-341 (64x2048 tiles through model(), D2H per tile),
 // :370-385 (heapq.nlargest over a dict per user), :419-429 + metrics.py:10-86.
 #include <cmath>
-#include "common.cuh"
+#include "topk_common.cuh"
 
 namespace ngacf {
 
@@ -16,24 +16,6 @@ template <int W> __host__ __device__ constexpr size_t ex_smem() {
     return (size_t)(W * EX_ITEMS + EX_USERS * W) * 4 + (size_t)EX_THREADS * K * 8 + EX_USERS * 8 + EX_ITEMS + 64;
 }
 constexpr size_t EX_SMEM = ex_smem<64>();
-
-// order: score descending, item id ascending
-__device__ __forceinline__ bool better(float s1, int i1, float s2, int i2) { return s1 > s2 || (s1 == s2 && i1 < i2); }
-
-// 2^L-term adjacent-pair tree evaluated incrementally: `add(d, v)` with d compile-time after unrolling (L = 6: 64-wide rows,
-// L = 7: 128-wide rows); the total ends in st[L-1]
-template <int L>
-struct TreeN {
-    float st[L];
-    __device__ __forceinline__ void add(int d, float v) {
-#pragma unroll
-        for (int l = 0; l < L; ++l) {
-            if (((d >> l) & 1) == 0) { st[l] = v; return; }
-            v = __fadd_rn(st[l], v);
-        }
-        st[L - 1] = v;   // d == 2^L - 1: v is the total (kept in st[L-1])
-    }
-};
 
 template <int W = 64>
 __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const float* __restrict__ F, int U, int I, const int* __restrict__ users,
@@ -78,14 +60,7 @@ __global__ void __launch_bounds__(EX_THREADS) score_topk_exact_kernel(const floa
 
     for (int i0 = i_begin; i0 < i_end; i0 += EX_ITEMS) {
         __syncthreads();
-        // item tile, transposed: It[d][j] = F[U+i0+j][d]
-        for (int idx = tid; idx < EX_ITEMS * (W / 4); idx += EX_THREADS) {
-            int j = idx / (W / 4), q = idx % (W / 4);
-            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (i0 + j < I) v = ld_gather4(F + (int64_t)(U + i0 + j) * W + q * 4);
-            It[(q * 4 + 0) * EX_ITEMS + j] = v.x; It[(q * 4 + 1) * EX_ITEMS + j] = v.y;
-            It[(q * 4 + 2) * EX_ITEMS + j] = v.z; It[(q * 4 + 3) * EX_ITEMS + j] = v.w;
-        }
+        NGACF_LOAD_ITEM_TILE(W, EX_ITEMS, EX_THREADS, It, F, U, I, i0, tid);     // It[d][j] = F[U+i0+j][d]
         if (tid < EX_ITEMS) Pool[tid] = (i0 + tid < I) ? in_pool[i0 + tid] : 0;
         if (il == 0) {      // train positives of this user inside the tile (sorted list, monotone cursor)
             unsigned long long m = 0ull;

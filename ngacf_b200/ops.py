@@ -302,6 +302,17 @@ def score_topk_tc(F, U, I, users, inter, top_ids, top_scores, fallback, ws, reus
               _p(inter.in_pool), _p(top_ids), _p(top_scores), _p(fallback), int(bool(reuse_mask)), _p(ws), ws.numel() * ws.element_size(), _s())
 
 
+def recommend_topk_workspace_bytes(width, I, n_users, K):
+    return int(_lib.load().ngacf_recommend_topk_workspace_bytes(int(width), int(I), int(n_users), int(K)))
+
+
+def recommend_topk(F, U, I, users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, ws):
+    """top-K lists of `users` (int32) from final features F (U+I, 64 or 128); excl_ptr/excl_items (CSR over users) and in_pool may be
+    None; ws: uint8 tensor of recommend_topk_workspace_bytes(...) bytes (may be empty)"""
+    _lib.call("ngacf_recommend_topk", _p(F), int(F.shape[-1]), int(U), int(I), _p(users), users.numel(), int(K), _p(excl_ptr),
+              _p(excl_items), _p(in_pool), _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
+
+
 def eval_metrics(top_ids, users, inter, hits, sums, ws):
     _lib.call("ngacf_eval_metrics", _p(top_ids), _p(users), users.numel(), _p(inter.test_ptr), _p(inter.test_items), _p(hits),
               _p(sums), _p(ws), ws.numel() * ws.element_size(), _s())
