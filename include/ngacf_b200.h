@@ -413,6 +413,28 @@ int ngacf_recommend_topk(const float* F, int32_t width, int32_t U, int32_t I, co
                          const int32_t* excl_ptr, const int32_t* excl_items, const uint8_t* in_pool, int32_t* top_ids,
                          float* top_scores, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Similar-item lists for any query items (K = 1 .. NGACF_RECOMMEND_MAX_K), by cosine similarity of the items' final features.  F as
+ * for ngacf_recommend_topk; item j's row is F[U+j].  With dot(a, b) the adjacent-pair tree of ngacf_recommend_topk over products
+ * rounded to fp32:
+ *   rn(j)      = 1 / sqrt(dot(F[U+j], F[U+j])) (correctly rounded division and square root), 0 when that sum is not > 0;
+ *   sim(q, j)  = (dot(F[U+q], F[U+j]) * rn(q)) * rn(j), each product rounded to fp32, in this order.  An all-zero row has
+ *                similarity 0 to every item.
+ *   candidates: items with in_pool[j] != 0 (in_pool NULL: every item) minus the query item itself.
+ *   order:      similarity descending, then item id ascending.  Row r of top_ids / top_scores ([n_items][K]) is items[r]'s list,
+ *               padded with id -1 / score 0.0 past the candidates; a query id outside [0, I) gives a padded row and reads nothing.
+ *               Duplicated queries get identical rows; a row does not depend on the other queries of the call.
+ *   workspace:  ngacf_similar_items_topk_workspace_bytes(width, I, n_items, K) bytes: the I inverse norms (the call computes them
+ *               itself), plus the partial lists when few queries split the item range.  Never 0 for n_items > 0.  A smaller
+ *               workspace returns NGACF_ERR_WORKSPACE and writes nothing; nothing beyond the reported size is written.
+ * Width other than 64 / 128 or K outside 1 .. NGACF_RECOMMEND_MAX_K returns NGACF_ERR_UNSUPPORTED.  Deterministic; no allocation, no
+ * synchronisation (CUDA-graph capturable).  n_items == 0 is a no-op.
+ * ------------------------------------------------------------------------------------------- */
+size_t ngacf_similar_items_topk_workspace_bytes(int32_t width, int32_t I, int32_t n_items, int32_t K);
+int ngacf_similar_items_topk(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* items, int32_t n_items, int32_t K,
+                             const uint8_t* in_pool, int32_t* top_ids, float* top_scores, void* workspace, size_t workspace_bytes,
+                             void* stream);
+
 #ifdef __cplusplus
 }
 #endif

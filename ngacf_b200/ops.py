@@ -313,6 +313,17 @@ def recommend_topk(F, U, I, users, K, excl_ptr, excl_items, in_pool, top_ids, to
               _p(excl_items), _p(in_pool), _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
 
 
+def similar_items_topk_workspace_bytes(width, I, n_items, K):
+    return int(_lib.load().ngacf_similar_items_topk_workspace_bytes(int(width), int(I), int(n_items), int(K)))
+
+
+def similar_items_topk(F, U, I, items, K, in_pool, top_ids, top_scores, ws):
+    """top-K cosine-similar items of the query `items` (int32) from final features F (U+I, 64 or 128), the query itself left out;
+    in_pool may be None; ws: uint8 tensor of similar_items_topk_workspace_bytes(...) bytes"""
+    _lib.call("ngacf_similar_items_topk", _p(F), int(F.shape[-1]), int(U), int(I), _p(items), items.numel(), int(K), _p(in_pool),
+              _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
+
+
 def eval_metrics(top_ids, users, inter, hits, sums, ws):
     _lib.call("ngacf_eval_metrics", _p(top_ids), _p(users), users.numel(), _p(inter.test_ptr), _p(inter.test_items), _p(hits),
               _p(sums), _p(ws), ws.numel() * ws.element_size(), _s())

@@ -1,7 +1,10 @@
-"""Top-K recommendation lists for any users of a trained SPUIGACF / SPUIMultiGACF (ngacf_recommend_topk, csrc/recommend.cu).
+"""Top-K lists from a trained SPUIGACF / SPUIMultiGACF (csrc/recommend.cu): items for users (ngacf_recommend_topk) and items like
+an item (ngacf_similar_items_topk).
 
-The lists are the AllNeg ranking's: exact fp32 scores with the specified summation tree, candidates = item pool minus the excluded
-items, order = score descending, then item id ascending (the reference's ranklist_by_heapq).  K is 1 .. 100."""
+User lists are the AllNeg ranking's: exact fp32 scores with the specified summation tree, candidates = item pool minus the excluded
+items, order = score descending, then item id ascending (the reference's ranklist_by_heapq).  Similar-item lists rank by the cosine
+of the items' final features (the same tree for the dot products and the norms), candidates = item pool minus the query item, same
+order.  K is 1 .. 100."""
 from __future__ import annotations
 
 import numpy as np
@@ -62,28 +65,33 @@ class Recommender:
         finally:
             m.train(was_training)
 
-    def _users(self, users):
-        if torch.is_tensor(users):
-            if users.dtype.is_floating_point or users.dtype.is_complex or users.dtype == torch.bool:
-                raise ValueError("users must be integer ids, got %s" % users.dtype)
-            t = users
+    def _ids(self, ids, bound, what):
+        """integer ids in [0, bound) -> int32 tensor on the features' device; ValueError otherwise (before any launch)"""
+        if torch.is_tensor(ids):
+            if ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool:
+                raise ValueError("%ss must be integer ids, got %s" % (what, ids.dtype))
+            t = ids
         else:
-            a = np.asarray(users)
+            a = np.asarray(ids)
             if a.size and not np.issubdtype(a.dtype, np.integer):
-                raise ValueError("users must be integer ids, got %s" % a.dtype)
+                raise ValueError("%ss must be integer ids, got %s" % (what, a.dtype))
             t = torch.from_numpy(a.astype(np.int64, copy=False).reshape(a.shape))
         if t.dim() != 1:
-            raise ValueError("users must be one-dimensional, got shape %s" % (tuple(t.shape),))
-        if t.numel() and (int(t.min()) < 0 or int(t.max()) >= self.U):
-            raise ValueError("user ids must lie in [0, %d)" % self.U)
+            raise ValueError("%ss must be one-dimensional, got shape %s" % (what, tuple(t.shape)))
+        if t.numel() and (int(t.min()) < 0 or int(t.max()) >= bound):
+            raise ValueError("%s ids must lie in [0, %d)" % (what, bound))
         return t.to(device=self.F.device, dtype=torch.int32).contiguous()
+
+    @staticmethod
+    def _k(K):
+        if isinstance(K, bool) or not isinstance(K, (int, np.integer)) or not 1 <= int(K) <= MAX_K:
+            raise ValueError("K must be an integer in 1..%d, got %r" % (MAX_K, K))
+        return int(K)
 
     def __call__(self, users, K: int = 20):
         """-> (ids int64 (n, K), scores float32 (n, K)) on the GPU; rows with fewer than K candidates end in id -1 / score 0.0"""
-        if isinstance(K, bool) or not isinstance(K, (int, np.integer)) or not 1 <= int(K) <= MAX_K:
-            raise ValueError("K must be an integer in 1..%d, got %r" % (MAX_K, K))
-        K = int(K)
-        u = self._users(users)
+        K = self._k(K)
+        u = self._ids(users, self.U, "user")
         n = u.numel()
         dev = self.F.device
         ids = torch.empty((n, K), dtype=torch.int32, device=dev)
@@ -91,6 +99,21 @@ class Recommender:
         if n:
             ws = torch.empty(ops.recommend_topk_workspace_bytes(self.F.shape[-1], self.I, n, K), dtype=torch.uint8, device=dev)
             ops.recommend_topk(self.F, self.U, self.I, u, K, self.excl_ptr, self.excl_items, self.in_pool, ids, scores, ws)
+        return ids.long(), scores
+
+    def similar_items(self, items, K: int = 20):
+        """-> (ids int64 (n, K), scores float32 (n, K)) on the GPU: for each query item the K items of highest cosine similarity of the
+        final features of the last refresh(), the query itself left out, candidates restricted to the item pool when the Recommender
+        has `inter` (`exclude` does not apply); rows with fewer than K candidates end in id -1 / score 0.0"""
+        K = self._k(K)
+        q = self._ids(items, self.I, "item")
+        n = q.numel()
+        dev = self.F.device
+        ids = torch.empty((n, K), dtype=torch.int32, device=dev)
+        scores = torch.empty((n, K), dtype=torch.float32, device=dev)
+        if n:
+            ws = torch.empty(ops.similar_items_topk_workspace_bytes(self.F.shape[-1], self.I, n, K), dtype=torch.uint8, device=dev)
+            ops.similar_items_topk(self.F, self.U, self.I, q, K, self.in_pool, ids, scores, ws)
         return ids.long(), scores
 
 
