@@ -435,6 +435,44 @@ int ngacf_similar_items_topk(const float* F, int32_t width, int32_t U, int32_t I
                              const uint8_t* in_pool, int32_t* top_ids, float* top_scores, void* workspace, size_t workspace_bytes,
                              void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Audience lists: the users to show each query item to (K = 1 .. NGACF_RECOMMEND_MAX_K).  F as for ngacf_recommend_topk.  The score
+ * of (item q, user u) is dot(F[U+q], F[u]) by the tree of ngacf_recommend_topk; the products commute exactly in IEEE fp32, so it has
+ * the bits of the recommend score of (u, q).
+ *   candidates: users with user_pool[u] != 0 (user_pool NULL: every user) minus the item's excluded users, given as a CSR over items
+ *               (excl_ptr[I+1], excl_users ascending per item; both NULL: nothing is excluded).
+ *   order:      score descending, then user id ascending.  Row r of top_ids / top_scores ([n_items][K]) is items[r]'s list, padded
+ *               with id -1 / score 0.0 past the candidates; a query id outside [0, I) gives a padded row and reads nothing.
+ *               Duplicated queries get identical rows; a row does not depend on the other queries of the call.
+ *   workspace:  ngacf_audience_topk_workspace_bytes(width, U, n_items, K) bytes (0 when there are enough queries to rank every user
+ *               range in one pass; few queries split the user range and merge partial lists there).  A smaller workspace returns
+ *               NGACF_ERR_WORKSPACE and writes nothing; nothing beyond the reported size is written.
+ * Width other than 64 / 128 or K outside 1 .. NGACF_RECOMMEND_MAX_K returns NGACF_ERR_UNSUPPORTED.  Deterministic; no allocation, no
+ * synchronisation (CUDA-graph capturable).  n_items == 0 is a no-op.
+ * ------------------------------------------------------------------------------------------- */
+size_t ngacf_audience_topk_workspace_bytes(int32_t width, int32_t U, int32_t n_items, int32_t K);
+int ngacf_audience_topk(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* items, int32_t n_items, int32_t K,
+                        const int32_t* excl_ptr, const int32_t* excl_users, const uint8_t* user_pool, int32_t* top_ids,
+                        float* top_scores, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Similar-user lists for any query users (K = 1 .. NGACF_RECOMMEND_MAX_K): ngacf_similar_items_topk with the users' rows F[u] in
+ * place of the items' rows.
+ *   rn(u)      = 1 / sqrt(dot(F[u], F[u])), 0 when that sum is not > 0;  sim(q, u) = (dot(F[q], F[u]) * rn(q)) * rn(u).
+ *   candidates: users with user_pool[u] != 0 (user_pool NULL: every user) minus the query user itself.
+ *   order:      similarity descending, then user id ascending.  Rows as for ngacf_similar_items_topk; a query id outside [0, U) gives
+ *               a padded row and reads nothing.
+ *   workspace:  ngacf_similar_users_topk_workspace_bytes(width, U, n_users, K) bytes: the U inverse norms (256-byte aligned), plus
+ *               the partial lists when few queries split the user range.  Never 0 for n_users > 0.  A smaller workspace returns
+ *               NGACF_ERR_WORKSPACE and writes nothing; nothing beyond the reported size is written.
+ * Width other than 64 / 128 or K outside 1 .. NGACF_RECOMMEND_MAX_K returns NGACF_ERR_UNSUPPORTED.  Deterministic; no allocation, no
+ * synchronisation (CUDA-graph capturable).  n_users == 0 is a no-op.
+ * ------------------------------------------------------------------------------------------- */
+size_t ngacf_similar_users_topk_workspace_bytes(int32_t width, int32_t U, int32_t n_users, int32_t K);
+int ngacf_similar_users_topk(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users, int32_t K,
+                             const uint8_t* user_pool, int32_t* top_ids, float* top_scores, void* workspace, size_t workspace_bytes,
+                             void* stream);
+
 #ifdef __cplusplus
 }
 #endif

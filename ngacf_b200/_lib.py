@@ -89,6 +89,11 @@ SIGNATURES = {
     # similar-item lists
     "ngacf_similar_items_topk_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
     "ngacf_similar_items_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, c_size_t, P]),
+    # audience and similar-user lists
+    "ngacf_audience_topk_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "ngacf_audience_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, P, P, c_size_t, P]),
+    "ngacf_similar_users_topk_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
+    "ngacf_similar_users_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, c_size_t, P]),
 }
 
 _lib = None

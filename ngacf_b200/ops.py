@@ -324,6 +324,28 @@ def similar_items_topk(F, U, I, items, K, in_pool, top_ids, top_scores, ws):
               _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
 
 
+def audience_topk_workspace_bytes(width, U, n_items, K):
+    return int(_lib.load().ngacf_audience_topk_workspace_bytes(int(width), int(U), int(n_items), int(K)))
+
+
+def audience_topk(F, U, I, items, K, excl_ptr, excl_users, user_pool, top_ids, top_scores, ws):
+    """top-K users of the query `items` (int32) from final features F (U+I, 64 or 128); excl_ptr/excl_users (CSR over items) and
+    user_pool may be None; ws: uint8 tensor of audience_topk_workspace_bytes(...) bytes (may be empty)"""
+    _lib.call("ngacf_audience_topk", _p(F), int(F.shape[-1]), int(U), int(I), _p(items), items.numel(), int(K), _p(excl_ptr),
+              _p(excl_users), _p(user_pool), _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
+
+
+def similar_users_topk_workspace_bytes(width, U, n_users, K):
+    return int(_lib.load().ngacf_similar_users_topk_workspace_bytes(int(width), int(U), int(n_users), int(K)))
+
+
+def similar_users_topk(F, U, I, users, K, user_pool, top_ids, top_scores, ws):
+    """top-K cosine-similar users of the query `users` (int32) from final features F (U+I, 64 or 128), the query itself left out;
+    user_pool may be None; ws: uint8 tensor of similar_users_topk_workspace_bytes(...) bytes"""
+    _lib.call("ngacf_similar_users_topk", _p(F), int(F.shape[-1]), int(U), int(I), _p(users), users.numel(), int(K), _p(user_pool),
+              _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
+
+
 def eval_metrics(top_ids, users, inter, hits, sums, ws):
     _lib.call("ngacf_eval_metrics", _p(top_ids), _p(users), users.numel(), _p(inter.test_ptr), _p(inter.test_items), _p(hits),
               _p(sums), _p(ws), ws.numel() * ws.element_size(), _s())

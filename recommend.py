@@ -14,7 +14,12 @@ writes recs/SPUIGACF_ml100k_010_top50.tsv: one line `user<TAB>rank<TAB>item<TAB>
   python recommend.py --dataset ml100k --model SPUIGACF --train_mode PairSampling --eval_mode AllNeg --resume_from 10 \\
       --topk 10 --similar-items 3,17,42
 
-writes recs/SPUIGACF_ml100k_010_similar10.tsv: one line `item<TAB>rank<TAB>similar_item<TAB>score` per entry.
+writes recs/SPUIGACF_ml100k_010_similar10.tsv: one line `item<TAB>rank<TAB>similar_item<TAB>score` per entry.  With
+--audience all|3,17,42|@file the lists are the users to show those items to (the score of the user lists, the users with any train
+or test item as candidates, minus those --exclude leaves out for the item), written to ..._audience{K}.tsv as
+`item<TAB>rank<TAB>user<TAB>score`; with --similar-users all|3,17,42|@file the users most similar to those users (cosine, as for
+items), written to ..._similarusers{K}.tsv as `user<TAB>rank<TAB>similar_user<TAB>score`.  At most one of the three flags is given,
+--users stays at its default with any of them, and --exclude too with --similar-items or --similar-users.
 """
 import os
 import sys
@@ -36,9 +41,19 @@ def build_parser():
     p.add_argument("--exclude", type=str, default="train", help="items left out of a user's list: train, all (train and test) or none")
     p.add_argument("--similar-items", type=str, default=None,
                    help="rank items like these items instead of items for users: all, a comma-separated id list, or @FILE")
+    p.add_argument("--audience", type=str, default=None,
+                   help="rank users for these items (--exclude applies per item): all, a comma-separated id list, or @FILE")
+    p.add_argument("--similar-users", type=str, default=None,
+                   help="rank users like these users: all, a comma-separated id list, or @FILE")
     p.add_argument("--out", type=str, default=None,
-                   help="output TSV (default recs/{model}_{dataset}_{N:03d}_top{K}.tsv, with --similar-items ..._similar{K}.tsv)")
+                   help="output TSV (default recs/{model}_{dataset}_{N:03d}_top{K}.tsv, with --similar-items ..._similar{K}.tsv, "
+                        "--audience ..._audience{K}.tsv, --similar-users ..._similarusers{K}.tsv)")
     return p
+
+
+# the query-list flags: (argparse dest, flag, file name tag); at most one is given
+QUERY_FLAGS = (("similar_items", "--similar-items", "similar"), ("audience", "--audience", "audience"),
+               ("similar_users", "--similar-users", "similarusers"))
 
 
 def parse_ids(spec, flag="--users", words=("eval", "all")):
@@ -58,7 +73,7 @@ def parse_ids(spec, flag="--users", words=("eval", "all")):
 
 
 def default_out(args):
-    kind = "similar" if args.similar_items is not None else "top"
+    kind = next((tag for dest, _, tag in QUERY_FLAGS if getattr(args, dest) is not None), "top")
     return os.path.join("recs", "{}_{}_{:03d}_{}{}.tsv".format(args.model, args.dataset, args.resume_from, kind, args.topk))
 
 
@@ -76,7 +91,18 @@ def parse_args(argv=None):
     if args.resume_from < 1:
         raise ValueError("--resume_from N is required: the checkpoint ckpts/{model}_{dataset}_{N:03d}.pkl to rank with")
     args.user_ids = parse_ids(args.users)
-    args.item_ids = None
+    given = [flag for dest, flag, _ in QUERY_FLAGS if getattr(args, dest) is not None]
+    if len(given) > 1:
+        raise ValueError("%s: give at most one of them" % " and ".join(given))
+    args.item_ids = args.audience_ids = args.similar_user_ids = None
+    if args.audience is not None:
+        if args.users != "eval":
+            raise ValueError("--audience ranks users for items: leave --users at its default")
+        args.audience_ids = parse_ids(args.audience, "--audience", ("all",))
+    if args.similar_users is not None:
+        if args.users != "eval" or args.exclude != "train":
+            raise ValueError("--similar-users ranks users like users: leave --users and --exclude at their defaults")
+        args.similar_user_ids = parse_ids(args.similar_users, "--similar-users", ("all",))
     if args.similar_items is not None:
         if args.users != "eval" or args.exclude != "train":
             raise ValueError("--similar-items ranks items like items: leave --users and --exclude at their defaults")
@@ -111,30 +137,39 @@ def load_model(args, userNum, itemNum):
     return model
 
 
-def similar_items(args, inter, userNum, itemNum, adj):
-    """--similar-items: -> (items int64, ids int64 (n, K), scores float32 (n, K)) as numpy arrays; writes args.out"""
-    items = np.arange(itemNum, dtype=np.int64) if isinstance(args.item_ids, str) else args.item_ids
-    if items.size and (items.min() < 0 or items.max() >= itemNum):
-        raise ValueError("--similar-items: ids must lie in [0, %d)" % itemNum)
-    rec = Recommender(load_model(args, userNum, itemNum), adj, inter, "none")
+def query_lists(args, inter, userNum, itemNum, adj, spec, bound, flag, exclude, method, what):
+    """--similar-items / --audience / --similar-users: the queries of `spec` ('all': every id in [0, bound)), ranked by
+    Recommender.`method`; -> (queries int64, ids int64 (n, K), scores float32 (n, K)) as numpy arrays; writes args.out.  Ids outside
+    [0, bound) are refused before the checkpoint loads; `what` % (n, K) names the lists in the report line"""
+    queries = np.arange(bound, dtype=np.int64) if isinstance(spec, str) else spec
+    if queries.size and (queries.min() < 0 or queries.max() >= bound):
+        raise ValueError("%s: ids must lie in [0, %d)" % (flag, bound))
+    rec = Recommender(load_model(args, userNum, itemNum), adj, inter, exclude)
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    ids, scores = rec.similar_items(items, args.topk)
+    ids, scores = getattr(rec, method)(queries, args.topk)
     torch.cuda.synchronize()
     ms = (time.perf_counter() - t0) * 1e3
     ids, scores = ids.cpu().numpy(), scores.cpu().numpy()
-    write_tsv(args.out, items, ids, scores)
-    print("recommend: %d items, %d most similar, %.2f ms -> %s" % (items.size, args.topk, ms, args.out))
-    return items, ids, scores
+    write_tsv(args.out, queries, ids, scores)
+    print("recommend: %s, %.2f ms -> %s" % (what % (queries.size, args.topk), ms, args.out))
+    return queries, ids, scores
 
 
 def main(args):
-    """-> (users int64, ids int64 (n, K), scores float32 (n, K)) as numpy arrays; writes args.out.  With --similar-items: the query
-    items in place of the users"""
+    """-> (users int64, ids int64 (n, K), scores float32 (n, K)) as numpy arrays; writes args.out.  With --similar-items,
+    --audience or --similar-users: the query ids in place of the users"""
     seed_all(args.seed)
     inter, _, _, _, userNum, itemNum, adj = R.prepareData(args)
     if args.item_ids is not None:
-        return similar_items(args, inter, userNum, itemNum, adj)
+        return query_lists(args, inter, userNum, itemNum, adj, args.item_ids, itemNum, "--similar-items", "none", "similar_items",
+                           "%d items, %d most similar")
+    if args.audience_ids is not None:
+        return query_lists(args, inter, userNum, itemNum, adj, args.audience_ids, itemNum, "--audience", args.exclude, "audience",
+                           "%d items, audience of %d")
+    if args.similar_user_ids is not None:
+        return query_lists(args, inter, userNum, itemNum, adj, args.similar_user_ids, userNum, "--similar-users", "none",
+                           "similar_users", "%d users, %d most similar")
     if isinstance(args.user_ids, str):
         users = inter.eval_users.long().cpu().numpy() if args.user_ids == "eval" else np.arange(userNum, dtype=np.int64)
     else:

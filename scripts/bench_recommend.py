@@ -12,8 +12,14 @@ K 20 / 100, the item pool as candidates, with the all-users recommend pass (K 20
 all-items call ranks I queries where the user pass ranks the eval users, so `ratio_to_scaled_recommend` divides by that pass times
 I / eval users) and the norm kernel's own time from a torch.profiler capture of the 1-item calls.
 
+--audience and --similar-users measure the user-side lists (ngacf_audience_topk with the train users excluded, ngacf_similar_users_topk)
+from the same features: 1 / 256 / every item (audience) or every user (similar users) as queries, K 20 / 100, the users with any train
+or test item as candidates.  `ratio_per_query_row` is (ms / queries) over (ms / eval users) of the all-users recommend pass at the
+same K, measured in the same process: an all-items audience pass does the same U x I products as that pass.
+
     python scripts/bench_recommend.py [--workload gowalla] [--out profiles/recommend_bench.json]
     python scripts/bench_recommend.py --similar [--out profiles/similar_bench.json]
+    python scripts/bench_recommend.py --audience --similar-users [--out profiles/user_lists_bench.json]
 """
 import argparse
 import json
@@ -76,11 +82,57 @@ def bench_similar(F, U, I, inter, all_users, d):
     return res
 
 
+def bench_user_side(rec, F, U, I, inter, all_users, d, kinds):
+    from ngacf_b200 import ops
+    dev = F.device
+    excl_ptr, excl_users, pool = rec.user_candidates()       # rec excludes "train": the item -> users CSR of the train pairs
+    # kind -> (workspace bytes, ranking call, query sets)
+    plans = dict(audience=(ops.audience_topk_workspace_bytes,
+                           lambda q, K, ids, sc, ws: ops.audience_topk(F, U, I, q, K, excl_ptr, excl_users, pool, ids, sc, ws), I),
+                 similar_users=(ops.similar_users_topk_workspace_bytes,
+                                lambda q, K, ids, sc, ws: ops.similar_users_topk(F, U, I, q, K, pool, ids, sc, ws), U))
+    plans = {k: (wb, run, {"1": torch.arange(1, dtype=torch.int32, device=dev), "256": torch.arange(256, dtype=torch.int32, device=dev),
+                           "all": torch.arange(n_all, dtype=torch.int32, device=dev)}) for k, (wb, run, n_all) in plans.items() if k in kinds}
+    res = dict(recommend_all_users_ms={})
+    for kind in kinds:
+        res[kind] = dict(queries_all=plans[kind][2]["all"].numel(), list_ms={}, ratio_per_query_row={})
+    for K in (20, 100):
+        for kind in kinds:
+            ws_bytes, run, sets = plans[kind]
+            lists = {}
+            for name, q in sets.items():
+                n = q.numel()
+                ids = torch.empty((n, K), dtype=torch.int32, device=dev)
+                sc = torch.empty((n, K), dtype=torch.float32, device=dev)
+                ws = torch.empty(ws_bytes(d, U, n, K), dtype=torch.uint8, device=dev)
+                call = lambda: run(q, K, ids, sc, ws)
+                call()
+                lists[name] = (ids, sc)
+                res[kind]["list_ms"]["K%d_queries_%s" % (K, name)] = median_block_ms(call, 3 if name == "all" else 20)
+            for name in ("1", "256"):    # a row does not depend on the other queries or on the user slicing
+                n = sets[name].numel()
+                assert torch.equal(lists[name][0], lists["all"][0][:n]) and torch.equal(lists[name][1], lists["all"][1][:n]), (kind, d, K)
+        n = all_users.numel()
+        ids = torch.empty((n, K), dtype=torch.int32, device=dev)
+        sc = torch.empty((n, K), dtype=torch.float32, device=dev)
+        ws = torch.empty(ops.recommend_topk_workspace_bytes(d, I, n, K), dtype=torch.uint8, device=dev)
+        call = lambda: ops.recommend_topk(F, U, I, all_users, K, inter.train_ptr, inter.train_items, inter.in_pool, ids, sc, ws)
+        call()
+        rms = res["recommend_all_users_ms"]["K%d" % K] = median_block_ms(call, 3)
+        for kind in kinds:
+            for name, q in plans[kind][2].items():
+                key = "K%d_queries_%s" % (K, name)
+                res[kind]["ratio_per_query_row"][key] = (res[kind]["list_ms"][key] / q.numel()) / (rms / n)
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--workload", default="gowalla")
     ap.add_argument("--out", default=None)
     ap.add_argument("--similar", action="store_true", help="measure the similar-item lists instead of the user lists")
+    ap.add_argument("--audience", action="store_true", help="measure the audience lists instead of the user lists")
+    ap.add_argument("--similar-users", action="store_true", help="measure the similar-user lists instead of the user lists")
     args = ap.parse_args()
     from ngacf_b200 import ops
     from ngacf_b200.data import Interactions
@@ -108,6 +160,12 @@ def main():
         F = rec.F
         if args.similar:
             out["widths"][str(d)] = bench_similar(F, U, I, inter, user_sets["all"], d)
+            del tr, model, rec
+            torch.cuda.synchronize()
+            continue
+        kinds = [k for k, on in (("audience", args.audience), ("similar_users", args.similar_users)) if on]
+        if kinds:
+            out["widths"][str(d)] = bench_user_side(rec, F, U, I, inter, user_sets["all"], d, kinds)
             del tr, model, rec
             torch.cuda.synchronize()
             continue
