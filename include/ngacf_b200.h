@@ -473,6 +473,28 @@ int ngacf_similar_users_topk(const float* F, int32_t width, int32_t U, int32_t I
                              const uint8_t* user_pool, int32_t* top_ids, float* top_scores, void* workspace, size_t workspace_bytes,
                              void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Full-ranking metrics at several cut-offs over ranked lists (the lists of ngacf_recommend_topk or of the AllNeg scorers).  Row j of
+ * top_ids ([n_users][K_list], -1 padded, distinct ids) is users[j]'s list; T = users[j]'s test items (test_ptr/test_items, a CSR over
+ * users, ascending per user).  For a cut-off k with h = the number of the first k entries that are in T (-1 is a miss):
+ *   precision = h / k;  recall = h / |T|;  hit_ratio = (h > 0);  mrr = 1 / (r + 1) for the first hit at rank r < k, else 0;
+ *   ndcg = DCG / IDCG with DCG = sum over hits at rank r < k of 1 / log2(r + 2) (in rank order) and IDCG = the same sum over the
+ *          ranks r < min(|T|, k) (the standard ideal list, not the reference's sorted hit list);
+ *   recall and ndcg are 0 for an empty T.  All fp64; the discounts are the bits of numpy's 1.0 / np.log2(np.arange(2, 102)).
+ *   ks:        HOST array of n_ks cut-offs, strictly increasing in 1..K_list (passed to the kernel by value).
+ *   sums:      [5 * n_ks], metric-major: precision at each cut-off, then recall, ndcg, hit_ratio, mrr; summed over the users in a
+ *              fixed order (two runs give the same bits).  n_users == 0 writes zeros.
+ *   per_user:  [n_users][5 * n_ks] in the layout of sums, or NULL.
+ *   workspace: ngacf_cutoff_metrics_workspace_bytes(n_users, n_ks) bytes; a smaller one returns NGACF_ERR_WORKSPACE and writes nothing.
+ * K_list outside 1 .. NGACF_RECOMMEND_MAX_K, n_ks outside 1 .. NGACF_CUTOFF_MAX_KS or cut-offs that are not strictly increasing in
+ * 1 .. K_list return NGACF_ERR_UNSUPPORTED before any launch.  No allocation, no synchronisation (CUDA-graph capturable).
+ * ------------------------------------------------------------------------------------------- */
+#define NGACF_CUTOFF_MAX_KS 8
+size_t ngacf_cutoff_metrics_workspace_bytes(int32_t n_users, int32_t n_ks);
+int ngacf_cutoff_metrics(const int32_t* top_ids, int32_t K_list, const int32_t* users, int32_t n_users, const int32_t* test_ptr,
+                         const int32_t* test_items, const int32_t* ks, int32_t n_ks, double* sums, double* per_user, void* workspace,
+                         size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -94,6 +94,9 @@ SIGNATURES = {
     "ngacf_audience_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, P, P, c_size_t, P]),
     "ngacf_similar_users_topk_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
     "ngacf_similar_users_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, c_size_t, P]),
+    # full-ranking metrics at several cut-offs
+    "ngacf_cutoff_metrics_workspace_bytes": (c_size_t, [c_int32, c_int32]),
+    "ngacf_cutoff_metrics": (c_int32, [P, c_int32, P, c_int32, P, P, P, c_int32, P, P, P, c_size_t, P]),
 }
 
 _lib = None

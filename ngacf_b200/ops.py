@@ -351,6 +351,19 @@ def eval_metrics(top_ids, users, inter, hits, sums, ws):
               _p(sums), _p(ws), ws.numel() * ws.element_size(), _s())
 
 
+def cutoff_metrics_workspace_bytes(n_users, n_ks):
+    return int(_lib.load().ngacf_cutoff_metrics_workspace_bytes(int(n_users), int(n_ks)))
+
+
+def cutoff_metrics(top_ids, users, inter, ks, sums, per_user, ws):
+    """precision/recall/ndcg/hit_ratio/mrr at the cut-offs `ks` (host ints, strictly increasing, <= top_ids.shape[1]) of the ranked
+    lists top_ids (n, K_list) int32 of `users` against inter.test_ptr/test_items: sums float64[5 * len(ks)] (metric-major), per_user
+    float64 (n, 5 * len(ks)) or None; ws: cutoff_metrics_workspace_bytes(n, len(ks)) bytes"""
+    ka = (ctypes.c_int32 * len(ks))(*[int(k) for k in ks])
+    _lib.call("ngacf_cutoff_metrics", _p(top_ids), int(top_ids.shape[-1]), _p(users), users.numel(), _p(inter.test_ptr),
+              _p(inter.test_items), ka, len(ks), _p(sums), _p(per_user), _p(ws), ws.numel() * ws.element_size(), _s())
+
+
 NEG_TAG_TRAIN, NEG_TAG_EVAL = 0x4E54, 0x4E45
 
 

@@ -20,7 +20,7 @@ from graphattention.BPRLoss import BPRLoss
 from graphattention.SPUIGACF import SPUIGACF, SPUIMultiGACF
 from ngacf_b200.data import Interactions
 from ngacf_b200.hostdata import load_dataset
-from train_eval_Gowalla import eval_neg_all, eval_neg_sample, train_bpr, train_neg_sample
+from train_eval_Gowalla import eval_full_ranking, eval_neg_all, eval_neg_sample, train_bpr, train_neg_sample
 
 
 def prepareData(args):
@@ -99,6 +99,7 @@ def main(args):
                 summaryWriter.add_scalar("metrics/NDCG", NDCG, epoch)
                 print("The time of evaluate epoch {:03d}".format(epoch) + " is: " + time.strftime("%H: %M: %S", time.gmtime(time.time() - t0)))
                 print("epoch:{}, HR:{:5f}, NDCG:{:5f}".format(epoch, HR, NDCG))
+                full_ranking(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0)
                 continue
             metrics = eval_neg_all(model, args.batch_size, test_df, test_pos_neg, adj, itemNum, args.parallel)
             print("epoch:{} metrics:{}".format(epoch, metrics))
@@ -108,6 +109,20 @@ def main(args):
                 summaryWriter.add_scalar("metrics@{}/ndcg".format(K), metrics["ndcg"][i], epoch)
                 summaryWriter.add_scalar("metrics@{}/hit_ratio".format(K), metrics["hit_ratio"][i], epoch)
             print("The time of evaluate epoch {:03d}".format(epoch) + " is: " + time.strftime("%H: %M: %S", time.gmtime(time.time() - t0)))
+            full_ranking(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0)
+
+
+def full_ranking(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0):
+    """--eval_ks: full-ranking metrics with the standard definitions (ngacf_b200.cutoff_eval), printed by rank 0 as one line of plain
+    Python values and logged as full@K/<metric>"""
+    if not args.eval_ks:
+        return
+    res = eval_full_ranking(model, test_df, test_pos_neg, adj, args.eval_ks, args.parallel)
+    for i, K in enumerate(res["ks"]):
+        for name in ("precision", "recall", "ndcg", "hit_ratio", "mrr"):
+            summaryWriter.add_scalar("full@{}/{}".format(K, name), res[name][i], epoch)
+    if rank0:
+        print("epoch:{} full-ranking metrics:{}".format(epoch, {k: v.tolist() if hasattr(v, "tolist") else v for k, v in res.items()}))
 
 
 def build_parser():
@@ -132,6 +147,9 @@ def build_parser():
     p.add_argument("--parallel", type=ast.literal_eval, default=False)
     p.add_argument("--gpu_id", type=str, default="0")
     p.add_argument("--data_root", type=str, default=None, help="directory holding 1K/u.data, Gowalla/g_train.csv, ... (default ./data)")
+    p.add_argument("--eval_ks", type=str, default=None,
+                   help="e.g. 20,50,100: also report full-ranking precision/recall/ndcg/hit_ratio/mrr at these cut-offs (up to 8 of 1..100) "
+                        "with the standard definitions, every evaluation epoch")
     return p
 
 
@@ -143,6 +161,9 @@ def parse_args(argv=None):
     if args.embedSize not in WIDTHS:
         raise ValueError("--embedSize %d is not supported: the sm_100a kernels are built for embedSize %s"
                          % (args.embedSize, " and ".join(map(str, WIDTHS))))
+    if args.eval_ks is not None:
+        from ngacf_b200.cutoff_eval import parse_ks
+        args.eval_ks = parse_ks(args.eval_ks)
     if args.parallel and args.embedSize != 64:
         raise ValueError("--parallel True is built for --embedSize 64 only; train --embedSize %d on one GPU (--parallel False)" % args.embedSize)
     return args

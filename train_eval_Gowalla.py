@@ -200,6 +200,34 @@ def eval_neg_all(model, batch_size, test_df, test_pos_neg, adj, itemNum, is_para
         return ev(Z)
 
 
+def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="auto"):
+    """Full-ranking metrics at the cut-offs `ks` (up to 8 of 1..100) with the standard definitions: precision, recall, NDCG with the
+    ideal DCG of min(|test|, k) hits, hit ratio and MRR, averaged over the users with train and test items
+    (ngacf_b200.cutoff_eval).  Returns FullRankingEvaluator.metrics()'s dict.  is_parallel under torchrun: the users are sharded over
+    the ranks and the sums merged, as in eval_neg_all."""
+    from ngacf_b200.cutoff_eval import FullRankingEvaluator, check_ks
+    m = _unwrap(model)
+    model.eval()
+    _require_plain(m, "eval_full_ranking")
+    ks = check_ks(ks)
+    inter = _interactions(model, None, test_pos_neg, test_df)
+    adj_t = _device_adj(model, adj)
+    with torch.no_grad():
+        Z = m.propagate(adj_t)
+        ev = getattr(m, "_full_evaluator", None)
+        world = _world() if is_parallel else 1
+        if ev is None or ev.inter is not inter or ev.mode != mode or ev.ks != ks or getattr(ev, "world", 1) != world:
+            users = None
+            if world > 1:
+                import torch.distributed as dist
+                from ngacf_b200.dist import shard_eval_users
+                users = shard_eval_users(inter.eval_users, dist.get_rank(), world)
+            ev = FullRankingEvaluator(inter, ks, mode, users=users)
+            ev.world = world
+            m._full_evaluator = ev
+        return ev(Z)
+
+
 # ------------------------------------------------------------------------------------------------
 # NegSampling training / SampledNeg evaluation (the reference CLI's default modes, SURVEY 8f-3)
 # ------------------------------------------------------------------------------------------------
