@@ -495,6 +495,33 @@ int ngacf_cutoff_metrics(const int32_t* top_ids, int32_t K_list, const int32_t* 
                          const int32_t* test_items, const int32_t* ks, int32_t n_ks, double* sums, double* per_user, void* workspace,
                          size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Beyond-accuracy statistics of ranked lists.  Row j of top_ids ([n_rows][K_list], -1 padded) is one list; an entry counts when its
+ * id lies in [0, I), any other id is skipped.  ks: HOST array of n_ks cut-offs, strictly increasing in 1..K_list (by value).
+ *   counts:    [n_ks][I] int32 or NULL: counts[q][i] = the number of entries with id i among the first ks[q] entries of every row
+ *              (exposure).  It counts entries, so a row that repeats an id counts it each time; for rows of distinct ids (the lists
+ *              of the ranking entry points) it is the number of rows whose first ks[q] entries contain item i.  The call zeroes
+ *              counts itself; integer atomics, so the result does not depend on the schedule.
+ *   item_vals: [n_vals][I] fp64 item tables, n_vals in 0..NGACF_LIST_MAX_VALS.
+ *   rows:      [n_rows][n_vals * n_ks] fp64 or NULL, table-major: rows[j][v * n_ks + q] = the mean of item_vals[v][id] over the
+ *              valid entries among row j's first ks[q], summed in rank order, then divided once by their number (0 with none).
+ * K_list, n_ks and the cut-offs are checked as in ngacf_cutoff_metrics; a bad n_vals also returns NGACF_ERR_UNSUPPORTED before any
+ * launch.  No allocation, no synchronisation (CUDA-graph capturable).
+ *
+ * Column sums of fp64 rows per group: sums[g][c] = the sum of rows[j][c] over the rows j with group[j] == g, for G groups
+ * (1..NGACF_GROUP_MAX) and n_cols columns (1..NGACF_GROUP_MAX_COLS; anything else returns NGACF_ERR_UNSUPPORTED).  Rows whose group
+ * lies outside [0, G) are skipped.  Summed in a fixed order (two runs give the same bits); n_rows == 0 writes zeros.
+ *   workspace: ngacf_group_sums_workspace_bytes(n_rows, n_cols, G) bytes; a smaller one returns NGACF_ERR_WORKSPACE and writes nothing.
+ * ------------------------------------------------------------------------------------------- */
+#define NGACF_LIST_MAX_VALS 2
+#define NGACF_GROUP_MAX 8
+#define NGACF_GROUP_MAX_COLS 56
+int ngacf_list_stats(const int32_t* top_ids, int32_t K_list, int32_t n_rows, int32_t I, const int32_t* ks, int32_t n_ks,
+                     const double* item_vals, int32_t n_vals, int32_t* counts, double* rows, void* stream);
+size_t ngacf_group_sums_workspace_bytes(int32_t n_rows, int32_t n_cols, int32_t G);
+int ngacf_group_sums(const double* rows, int32_t n_rows, int32_t n_cols, const int32_t* group, int32_t G, double* sums, void* workspace,
+                     size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -97,6 +97,10 @@ SIGNATURES = {
     # full-ranking metrics at several cut-offs
     "ngacf_cutoff_metrics_workspace_bytes": (c_size_t, [c_int32, c_int32]),
     "ngacf_cutoff_metrics": (c_int32, [P, c_int32, P, c_int32, P, P, P, c_int32, P, P, P, c_size_t, P]),
+    # beyond-accuracy list statistics and per-group column sums
+    "ngacf_list_stats": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, P, c_int32, P, P, P]),
+    "ngacf_group_sums_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
+    "ngacf_group_sums": (c_int32, [P, c_int32, c_int32, P, c_int32, P, P, c_size_t, P]),
 }
 
 _lib = None

@@ -12,11 +12,31 @@ users with train data (users without test items count as zeros) and normalise ND
 (a user with 30 test items and one hit at rank 1 scores NDCG@20 = 1); neither is the standard definition.
 
 Where the lists come from: for max(ks) <= 20 at width 64 the tcgen05 AllNeg scorer's top-20 lists (its flagged rows re-ranked
-exactly; the ids equal the exact path's for every user), otherwise ngacf_recommend_topk with K = max(ks)."""
+exactly; the ids equal the exact path's for every user), otherwise ngacf_recommend_topk with K = max(ks).
+
+Beyond-accuracy metrics of the same lists (list_metrics(), csrc/list_stats.cu).  An entry of a list is valid when its id lies in
+[0, I) (-1 pads).  Item statistics come from the train split only: d_i = the number of distinct users with item i among their train
+items, n_tr = inter.n_train_users.
+    exposure c_k(i) = the number of evaluated users whose first k entries contain item i (integers, all-reduced when sharded)
+    coverage@k      = |{i in pool : c_k(i) > 0}| / |pool|                          (pool = inter.pool)
+    gini@k          = sum_j (2 j - n - 1) c_(j) / (n sum c) over the pool items' c_k sorted ascending as c_(1..n), n = |pool|
+                      (0 when sum c = 0); numerator and denominator exact in int64, one fp64 division
+    novelty@k       = per user, the mean over the valid entries among the first k of nov(i) = -log2((d_i + 1) / (n_tr + 1))
+    arp@k           = per user, the mean of d_i over the same entries (average recommended popularity)
+The per-user sums run in rank order in fp64 and are divided once by the number of valid entries (0 when there is none); novelty and
+arp are then averaged over the evaluated users with the divisor of metrics().  nov and d are fp64 item tables built once per
+Interactions on the host.
+
+User-activity groups (group_metrics(G), the interaction sparsity levels of NGCF section 4.3.2): every user of inter.eval_users,
+sorted by (train degree, user id) ascending; with C_j the train degree summed over the users before user j and T the total, user j
+is in group min(G - 1, floor(G C_j / T)) (int64), G in 1..8.  The groups therefore hold about T / G train interactions each; one
+user with a very large degree can leave a group empty.  Per group: the number of evaluated users, their min / max train degree, their
+train interactions and the means over the group's users of the five metrics above and of novelty / arp at each cut-off."""
 from __future__ import annotations
 
 import numbers
 
+import numpy as np
 import torch
 
 from . import _lib, ops
@@ -26,6 +46,8 @@ from .evaluate import K as ALLNEG_K, AllNegEvaluator
 MAX_K = 100
 MAX_KS = 8
 METRICS = ("precision", "recall", "ndcg", "hit_ratio", "mrr")
+LIST_VALUES = ("novelty", "arp")
+MAX_GROUPS = 8
 MODES = ("auto", "tc", "exact")
 
 
@@ -49,6 +71,62 @@ def parse_ks(text: str):
     except ValueError:
         raise ValueError("cut-offs must be a comma-separated list of integers, got %r" % text) from None
     return check_ks(ks)
+
+
+def check_groups(G):
+    """-> G as an int; ValueError unless it is an integer in 1..8"""
+    if isinstance(G, bool) or not isinstance(G, numbers.Integral) or not 1 <= int(G) <= MAX_GROUPS:
+        raise ValueError("the number of user groups must be an integer in 1..%d, got %r" % (MAX_GROUPS, G))
+    return int(G)
+
+
+def item_degrees(inter: Interactions):
+    """d_i: the number of distinct users with item i among their train items, int64[I] (host)"""
+    return np.bincount(inter.host["train_items"], minlength=inter.I).astype(np.int64)
+
+
+def item_tables(inter: Interactions):
+    """float64 (2, I) device tables [nov | d] with nov(i) = -log2((d_i + 1) / (n_tr + 1)); built once per Interactions"""
+    t = inter.__dict__.get("_list_item_tables")
+    if t is None:
+        d = item_degrees(inter).astype(np.float64)
+        nov = -np.log2((d + 1.0) / (inter.n_train_users + 1.0))
+        t = torch.from_numpy(np.stack([nov, d])).to(inter.device)
+        inter._list_item_tables = t
+    return t
+
+
+def coverage_gini(counts, pool=None):
+    """counts: (n_ks, I) exposure counts, pool: item ids (None: counts holds the pool's columns already) -> (coverage, gini) float64
+    arrays of n_ks (definitions above)"""
+    c = np.asarray(counts) if pool is None else np.asarray(counts)[:, np.asarray(pool, np.int64)]
+    n = c.shape[1]
+    coverage = (c > 0).sum(1) / max(n, 1)
+    w = 2 * np.arange(1, n + 1, dtype=np.int64) - n - 1
+    num = np.sort(c, axis=1).astype(np.int64) @ w
+    den = n * c.sum(1, dtype=np.int64)
+    gini = np.where(den > 0, num / np.maximum(den, 1), 0.0)
+    return coverage, gini
+
+
+def split_groups(users, degrees, G):
+    """users, train degrees (host arrays) -> (users, degrees, group) sorted by (degree, user id) ascending, group[j] =
+    min(G - 1, floor(G C_j / T)) with C_j the degrees before j and T their total (int64)"""
+    G = check_groups(G)
+    users = np.asarray(users, np.int64)
+    degrees = np.asarray(degrees, np.int64)
+    order = np.lexsort((users, degrees))
+    users, degrees = users[order], degrees[order]
+    C = np.cumsum(degrees) - degrees
+    T = int(degrees.sum())
+    group = np.minimum(G - 1, (G * C) // max(T, 1))
+    return users, degrees, group
+
+
+def user_groups(inter: Interactions, G):
+    """the activity groups of every user of inter.eval_users (split_groups over their train degrees)"""
+    users = inter.eval_users.cpu().numpy().astype(np.int64)
+    return split_groups(users, np.diff(inter.host["train_ptr"])[users], G)
 
 
 class FullRankingEvaluator:
@@ -77,6 +155,8 @@ class FullRankingEvaluator:
         self._metric_ws = torch.empty(ops.cutoff_metrics_workspace_bytes(n, len(self.ks)), dtype=torch.uint8, device=dev)
         self.F = None
         self.source = None
+        self._tables = None            # list_metrics / group_metrics state, built on first use
+        self._groups = {}
 
     def rank(self, Z: torch.Tensor):
         """Z: pre-ELU last-stage output (N, 64) or (N, 128).  Ranks the lists of self.users."""
@@ -133,3 +213,102 @@ class FullRankingEvaluator:
     def __call__(self, Z):
         self.rank(Z)
         return self.metrics()
+
+    # ---- beyond-accuracy metrics and user-activity groups over the lists of the last rank() ----
+    def _list_setup(self):
+        if self._tables is not None:
+            return
+        it, dev = self.inter, self.inter.device
+        n, nk = self.users.numel(), len(self.ks)
+        self._tables = item_tables(it)
+        self._counts = torch.zeros((nk, it.I), dtype=torch.int32, device=dev)
+        self._list_rows = torch.zeros((n, len(LIST_VALUES) * nk), dtype=torch.float64, device=dev)
+        self._gsums = torch.zeros(MAX_GROUPS * (len(METRICS) + len(LIST_VALUES)) * nk + MAX_GROUPS, dtype=torch.float64, device=dev)
+        self._gs_ws = torch.empty(ops.group_sums_workspace_bytes(n, len(METRICS) * nk, MAX_GROUPS), dtype=torch.uint8, device=dev)
+        self._one_group = torch.zeros(max(n, 1), dtype=torch.int32, device=dev)
+
+    def _list_stats(self, counts: bool):
+        self._list_setup()
+        n = self.users.numel()
+        ops.list_stats(self.top_ids[:n], self.inter.I, self.ks, self._tables, self._counts if counts else None,
+                       self._list_rows if n else None)
+
+    def list_metrics(self):
+        """{"ks", "coverage", "gini", "novelty", "arp": float64 arrays of len(ks), "n_users", "n_items"}: exposure over the lists of
+        every rank (counts all-reduced when sharded; every rank returns the same dict); n_items = |pool|"""
+        from .dist import allreduce_sums
+        self._list_stats(True)
+        n, nk = self.users.numel(), len(self.ks)
+        nc = len(LIST_VALUES) * nk
+        buf = self._gsums[:nc + 1]
+        ops.group_sums(self._list_rows, self._one_group[:n], 1, buf[:nc].view(1, nc), self._gs_ws)
+        buf[-1] = float(n)
+        allreduce_sums(buf)
+        allreduce_sums(self._counts)
+        s = buf.cpu().numpy()
+        coverage, gini = coverage_gini(self._counts.index_select(1, self.inter.pool).cpu().numpy())
+        n_all = int(round(s[-1]))
+        means = s[:-1] / max(n_all, 1)
+        out = {"ks": list(self.ks), "coverage": coverage, "gini": gini}
+        for q, name in enumerate(LIST_VALUES):
+            out[name] = means[q * nk:(q + 1) * nk].copy()
+        out["n_users"] = n_all
+        out["n_items"] = int(self.inter.pool.numel())
+        return out
+
+    def _group_setup(self, G):
+        st = self._groups.get(G)
+        if st is not None:
+            return st
+        it = self.inter
+        mine = self.users.cpu().numpy().astype(np.int64)
+        users, deg, group = user_groups(it, G)
+        if not np.isin(mine, users).all():
+            raise ValueError("group_metrics: the evaluator's users must be evaluation users (users with train and test items)")
+        lookup = np.full(it.U, -1, np.int32)
+        lookup[users] = group
+        ev_groups = torch.from_numpy(lookup).to(it.device)[self.users.long()].to(torch.int32).contiguous()
+        n_users = np.bincount(lookup[mine], minlength=G).astype(np.float64)
+        degree = np.zeros((G, 2), np.int64)
+        inter_sum = np.zeros(G, np.int64)
+        for g in range(G):
+            d = deg[group == g]
+            if d.size:
+                degree[g] = (d.min(), d.max())
+                inter_sum[g] = d.sum()
+        st = dict(lookup=torch.from_numpy(lookup).to(it.device), rows=ev_groups,
+                  n_users=torch.from_numpy(n_users).to(it.device), degree=degree, interactions=inter_sum)
+        self._groups[G] = st
+        return st
+
+    def group_metrics(self, G=4):
+        """{"ks", "groups", "n_users", "degree", "interactions", "precision", "recall", "ndcg", "hit_ratio", "mrr", "novelty", "arp"}:
+        the user-activity groups (module docstring).  n_users (G,): the evaluated users of each group (all-reduced when sharded);
+        degree (G, 2): their min / max train degree; interactions (G,): their train interactions (both over inter.eval_users);
+        the metrics: (G, len(ks)) float64 means over each group's users, zeros for an empty group.  ValueError unless G is in 1..8
+        and the evaluator's users are evaluation users."""
+        from .dist import allreduce_sums
+        G = check_groups(G)
+        st = self._group_setup(G)
+        self._list_setup()
+        self._compute()
+        self._list_stats(False)
+        n, nk = self.users.numel(), len(self.ks)
+        na, nl = len(METRICS) * nk, len(LIST_VALUES) * nk
+        buf = self._gsums[:G * (na + nl) + G]
+        ops.group_sums(self._rows, st["rows"], G, buf[:G * na].view(G, na), self._gs_ws)
+        ops.group_sums(self._list_rows, st["rows"], G, buf[G * na:G * (na + nl)].view(G, nl), self._gs_ws)
+        buf[G * (na + nl):].copy_(st["n_users"])
+        allreduce_sums(buf)
+        s = buf.cpu().numpy()
+        counts = np.rint(s[G * (na + nl):]).astype(np.int64)
+        div = np.maximum(counts, 1)[:, None].astype(np.float64)
+        acc = s[:G * na].reshape(G, na) / div
+        lst = s[G * na:G * (na + nl)].reshape(G, nl) / div
+        out = {"ks": list(self.ks), "groups": G, "n_users": counts, "degree": st["degree"].copy(),
+               "interactions": st["interactions"].copy()}
+        for q, name in enumerate(METRICS):
+            out[name] = acc[:, q * nk:(q + 1) * nk].copy()
+        for q, name in enumerate(LIST_VALUES):
+            out[name] = lst[:, q * nk:(q + 1) * nk].copy()
+        return out

@@ -364,6 +364,27 @@ def cutoff_metrics(top_ids, users, inter, ks, sums, per_user, ws):
               _p(inter.test_items), ka, len(ks), _p(sums), _p(per_user), _p(ws), ws.numel() * ws.element_size(), _s())
 
 
+def list_stats(top_ids, I, ks, item_vals, counts, rows):
+    """exposure and per-row means over the ranked lists top_ids (n, K_list) int32 (-1 padded; ids outside [0, I) are skipped) at the
+    cut-offs `ks` (host ints, strictly increasing, <= K_list): counts int32 (len(ks), I) or None (zeroed by the call); item_vals
+    float64 (n_vals, I) with n_vals 0..2, or None; rows float64 (n, n_vals * len(ks)) (table-major) or None"""
+    ka = (ctypes.c_int32 * len(ks))(*[int(k) for k in ks])
+    n_vals = 0 if item_vals is None else int(item_vals.shape[0])
+    _lib.call("ngacf_list_stats", _p(top_ids), int(top_ids.shape[-1]), int(top_ids.shape[0]), int(I), ka, len(ks), _p(item_vals), n_vals,
+              _p(counts), _p(rows), _s())
+
+
+def group_sums_workspace_bytes(n_rows, n_cols, G):
+    return int(_lib.load().ngacf_group_sums_workspace_bytes(int(n_rows), int(n_cols), int(G)))
+
+
+def group_sums(rows, group, G, sums, ws):
+    """column sums of rows (n, n_cols) float64 per group: group (n,) int32 (ids outside [0, G) skipped), sums float64 (G, n_cols);
+    ws: group_sums_workspace_bytes(n, n_cols, G) bytes"""
+    _lib.call("ngacf_group_sums", _p(rows), int(rows.shape[0]), int(rows.shape[1]), _p(group), int(G), _p(sums), _p(ws),
+              ws.numel() * ws.element_size(), _s())
+
+
 NEG_TAG_TRAIN, NEG_TAG_EVAL = 0x4E54, 0x4E45
 
 

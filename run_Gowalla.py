@@ -20,7 +20,7 @@ from graphattention.BPRLoss import BPRLoss
 from graphattention.SPUIGACF import SPUIGACF, SPUIMultiGACF
 from ngacf_b200.data import Interactions
 from ngacf_b200.hostdata import load_dataset
-from train_eval_Gowalla import eval_full_ranking, eval_neg_all, eval_neg_sample, train_bpr, train_neg_sample
+from train_eval_Gowalla import eval_full_ranking, eval_neg_all, eval_neg_sample, list_reports, train_bpr, train_neg_sample
 
 
 def prepareData(args):
@@ -122,7 +122,31 @@ def full_ranking(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, 
         for name in ("precision", "recall", "ndcg", "hit_ratio", "mrr"):
             summaryWriter.add_scalar("full@{}/{}".format(K, name), res[name][i], epoch)
     if rank0:
-        print("epoch:{} full-ranking metrics:{}".format(epoch, {k: v.tolist() if hasattr(v, "tolist") else v for k, v in res.items()}))
+        print("epoch:{} full-ranking metrics:{}".format(epoch, _plain(res)))
+    if not (args.eval_beyond or args.eval_groups):
+        return
+    # --eval_beyond / --eval_groups: reports over the lists eval_full_ranking just ranked (every rank takes part in the all-reduce)
+    rep = list_reports(model, args.eval_beyond, args.eval_groups)
+    if rep["beyond"] is not None:
+        b = rep["beyond"]
+        for i, K in enumerate(b["ks"]):
+            for name in ("coverage", "gini", "novelty", "arp"):
+                summaryWriter.add_scalar("beyond@{}/{}".format(K, name), b[name][i], epoch)
+        if rank0:
+            print("epoch:{} beyond-accuracy metrics:{}".format(epoch, _plain(b)))
+    if rep["groups"] is not None:
+        g = rep["groups"]
+        for j in range(g["groups"]):
+            for i, K in enumerate(g["ks"]):
+                for name in ("precision", "recall", "ndcg", "hit_ratio", "mrr", "novelty", "arp"):
+                    summaryWriter.add_scalar("group{}@{}/{}".format(j, K, name), g[name][j][i], epoch)
+        if rank0:
+            print("epoch:{} user-group metrics:{}".format(epoch, _plain(g)))
+
+
+def _plain(res):
+    """a metrics dict with plain Python values, for one printed line"""
+    return {k: v.tolist() if hasattr(v, "tolist") else v for k, v in res.items()}
 
 
 def build_parser():
@@ -150,6 +174,12 @@ def build_parser():
     p.add_argument("--eval_ks", type=str, default=None,
                    help="e.g. 20,50,100: also report full-ranking precision/recall/ndcg/hit_ratio/mrr at these cut-offs (up to 8 of 1..100) "
                         "with the standard definitions, every evaluation epoch")
+    p.add_argument("--eval_beyond", type=str, default=False,
+                   help="True: also report catalogue coverage, the Gini index of item exposure, novelty and average recommended popularity "
+                        "of the ranked lists at the --eval_ks cut-offs")
+    p.add_argument("--eval_groups", type=str, default=None,
+                   help="G in 1..8: also report the --eval_ks metrics, novelty and popularity per group of users split by train degree "
+                        "into G groups of about equal train interactions (NGCF section 4.3.2)")
     return p
 
 
@@ -164,6 +194,24 @@ def parse_args(argv=None):
     if args.eval_ks is not None:
         from ngacf_b200.cutoff_eval import parse_ks
         args.eval_ks = parse_ks(args.eval_ks)
+    beyond = args.eval_beyond
+    if isinstance(beyond, str):
+        try:
+            beyond = ast.literal_eval(beyond)
+        except (ValueError, SyntaxError):
+            beyond = None
+    if not isinstance(beyond, bool):
+        raise ValueError("--eval_beyond must be True or False, got %r" % args.eval_beyond)
+    args.eval_beyond = beyond
+    if args.eval_groups is not None:
+        from ngacf_b200.cutoff_eval import check_groups
+        try:
+            G = int(args.eval_groups)
+        except ValueError:
+            raise ValueError("--eval_groups must be an integer in 1..8, got %r" % args.eval_groups) from None
+        args.eval_groups = check_groups(G)
+    if (args.eval_beyond or args.eval_groups) and not args.eval_ks:
+        raise ValueError("--eval_beyond and --eval_groups report at the --eval_ks cut-offs; give --eval_ks as well")
     if args.parallel and args.embedSize != 64:
         raise ValueError("--parallel True is built for --embedSize 64 only; train --embedSize %d on one GPU (--parallel False)" % args.embedSize)
     return args

@@ -228,6 +228,17 @@ def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="
         return ev(Z)
 
 
+def list_reports(model, beyond=True, groups=None):
+    """The beyond-accuracy metrics (coverage, Gini of the item exposure, novelty, ARP) and the metrics per user-activity group
+    (NGCF section 4.3.2) of the lists the preceding eval_full_ranking call ranked, from the evaluator it cached: no second
+    propagation or ranking.  Returns {"beyond": FullRankingEvaluator.list_metrics() or None, "groups":
+    FullRankingEvaluator.group_metrics(groups) or None}.  Under torchrun every rank calls it (the counts and sums are all-reduced)."""
+    ev = getattr(_unwrap(model), "_full_evaluator", None)
+    if ev is None or ev.source is None:
+        raise RuntimeError("list_reports: call eval_full_ranking first; it ranks the lists these reports read")
+    return {"beyond": ev.list_metrics() if beyond else None, "groups": ev.group_metrics(groups) if groups else None}
+
+
 # ------------------------------------------------------------------------------------------------
 # NegSampling training / SampledNeg evaluation (the reference CLI's default modes, SURVEY 8f-3)
 # ------------------------------------------------------------------------------------------------
