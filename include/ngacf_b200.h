@@ -414,6 +414,23 @@ int ngacf_recommend_topk(const float* F, int32_t width, int32_t U, int32_t I, co
                          float* top_scores, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Top-K lists ranked by an offset score (novelty-weighted or popularity-debiased lists): ngacf_recommend_topk with one fp32 offset
+ * per item added to every score of that item.
+ *   score:      s(u, i) = dot(F[u], F[U+i]) + item_offset[i], the sum rounded to fp32 once (round to nearest), where dot is the
+ *               score of ngacf_recommend_topk.  item_offset[I] is required (NULL returns NGACF_ERR_INVALID_ARG) and must be finite.
+ *               An all-zero item_offset gives the ids of ngacf_recommend_topk and its scores, except that -0.0 becomes +0.0.
+ *   candidates, order, padding, rows of out-of-range users: as for ngacf_recommend_topk, by the offset score.  top_scores holds the
+ *               offset scores.
+ *   workspace:  ngacf_recommend_topk_workspace_bytes(width, I, n_users, K) bytes.  A smaller workspace returns NGACF_ERR_WORKSPACE and
+ *               writes nothing; nothing beyond the reported size is written.
+ * Width other than 64 / 128 or K outside 1 .. NGACF_RECOMMEND_MAX_K returns NGACF_ERR_UNSUPPORTED.  Deterministic; no allocation, no
+ * synchronisation (CUDA-graph capturable).  n_users == 0 is a no-op.
+ * ------------------------------------------------------------------------------------------- */
+int ngacf_recommend_topk_offset(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users, int32_t K,
+                                const int32_t* excl_ptr, const int32_t* excl_items, const uint8_t* in_pool, const float* item_offset,
+                                int32_t* top_ids, float* top_scores, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Similar-item lists for any query items (K = 1 .. NGACF_RECOMMEND_MAX_K), by cosine similarity of the items' final features.  F as
  * for ngacf_recommend_topk; item j's row is F[U+j].  With dot(a, b) the adjacent-pair tree of ngacf_recommend_topk over products
  * rounded to fp32:

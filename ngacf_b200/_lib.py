@@ -86,6 +86,7 @@ SIGNATURES = {
     # top-K recommendation lists
     "ngacf_recommend_topk_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
     "ngacf_recommend_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, P, P, c_size_t, P]),
+    "ngacf_recommend_topk_offset": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, P, P, P, c_size_t, P]),
     # similar-item lists
     "ngacf_similar_items_topk_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
     "ngacf_similar_items_topk": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, P, P, P, c_size_t, P]),

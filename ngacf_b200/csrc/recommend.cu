@@ -9,6 +9,8 @@
 // for items), USERC the candidate rows (F[U..U+I) for items, F[0..U) for users).  Items for an item (similar-item lists) and users
 // for a user (similar-user lists) rank by the cosine dot * rn(q) * rn(j), with inverse norms from item_rnorm_kernel over the
 // candidate side, and exclude only q itself; users for an item (audience lists) rank by the plain score, excluding a CSR row.
+// OFF (user queries over items only) adds a per-item offset to the score before the threshold test (novelty-weighted lists), so
+// the selection, the compaction and the merge see the offset score and stay as they are.
 #include "topk_common.cuh"
 
 namespace ngacf {
@@ -63,20 +65,22 @@ __device__ __forceinline__ void rc_rank_user(int v, int K, float* Bs, int* Bi, i
 // The candidates are the items (NC = I, rows F[U+j]) or, USERC, the users (NC = U, rows F[j]); in_pool[NC] (NULL: all) restricts
 // them.  COS = ITEMQ != USERC (query and candidates on the same side, as the flags name opposite sides): the score is the cosine with rnorm[NC] the candidates' inverse norms and the
 // query itself is the only excluded candidate, excl_ptr / excl_items unused.  Otherwise excl_ptr / excl_items is a CSR over the
-// query ids of sorted excluded candidate ids (NULL: none) and rnorm is unused.  rnorm is the last parameter so that the user form
-// keeps its parameter offsets (and its SASS).
-template <int W, bool ITEMQ = false, bool USERC = false>
+// query ids of sorted excluded candidate ids (NULL: none) and rnorm is unused.  OFF: the score of (u, i) is dot + coff[i] (one fp32
+// add), coff[I] finite.  rnorm and then coff are the last parameters so that the forms without them keep their parameter offsets
+// (and their SASS).
+template <int W, bool ITEMQ = false, bool USERC = false, bool OFF = false>
 __global__ void __launch_bounds__(RC_THREADS) recommend_topk_kernel(const float* __restrict__ F, int U, int I, const int* __restrict__ users,
                                                                     int n_users, int K, const int* __restrict__ excl_ptr,
                                                                     const int* __restrict__ excl_items, const uint8_t* __restrict__ in_pool,
                                                                     int* __restrict__ top_ids, float* __restrict__ top_scores,
-                                                                    const float* __restrict__ rnorm) {
+                                                                    const float* __restrict__ rnorm, const float* __restrict__ coff) {
     // gridDim.y > 1 (few users): CTA (x, y) ranks its users on candidate slice y and writes the slice's list to row (uslot * gridDim.y + y)
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int L = W == 64 ? 6 : 7;
     // ITEMQ = true means item queries, USERC = true user candidates: they differ exactly when both sides are the same (items for an
     // item, users for a user), the cosine lists
     constexpr bool COS = ITEMQ != USERC;
+    static_assert(!(OFF && (ITEMQ || USERC)), "offsets are for user queries over item candidates");
     const int NC = USERC ? U : I;                                   // candidates, rows F[CB + j]
     const int CB = USERC ? 0 : U;
     float* It = reinterpret_cast<float*>(smem_raw);                 // [W d][64 candidates]
@@ -85,7 +89,7 @@ __global__ void __launch_bounds__(RC_THREADS) recommend_topk_kernel(const float*
     int* Bi = reinterpret_cast<int*>(Bs + RC_USERS * RC_CAP);       // [16 users][RC_CAP] buffered ids
     unsigned long long* Mk = reinterpret_cast<unsigned long long*>(Bi + RC_USERS * RC_CAP);   // [16] excluded candidates of the tile
     uint8_t* Pool = reinterpret_cast<uint8_t*>(Mk + RC_USERS);      // [64]
-    float* Rn = reinterpret_cast<float*>(Pool + RC_ITEMS);          // [64] inverse norms of the tile's candidates (COS only)
+    float* Rn = reinterpret_cast<float*>(Pool + RC_ITEMS);          // [64] the tile's inverse norms (COS) or score offsets (OFF)
     __shared__ int cursor[RC_USERS], cnt[RC_USERS], tau_i[RC_USERS], row_user[RC_USERS];
     __shared__ float tau_s[RC_USERS];
 
@@ -126,6 +130,7 @@ __global__ void __launch_bounds__(RC_THREADS) recommend_topk_kernel(const float*
         NGACF_LOAD_ITEM_TILE(W, RC_ITEMS, RC_THREADS, It, F, CB, NC, i0, tid);   // It[d][j] = F[CB+i0+j][d]
         if (tid < RC_ITEMS) Pool[tid] = (i0 + tid < NC) ? (in_pool ? in_pool[i0 + tid] : 1) : 0;
         if (COS && tid < RC_ITEMS) Rn[tid] = (i0 + tid < NC) ? rnorm[i0 + tid] : 0.f;
+        if (OFF && tid < RC_ITEMS) Rn[tid] = (i0 + tid < NC) ? coff[i0 + tid] : 0.f;
         if (!COS && il == 0) {        // excluded candidates of this query inside the tile (sorted list, monotone cursor)
             unsigned long long m = 0ull;
             int c = cursor[ul];
@@ -159,6 +164,7 @@ __global__ void __launch_bounds__(RC_THREADS) recommend_topk_kernel(const float*
             const int jj = il + 16 * j;
             const int item = i0 + jj;
             if (COS) sc[j] = __fmul_rn(__fmul_rn(sc[j], qrn), Rn[jj]);       // cosine: (dot * rn(q)) * rn(j), in this order
+            if (OFF) sc[j] = __fadd_rn(sc[j], Rn[jj]);
             const bool cand = user >= 0 && item < NC && Pool[jj] && (COS ? item != user : !((mk >> jj) & 1ull));
             if (cand && better(sc[j], item, ts, ti)) {
                 const int p = atomicAdd(&cnt[ul], 1);    // < RC_CAP: at most 64 entries per tile after the check above
@@ -269,33 +275,37 @@ extern "C" size_t ngacf_recommend_topk_workspace_bytes(int32_t width, int32_t I,
 // launch names for error messages, by [ITEMQ * 2 + USERC][merge]
 static const char* const RC_NAMES[4][2] = {{"recommend_topk", "recommend_topk merge"}, {"similar_users_topk", "similar_users_topk merge"},
                                            {"similar_items_topk", "similar_items_topk merge"}, {"audience_topk", "audience_topk merge"}};
+static const char* const RC_OFFSET_NAMES[2] = {"recommend_topk_offset", "recommend_topk_offset merge"};
 
-template <int W, bool ITEMQ, bool USERC>
+template <int W, bool ITEMQ, bool USERC, bool OFF>
 static int launch_recommend(const float* F, int U, int I, const int* users, int n_users, int K, const int* excl_ptr, const int* excl_items,
-                            const uint8_t* in_pool, int* top_ids, float* top_scores, const float* rnorm, int P, cudaStream_t st) {
-    constexpr bool COS = ITEMQ != USERC;          // same side: the cosine forms carry the tile's inverse norms
+                            const uint8_t* in_pool, int* top_ids, float* top_scores, const float* rnorm, const float* coff, int P,
+                            cudaStream_t st) {
+    // same side: the cosine forms carry the tile's inverse norms; the offset form the tile's offsets, in the same place
+    constexpr bool TILE_VALUES = (ITEMQ != USERC) || OFF;
     static PerDeviceOnce once;
     once.run([] {
-        cudaFuncSetAttribute(recommend_topk_kernel<W, ITEMQ, USERC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rc_smem<W, COS>());
+        cudaFuncSetAttribute(recommend_topk_kernel<W, ITEMQ, USERC, OFF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)rc_smem<W, TILE_VALUES>());
     });
-    recommend_topk_kernel<W, ITEMQ, USERC><<<dim3(ceil_div(n_users, RC_USERS), P), RC_THREADS, rc_smem<W, COS>(), st>>>(
-        F, U, I, users, n_users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, rnorm);
-    return check_launch(RC_NAMES[ITEMQ * 2 + USERC][0]);
+    recommend_topk_kernel<W, ITEMQ, USERC, OFF><<<dim3(ceil_div(n_users, RC_USERS), P), RC_THREADS, rc_smem<W, TILE_VALUES>(), st>>>(
+        F, U, I, users, n_users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, rnorm, coff);
+    return check_launch(OFF ? RC_OFFSET_NAMES[0] : RC_NAMES[ITEMQ * 2 + USERC][0]);
 }
 
 // one ranking pass (P == 1: straight into the outputs) or P candidate slices into the partial lists at `part` and their merge
-template <bool ITEMQ, bool USERC = false>
+template <bool ITEMQ, bool USERC = false, bool OFF = false>
 static int rank_and_merge(const float* F, int width, int U, int I, const int* queries, int n, int K, const int* excl_ptr,
-                          const int* excl_items, const uint8_t* in_pool, int* top_ids, float* top_scores, const float* rnorm, int P,
-                          char* part, cudaStream_t st) {
-    auto launch = width == 64 ? launch_recommend<64, ITEMQ, USERC> : launch_recommend<128, ITEMQ, USERC>;
-    if (P == 1) return launch(F, U, I, queries, n, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, rnorm, 1, st);
+                          const int* excl_items, const uint8_t* in_pool, int* top_ids, float* top_scores, const float* rnorm,
+                          const float* coff, int P, char* part, cudaStream_t st) {
+    auto launch = width == 64 ? launch_recommend<64, ITEMQ, USERC, OFF> : launch_recommend<128, ITEMQ, USERC, OFF>;
+    if (P == 1) return launch(F, U, I, queries, n, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, rnorm, coff, 1, st);
     int* part_ids = (int*)part;
     float* part_scores = (float*)(part + (size_t)n * P * K * 4);
-    const int rc = launch(F, U, I, queries, n, K, excl_ptr, excl_items, in_pool, part_ids, part_scores, rnorm, P, st);
+    const int rc = launch(F, U, I, queries, n, K, excl_ptr, excl_items, in_pool, part_ids, part_scores, rnorm, coff, P, st);
     if (rc != NGACF_OK) return rc;
     recommend_merge_kernel<<<n, RC_MERGE_THREADS, (size_t)P * K * 8, st>>>(part_ids, part_scores, P, K, top_ids, top_scores);
-    return check_launch(RC_NAMES[ITEMQ * 2 + USERC][1]);
+    return check_launch(OFF ? RC_OFFSET_NAMES[1] : RC_NAMES[ITEMQ * 2 + USERC][1]);
 }
 
 static char* align256(void* p) { return (char*)(((uintptr_t)p + 255) & ~(uintptr_t)255); }
@@ -314,8 +324,29 @@ extern "C" int ngacf_recommend_topk(const float* F, int32_t width, int32_t U, in
     }
     if (n_users == 0) return NGACF_OK;
     const int P = recommend_parts(n_users, I, K);
-    return rank_and_merge<false>(F, width, U, I, users, n_users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, nullptr, P,
-                                 P == 1 ? nullptr : align256(workspace), (cudaStream_t)stream);
+    return rank_and_merge<false>(F, width, U, I, users, n_users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, nullptr, nullptr,
+                                 P, P == 1 ? nullptr : align256(workspace), (cudaStream_t)stream);
+}
+
+// ngacf_recommend_topk with item_offset[i] added to every score of item i: the same launch shapes and the same workspace
+extern "C" int ngacf_recommend_topk_offset(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* users, int32_t n_users,
+                                           int32_t K, const int32_t* excl_ptr, const int32_t* excl_items, const uint8_t* in_pool,
+                                           const float* item_offset, int32_t* top_ids, float* top_scores, void* workspace,
+                                           size_t workspace_bytes, void* stream) {
+    if (!width_supported(width)) { set_error("recommend_topk_offset: width %d is not built (supported: 64, 128)", width); return NGACF_ERR_UNSUPPORTED; }
+    if (K < 1 || K > NGACF_RECOMMEND_MAX_K) { set_error("recommend_topk_offset: K = %d is outside 1..%d", K, NGACF_RECOMMEND_MAX_K); return NGACF_ERR_UNSUPPORTED; }
+    NGACF_REQUIRE(F && users && item_offset && top_ids && top_scores && U > 0 && I > 0 && n_users >= 0 &&
+                  (excl_ptr == nullptr) == (excl_items == nullptr),
+                  "recommend_topk_offset: null/empty argument (item_offset is required; excl_ptr and excl_items are both given or both NULL)");
+    const size_t need = ngacf_recommend_topk_workspace_bytes(width, I, n_users, K);
+    if (workspace_bytes < need || (need > 0 && workspace == nullptr)) {
+        set_error("recommend_topk_offset: workspace of %zu bytes, %zu needed", workspace_bytes, need);
+        return NGACF_ERR_WORKSPACE;
+    }
+    if (n_users == 0) return NGACF_OK;
+    const int P = recommend_parts(n_users, I, K);
+    return rank_and_merge<false, false, true>(F, width, U, I, users, n_users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores,
+                                              nullptr, item_offset, P, P == 1 ? nullptr : align256(workspace), (cudaStream_t)stream);
 }
 
 // the n inverse norms of the candidate side (256-byte aligned block), then the partial lists when the candidate range is split
@@ -352,8 +383,8 @@ extern "C" int ngacf_similar_items_topk(const float* F, int32_t width, int32_t U
     const int rc = row_rnorms(F, width, U, I, rnorm, st, "similar_items_topk norms");
     if (rc != NGACF_OK) return rc;
     const int P = recommend_parts(n_items, I, K);
-    return rank_and_merge<true>(F, width, U, I, items, n_items, K, nullptr, nullptr, in_pool, top_ids, top_scores, rnorm, P,
-                                w + rnorm_bytes(I), st);
+    return rank_and_merge<true>(F, width, U, I, items, n_items, K, nullptr, nullptr, in_pool, top_ids, top_scores, rnorm, nullptr,
+                                P, w + rnorm_bytes(I), st);
 }
 
 // audience lists: recommend_topk with the sides swapped, so the same workspace layout over the users
@@ -375,8 +406,8 @@ extern "C" int ngacf_audience_topk(const float* F, int32_t width, int32_t U, int
     }
     if (n_items == 0) return NGACF_OK;
     const int P = recommend_parts(n_items, U, K);
-    return rank_and_merge<true, true>(F, width, U, I, items, n_items, K, excl_ptr, excl_users, user_pool, top_ids, top_scores, nullptr, P,
-                                      P == 1 ? nullptr : align256(workspace), (cudaStream_t)stream);
+    return rank_and_merge<true, true>(F, width, U, I, items, n_items, K, excl_ptr, excl_users, user_pool, top_ids, top_scores, nullptr,
+                                      nullptr, P, P == 1 ? nullptr : align256(workspace), (cudaStream_t)stream);
 }
 
 // similar-user lists: similar_items_topk with the users' rows, so the same workspace layout over the users
@@ -402,6 +433,6 @@ extern "C" int ngacf_similar_users_topk(const float* F, int32_t width, int32_t U
     const int rc = row_rnorms(F, width, 0, U, rnorm, st, "similar_users_topk norms");
     if (rc != NGACF_OK) return rc;
     const int P = recommend_parts(n_users, U, K);
-    return rank_and_merge<false, true>(F, width, U, I, users, n_users, K, nullptr, nullptr, user_pool, top_ids, top_scores, rnorm, P,
-                                       w + rnorm_bytes(U), st);
+    return rank_and_merge<false, true>(F, width, U, I, users, n_users, K, nullptr, nullptr, user_pool, top_ids, top_scores, rnorm,
+                                       nullptr, P, w + rnorm_bytes(U), st);
 }

@@ -31,9 +31,15 @@ User-activity groups (group_metrics(G), the interaction sparsity levels of NGCF 
 sorted by (train degree, user id) ascending; with C_j the train degree summed over the users before user j and T the total, user j
 is in group min(G - 1, floor(G C_j / T)) (int64), G in 1..8.  The groups therefore hold about T / G train interactions each; one
 user with a very large degree can leave a group empty.  Per group: the number of evaluated users, their min / max train degree, their
-train interactions and the means over the group's users of the five metrics above and of novelty / arp at each cut-off."""
+train interactions and the means over the group's users of the five metrics above and of novelty / arp at each cut-off.
+
+Novelty-weighted lists (novelty_weight=w, any finite float): the lists rank by s(u, i) + off(i) with off(i) = float32(w * nov(i))
+(the fp64 product rounded once), the sum rounded to fp32 (ngacf_recommend_topk_offset).  Up to terms equal for every item this is
+s(u, i) - w log2(d_i + 1): a positive w moves popular items down, in the units of novelty@k.  The lists always come from the exact
+ranking (the tcgen05 scorer has no offsets), and every report above reads them unchanged."""
 from __future__ import annotations
 
+import math
 import numbers
 
 import numpy as np
@@ -96,6 +102,25 @@ def item_tables(inter: Interactions):
     return t
 
 
+def check_novelty_weight(w):
+    """-> w as a float; ValueError unless it is a finite real number"""
+    if isinstance(w, bool) or not isinstance(w, numbers.Real) or not math.isfinite(float(w)):
+        raise ValueError("the novelty weight must be a finite number, got %r" % (w,))
+    return float(w)
+
+
+def novelty_offsets(inter: Interactions, w):
+    """float32[I] device offsets off(i) = float32(w * nov(i)) of the novelty-weighted lists (fp64 product, rounded once); built once
+    per Interactions and weight"""
+    w = check_novelty_weight(w)
+    cache = inter.__dict__.setdefault("_novelty_offsets", {})
+    off = cache.get(w)
+    if off is None:
+        off = (w * item_tables(inter)[0]).to(torch.float32).contiguous()
+        cache[w] = off
+    return off
+
+
 def coverage_gini(counts, pool=None):
     """counts: (n_ks, I) exposure counts, pool: item ids (None: counts holds the pool's columns already) -> (coverage, gini) float64
     arrays of n_ks (definitions above)"""
@@ -130,23 +155,30 @@ def user_groups(inter: Interactions, G):
 
 
 class FullRankingEvaluator:
-    def __init__(self, inter: Interactions, ks, mode: str = "auto", users=None):
+    def __init__(self, inter: Interactions, ks, mode: str = "auto", users=None, novelty_weight=0.0):
         """ks: cut-offs (1..8 integers in 1..100).  mode: 'auto' (the tcgen05 AllNeg lists when they are long enough and the features
         64-wide, otherwise the exact ranking lists), 'tc' (the tcgen05 lists only) or 'exact' (always the ranking lists).
-        users: int32 device tensor of the users this rank evaluates (default: inter.eval_users)."""
+        users: int32 device tensor of the users this rank evaluates (default: inter.eval_users).  novelty_weight: w of the
+        novelty-weighted lists (module docstring); non-zero always ranks exactly at K = max(ks), so mode='tc' refuses it."""
         self.ks = check_ks(ks)
         if mode not in MODES:
             raise ValueError("mode must be one of %s, got %r" % ("/".join(MODES), mode))
         self.K = self.ks[-1]
         if mode == "tc" and self.K > ALLNEG_K:
             raise _lib.NgacfError("the tcgen05 AllNeg scorer ranks top-%d lists; cut-off %d needs mode='exact' or 'auto'" % (ALLNEG_K, self.K))
+        self.novelty_weight = check_novelty_weight(novelty_weight)
+        if mode == "tc" and self.novelty_weight != 0.0:
+            raise _lib.NgacfError("the tcgen05 AllNeg scorer has no score offsets; novelty_weight=%r needs mode='exact' or 'auto'"
+                                  % self.novelty_weight)
         self.inter = inter
         self.mode = mode
+        self._offset = novelty_offsets(inter, self.novelty_weight) if self.novelty_weight != 0.0 else None
         self.users = inter.eval_users if users is None else users.to(torch.int32).contiguous()
         dev = inter.device
         n = self.users.numel()
         nc = len(METRICS) * len(self.ks)
-        self._allneg = AllNegEvaluator(inter, mode, self.users) if mode != "exact" and self.K <= ALLNEG_K else None
+        use_tc = mode != "exact" and self.K <= ALLNEG_K and self._offset is None
+        self._allneg = AllNegEvaluator(inter, mode, self.users) if use_tc else None
         self._ids = torch.empty((max(n, 1), self.K), dtype=torch.int32, device=dev)
         self._scores = torch.empty((max(n, 1), self.K), dtype=torch.float32, device=dev)
         self._list_ws = None
@@ -172,7 +204,7 @@ class FullRankingEvaluator:
             self._list_ws = torch.empty(ops.recommend_topk_workspace_bytes(width, it.I, n, self.K), dtype=torch.uint8, device=Z.device)
         ops.final_features(Z, self.F)
         ops.recommend_topk(self.F, it.U, it.I, self.users, self.K, it.train_ptr, it.train_items, it.in_pool, self._ids, self._scores,
-                           self._list_ws)
+                           self._list_ws, self._offset)
         self.source = "list"
 
     @property

@@ -306,11 +306,17 @@ def recommend_topk_workspace_bytes(width, I, n_users, K):
     return int(_lib.load().ngacf_recommend_topk_workspace_bytes(int(width), int(I), int(n_users), int(K)))
 
 
-def recommend_topk(F, U, I, users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, ws):
+def recommend_topk(F, U, I, users, K, excl_ptr, excl_items, in_pool, top_ids, top_scores, ws, item_offset=None):
     """top-K lists of `users` (int32) from final features F (U+I, 64 or 128); excl_ptr/excl_items (CSR over users) and in_pool may be
-    None; ws: uint8 tensor of recommend_topk_workspace_bytes(...) bytes (may be empty)"""
-    _lib.call("ngacf_recommend_topk", _p(F), int(F.shape[-1]), int(U), int(I), _p(users), users.numel(), int(K), _p(excl_ptr),
-              _p(excl_items), _p(in_pool), _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
+    None; ws: uint8 tensor of recommend_topk_workspace_bytes(...) bytes (may be empty).  item_offset: float32[I] of finite values
+    added to every score of each item (ngacf_recommend_topk_offset), None for the plain scores"""
+    if item_offset is None:
+        _lib.call("ngacf_recommend_topk", _p(F), int(F.shape[-1]), int(U), int(I), _p(users), users.numel(), int(K), _p(excl_ptr),
+                  _p(excl_items), _p(in_pool), _p(top_ids), _p(top_scores), _p(ws) if ws.numel() else None, ws.numel(), _s())
+    else:
+        _lib.call("ngacf_recommend_topk_offset", _p(F), int(F.shape[-1]), int(U), int(I), _p(users), users.numel(), int(K),
+                  _p(excl_ptr), _p(excl_items), _p(in_pool), _p(item_offset), _p(top_ids), _p(top_scores),
+                  _p(ws) if ws.numel() else None, ws.numel(), _s())
 
 
 def similar_items_topk_workspace_bytes(width, I, n_items, K):

@@ -126,12 +126,20 @@ class Recommender:
             self._user_side = (ptr, users, pool)
         return self._user_side
 
-    def __call__(self, users, K: int = 20):
-        """-> (ids int64 (n, K), scores float32 (n, K)) on the GPU; rows with fewer than K candidates end in id -1 / score 0.0"""
+    def __call__(self, users, K: int = 20, novelty_weight=0.0):
+        """-> (ids int64 (n, K), scores float32 (n, K)) on the GPU; rows with fewer than K candidates end in id -1 / score 0.0.
+        novelty_weight w != 0: novelty-weighted lists, ranked (and scored) by s(u, i) + float32(w * nov(i)) with the item novelty of
+        the train split of `inter` (ngacf_b200.cutoff_eval.novelty_offsets); a positive w moves popular items down.  w = 0 is the
+        plain ranking."""
+        from .cutoff_eval import check_novelty_weight, novelty_offsets
         K = self._k(K)
+        w = check_novelty_weight(novelty_weight)
+        if w != 0.0 and self.inter is None:
+            raise ValueError("novelty_weight needs the interactions (inter=...): the item novelty comes from their train split")
+        off = novelty_offsets(self.inter, w) if w != 0.0 else None
         u = self._ids(users, self.U, "user")
         return self._lists(u, K, self.I, ops.recommend_topk_workspace_bytes, lambda q, K, ids, scores, ws: ops.recommend_topk(
-            self.F, self.U, self.I, q, K, self.excl_ptr, self.excl_items, self.in_pool, ids, scores, ws))
+            self.F, self.U, self.I, q, K, self.excl_ptr, self.excl_items, self.in_pool, ids, scores, ws, off))
 
     def similar_items(self, items, K: int = 20):
         """-> (ids int64 (n, K), scores float32 (n, K)) on the GPU: for each query item the K items of highest cosine similarity of the

@@ -20,6 +20,10 @@ or test item as candidates, minus those --exclude leaves out for the item), writ
 `item<TAB>rank<TAB>user<TAB>score`; with --similar-users all|3,17,42|@file the users most similar to those users (cosine, as for
 items), written to ..._similarusers{K}.tsv as `user<TAB>rank<TAB>similar_user<TAB>score`.  At most one of the three flags is given,
 --users stays at its default with any of them, and --exclude too with --similar-items or --similar-users.
+
+With --novelty-weight w (user lists only) the user lists rank by score + float32(w * novelty(item)), the item novelty of the train
+split (Recommender(..., novelty_weight=w)); a positive w moves popular items down.  The scores written are those offset scores and
+the default output name gains _nw{w}, e.g. recs/SPUIGACF_ml100k_010_top50_nw1.0.tsv.
 """
 import os
 import sys
@@ -29,6 +33,7 @@ import numpy as np
 import torch
 
 import run_Gowalla as R
+from ngacf_b200.cutoff_eval import check_novelty_weight
 from ngacf_b200.recommend import EXCLUDE, MAX_K, Recommender
 
 
@@ -45,6 +50,8 @@ def build_parser():
                    help="rank users for these items (--exclude applies per item): all, a comma-separated id list, or @FILE")
     p.add_argument("--similar-users", type=str, default=None,
                    help="rank users like these users: all, a comma-separated id list, or @FILE")
+    p.add_argument("--novelty-weight", type=float, default=0.0,
+                   help="w: rank the user lists by score + w * novelty(item) (a positive w moves popular items down); 0 is the plain ranking")
     p.add_argument("--out", type=str, default=None,
                    help="output TSV (default recs/{model}_{dataset}_{N:03d}_top{K}.tsv, with --similar-items ..._similar{K}.tsv, "
                         "--audience ..._audience{K}.tsv, --similar-users ..._similarusers{K}.tsv)")
@@ -74,7 +81,8 @@ def parse_ids(spec, flag="--users", words=("eval", "all")):
 
 def default_out(args):
     kind = next((tag for dest, _, tag in QUERY_FLAGS if getattr(args, dest) is not None), "top")
-    return os.path.join("recs", "{}_{}_{:03d}_{}{}.tsv".format(args.model, args.dataset, args.resume_from, kind, args.topk))
+    nw = "_nw{}".format(args.novelty_weight) if args.novelty_weight != 0.0 else ""
+    return os.path.join("recs", "{}_{}_{:03d}_{}{}{}.tsv".format(args.model, args.dataset, args.resume_from, kind, args.topk, nw))
 
 
 def parse_args(argv=None):
@@ -94,6 +102,9 @@ def parse_args(argv=None):
     given = [flag for dest, flag, _ in QUERY_FLAGS if getattr(args, dest) is not None]
     if len(given) > 1:
         raise ValueError("%s: give at most one of them" % " and ".join(given))
+    args.novelty_weight = check_novelty_weight(args.novelty_weight)
+    if given and args.novelty_weight != 0.0:
+        raise ValueError("--novelty-weight applies to the user lists only; drop it with %s" % given[0])
     args.item_ids = args.audience_ids = args.similar_user_ids = None
     if args.audience is not None:
         if args.users != "eval":
@@ -179,12 +190,13 @@ def main(args):
     rec = Recommender(load_model(args, userNum, itemNum), adj, inter, args.exclude)
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    ids, scores = rec(users, args.topk)
+    ids, scores = rec(users, args.topk, novelty_weight=args.novelty_weight)
     torch.cuda.synchronize()
     ms = (time.perf_counter() - t0) * 1e3
     ids, scores = ids.cpu().numpy(), scores.cpu().numpy()
     write_tsv(args.out, users, ids, scores)
-    print("recommend: %d users, top-%d, %.2f ms -> %s" % (users.size, args.topk, ms, args.out))
+    nw = ", novelty weight %r" % args.novelty_weight if args.novelty_weight != 0.0 else ""
+    print("recommend: %d users, top-%d%s, %.2f ms -> %s" % (users.size, args.topk, nw, ms, args.out))
     return users, ids, scores
 
 

@@ -8,6 +8,7 @@ TensorBoard scalar tags (:139,149-153).  Example (the reference's README smoke t
 """
 import argparse
 import ast
+import math
 import os
 import sys
 import time
@@ -114,34 +115,62 @@ def main(args):
 
 def full_ranking(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0):
     """--eval_ks: full-ranking metrics with the standard definitions (ngacf_b200.cutoff_eval), printed by rank 0 as one line of plain
-    Python values and logged as full@K/<metric>"""
+    Python values and logged as full@K/<metric>; then the same lines for the lists of each --eval_novelty_weights weight w, printed
+    as `epoch:{e} novelty weight {w} ...` and logged under novelty{w}/"""
     if not args.eval_ks:
         return
-    res = eval_full_ranking(model, test_df, test_pos_neg, adj, args.eval_ks, args.parallel)
+    rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, 0.0)
+    for w in args.eval_novelty_weights or ():
+        rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, w)
+
+
+def rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, w):
+    """full_ranking's lines for the lists of novelty weight w (0: the plain lists)"""
+    line = "epoch:{} ".format(epoch) if w == 0.0 else "epoch:{} novelty weight {} ".format(epoch, w)
+    tag = "" if w == 0.0 else "novelty{}/".format(w)
+    res = eval_full_ranking(model, test_df, test_pos_neg, adj, args.eval_ks, args.parallel, novelty_weight=w)
     for i, K in enumerate(res["ks"]):
         for name in ("precision", "recall", "ndcg", "hit_ratio", "mrr"):
-            summaryWriter.add_scalar("full@{}/{}".format(K, name), res[name][i], epoch)
+            summaryWriter.add_scalar("{}full@{}/{}".format(tag, K, name), res[name][i], epoch)
     if rank0:
-        print("epoch:{} full-ranking metrics:{}".format(epoch, _plain(res)))
+        print("{}full-ranking metrics:{}".format(line, _plain(res)))
     if not (args.eval_beyond or args.eval_groups):
         return
     # --eval_beyond / --eval_groups: reports over the lists eval_full_ranking just ranked (every rank takes part in the all-reduce)
-    rep = list_reports(model, args.eval_beyond, args.eval_groups)
+    rep = list_reports(model, args.eval_beyond, args.eval_groups, novelty_weight=w)
     if rep["beyond"] is not None:
         b = rep["beyond"]
         for i, K in enumerate(b["ks"]):
             for name in ("coverage", "gini", "novelty", "arp"):
-                summaryWriter.add_scalar("beyond@{}/{}".format(K, name), b[name][i], epoch)
+                summaryWriter.add_scalar("{}beyond@{}/{}".format(tag, K, name), b[name][i], epoch)
         if rank0:
-            print("epoch:{} beyond-accuracy metrics:{}".format(epoch, _plain(b)))
+            print("{}beyond-accuracy metrics:{}".format(line, _plain(b)))
     if rep["groups"] is not None:
         g = rep["groups"]
         for j in range(g["groups"]):
             for i, K in enumerate(g["ks"]):
                 for name in ("precision", "recall", "ndcg", "hit_ratio", "mrr", "novelty", "arp"):
-                    summaryWriter.add_scalar("group{}@{}/{}".format(j, K, name), g[name][j][i], epoch)
+                    summaryWriter.add_scalar("{}group{}@{}/{}".format(tag, j, K, name), g[name][j][i], epoch)
         if rank0:
-            print("epoch:{} user-group metrics:{}".format(epoch, _plain(g)))
+            print("{}user-group metrics:{}".format(line, _plain(g)))
+
+
+def parse_novelty_weights(text):
+    """'0.5,1,2' -> [0.5, 1.0, 2.0]; ValueError unless it is 1..8 distinct finite non-zero numbers"""
+    try:
+        ws = [float(x) for x in str(text).split(",")]
+    except ValueError:
+        raise ValueError("--eval_novelty_weights must be a comma-separated list of numbers, got %r" % text) from None
+    if not 1 <= len(ws) <= MAX_NOVELTY_WEIGHTS:
+        raise ValueError("--eval_novelty_weights takes 1..%d weights, got %d" % (MAX_NOVELTY_WEIGHTS, len(ws)))
+    if not all(math.isfinite(w) and w != 0.0 for w in ws):
+        raise ValueError("--eval_novelty_weights must be finite and non-zero (the plain lists are reported anyway), got %r" % text)
+    if len(set(ws)) != len(ws):
+        raise ValueError("--eval_novelty_weights must be distinct, got %r" % text)
+    return ws
+
+
+MAX_NOVELTY_WEIGHTS = 8
 
 
 def _plain(res):
@@ -180,6 +209,9 @@ def build_parser():
     p.add_argument("--eval_groups", type=str, default=None,
                    help="G in 1..8: also report the --eval_ks metrics, novelty and popularity per group of users split by train degree "
                         "into G groups of about equal train interactions (NGCF section 4.3.2)")
+    p.add_argument("--eval_novelty_weights", type=str, default=None,
+                   help="e.g. 0.5,1,2 (1..8 distinct non-zero numbers): also rank novelty-weighted lists, by score + w * novelty(item), "
+                        "and report the --eval_ks metrics (and --eval_beyond / --eval_groups) of each weight's lists")
     return p
 
 
@@ -212,6 +244,10 @@ def parse_args(argv=None):
         args.eval_groups = check_groups(G)
     if (args.eval_beyond or args.eval_groups) and not args.eval_ks:
         raise ValueError("--eval_beyond and --eval_groups report at the --eval_ks cut-offs; give --eval_ks as well")
+    if args.eval_novelty_weights is not None:
+        args.eval_novelty_weights = parse_novelty_weights(args.eval_novelty_weights)
+        if not args.eval_ks:
+            raise ValueError("--eval_novelty_weights reports at the --eval_ks cut-offs; give --eval_ks as well")
     if args.parallel and args.embedSize != 64:
         raise ValueError("--parallel True is built for --embedSize 64 only; train --embedSize %d on one GPU (--parallel False)" % args.embedSize)
     return args

@@ -200,21 +200,23 @@ def eval_neg_all(model, batch_size, test_df, test_pos_neg, adj, itemNum, is_para
         return ev(Z)
 
 
-def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="auto"):
+def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="auto", novelty_weight=0.0):
     """Full-ranking metrics at the cut-offs `ks` (up to 8 of 1..100) with the standard definitions: precision, recall, NDCG with the
     ideal DCG of min(|test|, k) hits, hit ratio and MRR, averaged over the users with train and test items
     (ngacf_b200.cutoff_eval).  Returns FullRankingEvaluator.metrics()'s dict.  is_parallel under torchrun: the users are sharded over
-    the ranks and the sums merged, as in eval_neg_all."""
-    from ngacf_b200.cutoff_eval import FullRankingEvaluator, check_ks
+    the ranks and the sums merged, as in eval_neg_all.  novelty_weight w != 0: the metrics of the novelty-weighted lists
+    (FullRankingEvaluator(novelty_weight=w)), from an evaluator cached per weight next to the plain one."""
+    from ngacf_b200.cutoff_eval import FullRankingEvaluator, check_ks, check_novelty_weight
     m = _unwrap(model)
     model.eval()
     _require_plain(m, "eval_full_ranking")
     ks = check_ks(ks)
+    w = check_novelty_weight(novelty_weight)
     inter = _interactions(model, None, test_pos_neg, test_df)
     adj_t = _device_adj(model, adj)
     with torch.no_grad():
         Z = m.propagate(adj_t)
-        ev = getattr(m, "_full_evaluator", None)
+        ev = _full_evaluator(m, w)
         world = _world() if is_parallel else 1
         if ev is None or ev.inter is not inter or ev.mode != mode or ev.ks != ks or getattr(ev, "world", 1) != world:
             users = None
@@ -222,20 +224,33 @@ def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="
                 import torch.distributed as dist
                 from ngacf_b200.dist import shard_eval_users
                 users = shard_eval_users(inter.eval_users, dist.get_rank(), world)
-            ev = FullRankingEvaluator(inter, ks, mode, users=users)
+            ev = FullRankingEvaluator(inter, ks, mode, users=users, novelty_weight=w)
             ev.world = world
-            m._full_evaluator = ev
+            if w == 0.0:
+                m._full_evaluator = ev
+            else:
+                m.__dict__.setdefault("_novelty_evaluators", {})[w] = ev
         return ev(Z)
 
 
-def list_reports(model, beyond=True, groups=None):
+def _full_evaluator(m, w):
+    """the evaluator eval_full_ranking cached for novelty weight w (0: the plain one), or None"""
+    if w == 0.0:
+        return getattr(m, "_full_evaluator", None)
+    return m.__dict__.get("_novelty_evaluators", {}).get(w)
+
+
+def list_reports(model, beyond=True, groups=None, novelty_weight=0.0):
     """The beyond-accuracy metrics (coverage, Gini of the item exposure, novelty, ARP) and the metrics per user-activity group
     (NGCF section 4.3.2) of the lists the preceding eval_full_ranking call ranked, from the evaluator it cached: no second
     propagation or ranking.  Returns {"beyond": FullRankingEvaluator.list_metrics() or None, "groups":
-    FullRankingEvaluator.group_metrics(groups) or None}.  Under torchrun every rank calls it (the counts and sums are all-reduced)."""
-    ev = getattr(_unwrap(model), "_full_evaluator", None)
+    FullRankingEvaluator.group_metrics(groups) or None}.  novelty_weight: read the lists of the eval_full_ranking call with that
+    weight.  Under torchrun every rank calls it (the counts and sums are all-reduced)."""
+    from ngacf_b200.cutoff_eval import check_novelty_weight
+    ev = _full_evaluator(_unwrap(model), check_novelty_weight(novelty_weight))
     if ev is None or ev.source is None:
-        raise RuntimeError("list_reports: call eval_full_ranking first; it ranks the lists these reports read")
+        raise RuntimeError("list_reports: call eval_full_ranking first (with the same novelty_weight); it ranks the lists these "
+                           "reports read")
     return {"beyond": ev.list_metrics() if beyond else None, "groups": ev.group_metrics(groups) if groups else None}
 
 
