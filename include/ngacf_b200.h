@@ -539,6 +539,38 @@ size_t ngacf_group_sums_workspace_bytes(int32_t n_rows, int32_t n_cols, int32_t 
 int ngacf_group_sums(const double* rows, int32_t n_rows, int32_t n_cols, const int32_t* group, int32_t G, double* sums, void* workspace,
                      size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Diversity of ranked lists from the cosine of the items' final features.  F as for ngacf_recommend_topk (width 64 or 128); an entry
+ * of a list is valid when its id lies in [0, I), any other id (-1 padding) is skipped.  With dot, rn(j) and the fp32 products of
+ * ngacf_similar_items_topk, the similarity of two entries x, y of one list, x the one of lower rank (earlier position), is
+ *   sim(x, y) = (dot(F[U+x], F[U+y]) * rn(x)) * rn(y), the similar-item score of query x, candidate y (computed once per pair).
+ *
+ * Intra-list diversity.  Row j of top_ids ([n_rows][K_list], K_list 1..NGACF_RECOMMEND_MAX_K) is one list; ks: HOST array of n_ks
+ * cut-offs, strictly increasing in 1..K_list (by value; checked as in ngacf_list_stats).  For cut-off q, with v_1..v_m the valid
+ * entries among the first ks[q] in rank order and t_ab = 1.0 - (double)sim(v_a, v_b):
+ *   r_b = sum over a < b of t_ab, in fp64, a ascending from 0.0;  num = sum over b = 2..m of r_b, b ascending from 0.0;
+ *   rows[j][q] = num / (m (m - 1) / 2), one fp64 division; 0 when m < 2.
+ *
+ * MMR re-ranking (maximal marginal relevance).  Row j of cand_ids / cand_scores ([n_rows][N], N 1..NGACF_RECOMMEND_MAX_K) is one
+ * candidate list (normally the top-N of ngacf_recommend_topk); K in 1..N picks are made greedily, lam in [0, 1], oml = 1 - lam (fp32):
+ *   rel(c) = (s_c - smin) / (smax - smin) over the valid candidates' scores when smax > smin, else 0 (fp32, round to nearest);
+ *   m(c)   = the max of sim(c, p) over the picks p so far (the argument of lower candidate position first), 0 before the first pick;
+ *   the next pick is the unpicked valid candidate of largest lam * rel(c) - oml * m(c) (each operation rounded to fp32), ties to the
+ *   lower candidate position, until K picks are made or the valid candidates run out.  A value that is NaN (non-finite scores or
+ *   features, e.g. finite scores spanning more than FLT_MAX, whose rel is inf / inf) ranks below every number, ties again to the
+ *   lower position, so every valid candidate is picked in turn; smax / smin skip NaN scores (fmaxf / fminf), and m(c) takes the max by fmaxf (a NaN similarity is skipped).  Row j of out_ids / out_scores ([n_rows][K])
+ *   holds the picks in pick order with their candidate scores (not sorted), padded with -1 / 0.0.  lam = 1 returns the first K valid
+ *   candidates of a list sorted by score descending, in order; a row does not depend on the other rows of the call.
+ *
+ * A width other than 64 / 128, K_list / N outside 1..NGACF_RECOMMEND_MAX_K, K outside 1..N or bad cut-offs return
+ * NGACF_ERR_UNSUPPORTED; NULL pointers or a lam that is NaN or outside [0, 1] return NGACF_ERR_INVALID_ARG; both before any launch.
+ * n_rows == 0 is a no-op.  Deterministic; no workspace, no allocation, no synchronisation (CUDA-graph capturable).
+ * ------------------------------------------------------------------------------------------- */
+int ngacf_list_diversity(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* top_ids, int32_t K_list, int32_t n_rows,
+                         const int32_t* ks, int32_t n_ks, double* rows, void* stream);
+int ngacf_mmr_rerank(const float* F, int32_t width, int32_t U, int32_t I, const int32_t* cand_ids, const float* cand_scores,
+                     int32_t n_rows, int32_t N, int32_t K, float lam, int32_t* out_ids, float* out_scores, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -102,6 +102,9 @@ SIGNATURES = {
     "ngacf_list_stats": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, P, c_int32, P, P, P]),
     "ngacf_group_sums_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32]),
     "ngacf_group_sums": (c_int32, [P, c_int32, c_int32, P, c_int32, P, P, c_size_t, P]),
+    # intra-list diversity and MMR re-ranking
+    "ngacf_list_diversity": (c_int32, [P, c_int32, c_int32, c_int32, P, c_int32, c_int32, P, c_int32, P, P]),
+    "ngacf_mmr_rerank": (c_int32, [P, c_int32, c_int32, c_int32, P, P, c_int32, c_int32, c_int32, c_float, P, P, P]),
 }
 
 _lib = None

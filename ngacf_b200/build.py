@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libngacf_b200.so")
 SOURCES = ["util.cu", "graph_build.cu", "propagate_fwd.cu", "propagate_bwd.cu", "pruned_stage.cu", "laplacian.cu", "spgat.cu", "transform_bwd_split.cu", "transform_tc.cu", "train_misc.cu", "neg_sampling.cu", "eval_topk.cu",
-           "eval_topk_tc.cu", "recommend.cu", "cutoff_metrics.cu", "list_stats.cu"]
+           "eval_topk_tc.cu", "recommend.cu", "cutoff_metrics.cu", "list_stats.cu", "diversity.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]
 

@@ -36,7 +36,17 @@ train interactions and the means over the group's users of the five metrics abov
 Novelty-weighted lists (novelty_weight=w, any finite float): the lists rank by s(u, i) + off(i) with off(i) = float32(w * nov(i))
 (the fp64 product rounded once), the sum rounded to fp32 (ngacf_recommend_topk_offset).  Up to terms equal for every item this is
 s(u, i) - w log2(d_i + 1): a positive w moves popular items down, in the units of novelty@k.  The lists always come from the exact
-ranking (the tcgen05 scorer has no offsets), and every report above reads them unchanged."""
+ranking (the tcgen05 scorer has no offsets), and every report above reads them unchanged.
+
+Intra-list diversity (diversity_metrics(), csrc/diversity.cu) of the same lists, with sim(x, y) the cosine of the items' final
+features as the similar-item lists compute it (x the entry of lower rank) and v_1..v_m the valid entries among the first k:
+    ild@k = sum over b = 2..m of (sum over a < b of (1 - sim(v_a, v_b))) / (m (m - 1) / 2), 0 when m < 2
+summed in fp64, a ascending inside b ascending, one division; averaged over the evaluated users with the divisor of metrics().
+
+MMR-diversified lists (mmr_lambda=lam in [0, 1]): rank() first ranks N = mmr_candidates candidates exactly (with the novelty offsets
+when novelty_weight is set), then picks K = max(ks) of them greedily by lam * rel(c) - (1 - lam) * max similarity to the picks so
+far, rel being the candidate score min-max normalised over the row (ngacf_mmr_rerank).  lam = 1 gives the exact lists; every report
+above reads the re-ranked lists unchanged."""
 from __future__ import annotations
 
 import math
@@ -121,6 +131,20 @@ def novelty_offsets(inter: Interactions, w):
     return off
 
 
+def check_mmr_lambda(lam):
+    """-> lam as a float; ValueError unless it is a real number in [0, 1]"""
+    if isinstance(lam, bool) or not isinstance(lam, numbers.Real) or not 0.0 <= float(lam) <= 1.0:
+        raise ValueError("the MMR lambda must be a number in [0, 1], got %r" % (lam,))
+    return float(lam)
+
+
+def check_mmr_candidates(n, K):
+    """-> n as an int; ValueError unless it is an integer in K..100"""
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not K <= int(n) <= MAX_K:
+        raise ValueError("the MMR candidates must be an integer in %d..%d (the list length .. 100), got %r" % (K, MAX_K, n))
+    return int(n)
+
+
 def coverage_gini(counts, pool=None):
     """counts: (n_ks, I) exposure counts, pool: item ids (None: counts holds the pool's columns already) -> (coverage, gini) float64
     arrays of n_ks (definitions above)"""
@@ -155,11 +179,13 @@ def user_groups(inter: Interactions, G):
 
 
 class FullRankingEvaluator:
-    def __init__(self, inter: Interactions, ks, mode: str = "auto", users=None, novelty_weight=0.0):
+    def __init__(self, inter: Interactions, ks, mode: str = "auto", users=None, novelty_weight=0.0, mmr_lambda=None, mmr_candidates=100):
         """ks: cut-offs (1..8 integers in 1..100).  mode: 'auto' (the tcgen05 AllNeg lists when they are long enough and the features
         64-wide, otherwise the exact ranking lists), 'tc' (the tcgen05 lists only) or 'exact' (always the ranking lists).
         users: int32 device tensor of the users this rank evaluates (default: inter.eval_users).  novelty_weight: w of the
-        novelty-weighted lists (module docstring); non-zero always ranks exactly at K = max(ks), so mode='tc' refuses it."""
+        novelty-weighted lists (module docstring); non-zero always ranks exactly at K = max(ks), so mode='tc' refuses it.
+        mmr_lambda: lam of the MMR-diversified lists (module docstring), re-ranked from the exact top mmr_candidates (max(ks)..100);
+        None: no re-ranking.  mode='tc' refuses it too."""
         self.ks = check_ks(ks)
         if mode not in MODES:
             raise ValueError("mode must be one of %s, got %r" % ("/".join(MODES), mode))
@@ -170,6 +196,11 @@ class FullRankingEvaluator:
         if mode == "tc" and self.novelty_weight != 0.0:
             raise _lib.NgacfError("the tcgen05 AllNeg scorer has no score offsets; novelty_weight=%r needs mode='exact' or 'auto'"
                                   % self.novelty_weight)
+        self.mmr_lambda = None if mmr_lambda is None else check_mmr_lambda(mmr_lambda)
+        self.mmr_candidates = check_mmr_candidates(mmr_candidates, self.K)
+        if mode == "tc" and self.mmr_lambda is not None:
+            raise _lib.NgacfError("the tcgen05 AllNeg scorer has no MMR re-ranking; mmr_lambda=%r needs mode='exact' or 'auto'"
+                                  % self.mmr_lambda)
         self.inter = inter
         self.mode = mode
         self._offset = novelty_offsets(inter, self.novelty_weight) if self.novelty_weight != 0.0 else None
@@ -177,11 +208,15 @@ class FullRankingEvaluator:
         dev = inter.device
         n = self.users.numel()
         nc = len(METRICS) * len(self.ks)
-        use_tc = mode != "exact" and self.K <= ALLNEG_K and self._offset is None
+        use_tc = mode != "exact" and self.K <= ALLNEG_K and self._offset is None and self.mmr_lambda is None
         self._allneg = AllNegEvaluator(inter, mode, self.users) if use_tc else None
         self._ids = torch.empty((max(n, 1), self.K), dtype=torch.int32, device=dev)
         self._scores = torch.empty((max(n, 1), self.K), dtype=torch.float32, device=dev)
         self._list_ws = None
+        if self.mmr_lambda is not None:      # the candidate lists the re-ranking reads
+            self._cand_ids = torch.empty((max(n, 1), self.mmr_candidates), dtype=torch.int32, device=dev)
+            self._cand_scores = torch.empty((max(n, 1), self.mmr_candidates), dtype=torch.float32, device=dev)
+        self._div_rows = None
         self._rows = torch.zeros((n, nc), dtype=torch.float64, device=dev)
         self._sums = torch.zeros(nc + 1, dtype=torch.float64, device=dev)      # the metric sums, then the number of users
         self._metric_ws = torch.empty(ops.cutoff_metrics_workspace_bytes(n, len(self.ks)), dtype=torch.uint8, device=dev)
@@ -201,15 +236,25 @@ class FullRankingEvaluator:
         if self.F is None or self.F.shape != Z.shape:
             self.F = torch.empty_like(Z)
             n = self.users.numel()
-            self._list_ws = torch.empty(ops.recommend_topk_workspace_bytes(width, it.I, n, self.K), dtype=torch.uint8, device=Z.device)
+            K = self.K if self.mmr_lambda is None else self.mmr_candidates
+            self._list_ws = torch.empty(ops.recommend_topk_workspace_bytes(width, it.I, n, K), dtype=torch.uint8, device=Z.device)
         ops.final_features(Z, self.F)
-        ops.recommend_topk(self.F, it.U, it.I, self.users, self.K, it.train_ptr, it.train_items, it.in_pool, self._ids, self._scores,
-                           self._list_ws, self._offset)
-        self.source = "list"
+        if self.mmr_lambda is None:
+            ops.recommend_topk(self.F, it.U, it.I, self.users, self.K, it.train_ptr, it.train_items, it.in_pool, self._ids, self._scores,
+                               self._list_ws, self._offset)
+            self.source = "list"
+            return
+        n = self.users.numel()
+        ops.recommend_topk(self.F, it.U, it.I, self.users, self.mmr_candidates, it.train_ptr, it.train_items, it.in_pool,
+                           self._cand_ids, self._cand_scores, self._list_ws, self._offset)
+        if n:
+            ops.mmr_rerank(self.F, it.U, it.I, self._cand_ids[:n], self._cand_scores[:n], self.K, self.mmr_lambda, self._ids, self._scores)
+        self.source = "mmr"
 
     @property
     def top_ids(self):
-        """(n_users, L) int32 lists of the last rank(), -1 padded: L = 20 from the tcgen05 source, max(ks) otherwise"""
+        """(n_users, L) int32 lists of the last rank(), -1 padded: L = 20 from the tcgen05 source, max(ks) otherwise (the exact
+        ranking, source "list", or its MMR re-ranking, source "mmr")"""
         if self.source is None:
             raise RuntimeError("FullRankingEvaluator: call rank(Z) first")
         return self._allneg.top_ids if self.source == "tc" else self._ids
@@ -344,3 +389,26 @@ class FullRankingEvaluator:
         for q, name in enumerate(LIST_VALUES):
             out[name] = lst[:, q * nk:(q + 1) * nk].copy()
         return out
+
+    # ---- intra-list diversity over the lists of the last rank() ----
+    def diversity_metrics(self):
+        """{"ks", "ild": float64 array of len(ks), "n_users"}: the mean intra-list diversity (module docstring) over the evaluated
+        users of every rank (sums all-reduced when sharded; every rank returns the same dict), from the final features rank()
+        computed"""
+        from .dist import allreduce_sums
+        top = self.top_ids
+        self._list_setup()
+        it = self.inter
+        n, nk = self.users.numel(), len(self.ks)
+        if self._div_rows is None:
+            self._div_rows = torch.zeros((n, nk), dtype=torch.float64, device=it.device)
+        F = self._allneg.F if self.source == "tc" else self.F
+        if n:
+            ops.list_diversity(F, it.U, it.I, top[:n], self.ks, self._div_rows)
+        buf = self._gsums[:nk + 1]
+        ops.group_sums(self._div_rows, self._one_group[:n], 1, buf[:nk].view(1, nk), self._gs_ws)
+        buf[-1] = float(n)
+        allreduce_sums(buf)
+        s = buf.cpu().numpy()
+        n_all = int(round(s[-1]))
+        return {"ks": list(self.ks), "ild": s[:nk] / max(n_all, 1), "n_users": n_all}

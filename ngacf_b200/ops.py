@@ -391,6 +391,26 @@ def group_sums(rows, group, G, sums, ws):
               ws.numel() * ws.element_size(), _s())
 
 
+def list_diversity(F, U, I, top_ids, ks, rows):
+    """intra-list diversity of the ranked lists top_ids (n, K_list) int32 (-1 padded; ids outside [0, I) are skipped) at the cut-offs
+    `ks` (host ints, strictly increasing, <= K_list), from the cosine of the items' rows of F (U+I, 64 or 128): rows float64
+    (n, len(ks))"""
+    for t in (F, top_ids, rows):
+        _lib.require_cuda(t)
+    ka = (ctypes.c_int32 * len(ks))(*[int(k) for k in ks])
+    _lib.call("ngacf_list_diversity", _p(F), int(F.shape[-1]), int(U), int(I), _p(top_ids), int(top_ids.shape[-1]), int(top_ids.shape[0]),
+              ka, len(ks), _p(rows), _s())
+
+
+def mmr_rerank(F, U, I, cand_ids, cand_scores, K, lam, out_ids, out_scores):
+    """MMR re-ranking of the candidate lists cand_ids (n, N) int32 / cand_scores (n, N) float32 (N <= 100) into K picks per row,
+    lam in [0, 1]: out_ids (n, K) int32 and out_scores (n, K) float32 (the picks' candidate scores, in pick order, -1 / 0.0 padded)"""
+    for t in (F, cand_ids, cand_scores, out_ids, out_scores):
+        _lib.require_cuda(t)
+    _lib.call("ngacf_mmr_rerank", _p(F), int(F.shape[-1]), int(U), int(I), _p(cand_ids), _p(cand_scores), int(cand_ids.shape[0]),
+              int(cand_ids.shape[-1]), int(K), float(lam), _p(out_ids), _p(out_scores), _s())
+
+
 NEG_TAG_TRAIN, NEG_TAG_EVAL = 0x4E54, 0x4E45
 
 

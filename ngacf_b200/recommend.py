@@ -6,7 +6,11 @@ items, order = score descending, then item id ascending (the reference's ranklis
 of the items' final features (the same tree for the dot products and the norms), candidates = item pool minus the query item, same
 order.  Audience lists rank users by the same score as the user lists (the same bits for each (user, item) pair), candidates = user
 pool minus the users the exclusion rule leaves out for that item; similar-user lists are the similar-item lists over the users'
-features.  K is 1 .. 100."""
+features.  K is 1 .. 100.
+
+Diversified user lists (diversified()) re-rank the top `candidates` of the user lists by maximal marginal relevance against the
+cosine of the items' final features (ngacf_mmr_rerank); list_diversity() scores any item lists by their intra-list diversity
+(ngacf_list_diversity).  Both are defined in ngacf_b200.cutoff_eval."""
 from __future__ import annotations
 
 import numpy as np
@@ -93,9 +97,9 @@ class Recommender:
             raise ValueError("K must be an integer in 1..%d, got %r" % (MAX_K, K))
         return int(K)
 
-    def _lists(self, q, K, n_cand, ws_bytes, rank):
+    def _rank(self, q, K, n_cand, ws_bytes, rank):
         """(n, K) outputs for the int32 queries q, a workspace of ws_bytes(width, n_cand, n, K) bytes and rank(q, K, ids, scores, ws)
-        -> (ids int64, scores float32)"""
+        -> (ids int32, scores float32)"""
         n = q.numel()
         dev = self.F.device
         ids = torch.empty((n, K), dtype=torch.int32, device=dev)
@@ -103,7 +107,24 @@ class Recommender:
         if n:
             ws = torch.empty(ws_bytes(self.F.shape[-1], n_cand, n, K), dtype=torch.uint8, device=dev)
             rank(q, K, ids, scores, ws)
+        return ids, scores
+
+    def _lists(self, q, K, n_cand, ws_bytes, rank):
+        """_rank with int64 ids"""
+        ids, scores = self._rank(q, K, n_cand, ws_bytes, rank)
         return ids.long(), scores
+
+    def _user_lists(self, users, K, novelty_weight):
+        """the user lists of __call__ for a checked K -> (ids int32 (n, K), scores float32 (n, K)); the weight is checked before any
+        feature is read"""
+        from .cutoff_eval import check_novelty_weight, novelty_offsets
+        w = check_novelty_weight(novelty_weight)
+        if w != 0.0 and self.inter is None:
+            raise ValueError("novelty_weight needs the interactions (inter=...): the item novelty comes from their train split")
+        off = novelty_offsets(self.inter, w) if w != 0.0 else None
+        u = self._ids(users, self.U, "user")
+        return self._rank(u, K, self.I, ops.recommend_topk_workspace_bytes, lambda q, K, ids, scores, ws: ops.recommend_topk(
+            self.F, self.U, self.I, q, K, self.excl_ptr, self.excl_items, self.in_pool, ids, scores, ws, off))
 
     def user_candidates(self):
         """-> (excl_ptr, excl_users, user_pool): the candidate inputs of ngacf_audience_topk / ngacf_similar_users_topk that audience()
@@ -131,15 +152,46 @@ class Recommender:
         novelty_weight w != 0: novelty-weighted lists, ranked (and scored) by s(u, i) + float32(w * nov(i)) with the item novelty of
         the train split of `inter` (ngacf_b200.cutoff_eval.novelty_offsets); a positive w moves popular items down.  w = 0 is the
         plain ranking."""
-        from .cutoff_eval import check_novelty_weight, novelty_offsets
+        ids, scores = self._user_lists(users, self._k(K), novelty_weight)
+        return ids.long(), scores
+
+    def diversified(self, users, K: int = 20, mmr_lambda=0.5, candidates: int = 100, novelty_weight=0.0):
+        """-> (ids int64 (n, K), scores float32 (n, K)) on the GPU: MMR-diversified lists.  Each user's top `candidates` (K..100) of
+        __call__(users, candidates, novelty_weight) (the same exclusion, pool and scores) are re-ranked greedily by mmr_lambda *
+        rel(c) - (1 - mmr_lambda) * (max cosine similarity to the items picked so far), rel being the score min-max normalised over
+        the candidates (ngacf_b200.cutoff_eval).  Rows hold the picks in pick order with their scores (so the scores are not
+        sorted), padded with id -1 / score 0.0.  mmr_lambda = 1 gives __call__(users, K, novelty_weight)."""
+        from .cutoff_eval import check_mmr_candidates, check_mmr_lambda
         K = self._k(K)
-        w = check_novelty_weight(novelty_weight)
-        if w != 0.0 and self.inter is None:
-            raise ValueError("novelty_weight needs the interactions (inter=...): the item novelty comes from their train split")
-        off = novelty_offsets(self.inter, w) if w != 0.0 else None
-        u = self._ids(users, self.U, "user")
-        return self._lists(u, K, self.I, ops.recommend_topk_workspace_bytes, lambda q, K, ids, scores, ws: ops.recommend_topk(
-            self.F, self.U, self.I, q, K, self.excl_ptr, self.excl_items, self.in_pool, ids, scores, ws, off))
+        lam = check_mmr_lambda(mmr_lambda)
+        N = check_mmr_candidates(candidates, K)
+        cand_ids, cand_scores = self._user_lists(users, N, novelty_weight)
+        n = cand_ids.shape[0]
+        ids = torch.empty((n, K), dtype=torch.int32, device=self.F.device)
+        scores = torch.empty((n, K), dtype=torch.float32, device=self.F.device)
+        if n:
+            ops.mmr_rerank(self.F, self.U, self.I, cand_ids, cand_scores, K, lam, ids, scores)
+        return ids.long(), scores
+
+    def list_diversity(self, ids, ks):
+        """ids: (n, L) item lists (L 1..100, integer ids; entries outside [0, I), such as -1 padding, are skipped), ks: cut-offs
+        (1..8 integers in 1..L) -> float64 (n, len(ks)) on the GPU: each row's intra-list diversity at each cut-off
+        (ngacf_b200.cutoff_eval) from the final features of the last refresh()"""
+        from .cutoff_eval import check_ks
+        ks = check_ks(ks)
+        t = ids if torch.is_tensor(ids) else torch.from_numpy(np.asarray(ids))
+        if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+            raise ValueError("item lists must hold integer ids, got %s" % t.dtype)
+        if t.dim() != 2 or not 1 <= t.shape[1] <= MAX_K:
+            raise ValueError("item lists must be (n, L) with L in 1..%d, got shape %s" % (MAX_K, tuple(t.shape)))
+        if ks[-1] > t.shape[1]:
+            raise ValueError("cut-off %d is longer than the lists (%d entries)" % (ks[-1], t.shape[1]))
+        lo, hi = np.iinfo(np.int32).min, np.iinfo(np.int32).max
+        t = t.to(device=self.F.device, dtype=torch.int64).clamp(lo, hi).to(torch.int32).contiguous()
+        rows = torch.zeros((t.shape[0], len(ks)), dtype=torch.float64, device=self.F.device)
+        if t.shape[0]:
+            ops.list_diversity(self.F, self.U, self.I, t, ks, rows)
+        return rows
 
     def similar_items(self, items, K: int = 20):
         """-> (ids int64 (n, K), scores float32 (n, K)) on the GPU: for each query item the K items of highest cosine similarity of the

@@ -24,6 +24,11 @@ items), written to ..._similarusers{K}.tsv as `user<TAB>rank<TAB>similar_user<TA
 With --novelty-weight w (user lists only) the user lists rank by score + float32(w * novelty(item)), the item novelty of the train
 split (Recommender(..., novelty_weight=w)); a positive w moves popular items down.  The scores written are those offset scores and
 the default output name gains _nw{w}, e.g. recs/SPUIGACF_ml100k_010_top50_nw1.0.tsv.
+
+With --mmr-lambda lam (user lists only, lam in [0, 1]) the user lists are diversified: the top --mmr-candidates N (default 100,
+--topk..100) of each user are re-ranked by maximal marginal relevance against the cosine of the items' final features
+(Recommender.diversified).  The lines keep the format, in pick order with each item's own score (so the scores are not sorted), and
+the default output name gains _mmr{lam}, e.g. recs/SPUIGACF_ml100k_010_top20_mmr0.5.tsv.
 """
 import os
 import sys
@@ -33,7 +38,7 @@ import numpy as np
 import torch
 
 import run_Gowalla as R
-from ngacf_b200.cutoff_eval import check_novelty_weight
+from ngacf_b200.cutoff_eval import check_mmr_candidates, check_mmr_lambda, check_novelty_weight
 from ngacf_b200.recommend import EXCLUDE, MAX_K, Recommender
 
 
@@ -52,6 +57,10 @@ def build_parser():
                    help="rank users like these users: all, a comma-separated id list, or @FILE")
     p.add_argument("--novelty-weight", type=float, default=0.0,
                    help="w: rank the user lists by score + w * novelty(item) (a positive w moves popular items down); 0 is the plain ranking")
+    p.add_argument("--mmr-lambda", type=float, default=None,
+                   help="lam in [0, 1]: diversify the user lists by maximal marginal relevance (1 keeps the ranking, 0 the least similar items)")
+    p.add_argument("--mmr-candidates", type=int, default=None,
+                   help="N in --topk..100: the candidates --mmr-lambda re-ranks per user (default 100)")
     p.add_argument("--out", type=str, default=None,
                    help="output TSV (default recs/{model}_{dataset}_{N:03d}_top{K}.tsv, with --similar-items ..._similar{K}.tsv, "
                         "--audience ..._audience{K}.tsv, --similar-users ..._similarusers{K}.tsv)")
@@ -82,6 +91,7 @@ def parse_ids(spec, flag="--users", words=("eval", "all")):
 def default_out(args):
     kind = next((tag for dest, _, tag in QUERY_FLAGS if getattr(args, dest) is not None), "top")
     nw = "_nw{}".format(args.novelty_weight) if args.novelty_weight != 0.0 else ""
+    nw += "_mmr{}".format(args.mmr_lambda) if args.mmr_lambda is not None else ""
     return os.path.join("recs", "{}_{}_{:03d}_{}{}{}.tsv".format(args.model, args.dataset, args.resume_from, kind, args.topk, nw))
 
 
@@ -105,6 +115,16 @@ def parse_args(argv=None):
     args.novelty_weight = check_novelty_weight(args.novelty_weight)
     if given and args.novelty_weight != 0.0:
         raise ValueError("--novelty-weight applies to the user lists only; drop it with %s" % given[0])
+    if args.mmr_lambda is not None:
+        if given:
+            raise ValueError("--mmr-lambda applies to the user lists only; drop it with %s" % given[0])
+        try:
+            args.mmr_lambda = check_mmr_lambda(args.mmr_lambda)
+            args.mmr_candidates = check_mmr_candidates(100 if args.mmr_candidates is None else args.mmr_candidates, args.topk)
+        except ValueError as e:
+            raise ValueError("--mmr-lambda / --mmr-candidates: %s" % e) from None
+    elif args.mmr_candidates is not None:
+        raise ValueError("--mmr-candidates sets the candidates of --mmr-lambda; give --mmr-lambda as well")
     args.item_ids = args.audience_ids = args.similar_user_ids = None
     if args.audience is not None:
         if args.users != "eval":
@@ -190,12 +210,16 @@ def main(args):
     rec = Recommender(load_model(args, userNum, itemNum), adj, inter, args.exclude)
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    ids, scores = rec(users, args.topk, novelty_weight=args.novelty_weight)
+    if args.mmr_lambda is None:
+        ids, scores = rec(users, args.topk, novelty_weight=args.novelty_weight)
+    else:
+        ids, scores = rec.diversified(users, args.topk, args.mmr_lambda, args.mmr_candidates, novelty_weight=args.novelty_weight)
     torch.cuda.synchronize()
     ms = (time.perf_counter() - t0) * 1e3
     ids, scores = ids.cpu().numpy(), scores.cpu().numpy()
     write_tsv(args.out, users, ids, scores)
     nw = ", novelty weight %r" % args.novelty_weight if args.novelty_weight != 0.0 else ""
+    nw += ", mmr lambda %r of %d candidates" % (args.mmr_lambda, args.mmr_candidates) if args.mmr_lambda is not None else ""
     print("recommend: %d users, top-%d%s, %.2f ms -> %s" % (users.size, args.topk, nw, ms, args.out))
     return users, ids, scores
 

@@ -21,7 +21,8 @@ from graphattention.BPRLoss import BPRLoss
 from graphattention.SPUIGACF import SPUIGACF, SPUIMultiGACF
 from ngacf_b200.data import Interactions
 from ngacf_b200.hostdata import load_dataset
-from train_eval_Gowalla import eval_full_ranking, eval_neg_all, eval_neg_sample, list_reports, train_bpr, train_neg_sample
+from train_eval_Gowalla import (diversity_report, eval_full_ranking, eval_neg_all, eval_neg_sample, list_reports, train_bpr,
+                                train_neg_sample)
 
 
 def prepareData(args):
@@ -116,28 +117,43 @@ def main(args):
 def full_ranking(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0):
     """--eval_ks: full-ranking metrics with the standard definitions (ngacf_b200.cutoff_eval), printed by rank 0 as one line of plain
     Python values and logged as full@K/<metric>; then the same lines for the lists of each --eval_novelty_weights weight w, printed
-    as `epoch:{e} novelty weight {w} ...` and logged under novelty{w}/"""
+    as `epoch:{e} novelty weight {w} ...` and logged under novelty{w}/; then those of each --eval_mmr_lambdas lambda's
+    MMR-diversified lists, printed as `epoch:{e} mmr lambda {lam} ...` and logged under mmr{lam}/"""
     if not args.eval_ks:
         return
     rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, 0.0)
     for w in args.eval_novelty_weights or ():
         rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, w)
+    for lam in args.eval_mmr_lambdas or ():
+        rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, 0.0, lam)
 
 
-def rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, w):
-    """full_ranking's lines for the lists of novelty weight w (0: the plain lists)"""
-    line = "epoch:{} ".format(epoch) if w == 0.0 else "epoch:{} novelty weight {} ".format(epoch, w)
-    tag = "" if w == 0.0 else "novelty{}/".format(w)
-    res = eval_full_ranking(model, test_df, test_pos_neg, adj, args.eval_ks, args.parallel, novelty_weight=w)
+def rank_report(args, model, test_df, test_pos_neg, adj, epoch, summaryWriter, rank0, w, lam=None):
+    """full_ranking's lines for the lists of novelty weight w (0: the plain lists), or of MMR lambda lam (None: no re-ranking)"""
+    if lam is not None:
+        line, tag = "epoch:{} mmr lambda {} ".format(epoch, lam), "mmr{}/".format(lam)
+    else:
+        line = "epoch:{} ".format(epoch) if w == 0.0 else "epoch:{} novelty weight {} ".format(epoch, w)
+        tag = "" if w == 0.0 else "novelty{}/".format(w)
+    res = eval_full_ranking(model, test_df, test_pos_neg, adj, args.eval_ks, args.parallel, novelty_weight=w, mmr_lambda=lam)
     for i, K in enumerate(res["ks"]):
         for name in ("precision", "recall", "ndcg", "hit_ratio", "mrr"):
             summaryWriter.add_scalar("{}full@{}/{}".format(tag, K, name), res[name][i], epoch)
     if rank0:
         print("{}full-ranking metrics:{}".format(line, _plain(res)))
-    if not (args.eval_beyond or args.eval_groups):
-        return
-    # --eval_beyond / --eval_groups: reports over the lists eval_full_ranking just ranked (every rank takes part in the all-reduce)
-    rep = list_reports(model, args.eval_beyond, args.eval_groups, novelty_weight=w)
+    if args.eval_beyond or args.eval_groups:
+        list_lines(args, model, epoch, summaryWriter, rank0, w, lam, line, tag)
+    if args.eval_diversity:
+        d = diversity_report(model, novelty_weight=w, mmr_lambda=lam)
+        for i, K in enumerate(d["ks"]):
+            summaryWriter.add_scalar("{}diversity@{}/ild".format(tag, K), d["ild"][i], epoch)
+        if rank0:
+            print("{}diversity metrics:{}".format(line, _plain(d)))
+
+
+def list_lines(args, model, epoch, summaryWriter, rank0, w, lam, line, tag):
+    """--eval_beyond / --eval_groups: reports over the lists eval_full_ranking just ranked (every rank takes part in the all-reduce)"""
+    rep = list_reports(model, args.eval_beyond, args.eval_groups, novelty_weight=w, mmr_lambda=lam)
     if rep["beyond"] is not None:
         b = rep["beyond"]
         for i, K in enumerate(b["ks"]):
@@ -171,6 +187,24 @@ def parse_novelty_weights(text):
 
 
 MAX_NOVELTY_WEIGHTS = 8
+
+
+def parse_mmr_lambdas(text):
+    """'0.5,0.8' -> [0.5, 0.8]; ValueError unless it is 1..8 distinct numbers in [0, 1)"""
+    try:
+        ls = [float(x) for x in str(text).split(",")]
+    except ValueError:
+        raise ValueError("--eval_mmr_lambdas must be a comma-separated list of numbers, got %r" % text) from None
+    if not 1 <= len(ls) <= MAX_MMR_LAMBDAS:
+        raise ValueError("--eval_mmr_lambdas takes 1..%d values, got %d" % (MAX_MMR_LAMBDAS, len(ls)))
+    if not all(0.0 <= x < 1.0 for x in ls):
+        raise ValueError("--eval_mmr_lambdas must lie in [0, 1) (1 gives the plain lists, which are reported anyway), got %r" % text)
+    if len(set(ls)) != len(ls):
+        raise ValueError("--eval_mmr_lambdas must be distinct, got %r" % text)
+    return ls
+
+
+MAX_MMR_LAMBDAS = 8
 
 
 def _plain(res):
@@ -212,7 +246,27 @@ def build_parser():
     p.add_argument("--eval_novelty_weights", type=str, default=None,
                    help="e.g. 0.5,1,2 (1..8 distinct non-zero numbers): also rank novelty-weighted lists, by score + w * novelty(item), "
                         "and report the --eval_ks metrics (and --eval_beyond / --eval_groups) of each weight's lists")
+    p.add_argument("--eval_diversity", type=str, default=False,
+                   help="True: also report the intra-list diversity (mean pairwise cosine distance of the items' final features) of the "
+                        "ranked lists at the --eval_ks cut-offs")
+    p.add_argument("--eval_mmr_lambdas", type=str, default=None,
+                   help="e.g. 0.5,0.8 (1..8 distinct values in [0, 1)): also re-rank the top 100 of each list by maximal marginal "
+                        "relevance with these lambdas and report the --eval_ks metrics (and --eval_beyond / --eval_groups / "
+                        "--eval_diversity) of each lambda's lists")
     return p
+
+
+def parse_bool(value, flag):
+    """'True' / 'False' (or a bool) -> the bool; ValueError for anything else"""
+    v = value
+    if isinstance(v, str):
+        try:
+            v = ast.literal_eval(v)
+        except (ValueError, SyntaxError):
+            v = None
+    if not isinstance(v, bool):
+        raise ValueError("%s must be True or False, got %r" % (flag, value))
+    return v
 
 
 def parse_args(argv=None):
@@ -226,15 +280,8 @@ def parse_args(argv=None):
     if args.eval_ks is not None:
         from ngacf_b200.cutoff_eval import parse_ks
         args.eval_ks = parse_ks(args.eval_ks)
-    beyond = args.eval_beyond
-    if isinstance(beyond, str):
-        try:
-            beyond = ast.literal_eval(beyond)
-        except (ValueError, SyntaxError):
-            beyond = None
-    if not isinstance(beyond, bool):
-        raise ValueError("--eval_beyond must be True or False, got %r" % args.eval_beyond)
-    args.eval_beyond = beyond
+    args.eval_beyond = parse_bool(args.eval_beyond, "--eval_beyond")
+    args.eval_diversity = parse_bool(args.eval_diversity, "--eval_diversity")
     if args.eval_groups is not None:
         from ngacf_b200.cutoff_eval import check_groups
         try:
@@ -248,6 +295,12 @@ def parse_args(argv=None):
         args.eval_novelty_weights = parse_novelty_weights(args.eval_novelty_weights)
         if not args.eval_ks:
             raise ValueError("--eval_novelty_weights reports at the --eval_ks cut-offs; give --eval_ks as well")
+    if args.eval_diversity and not args.eval_ks:
+        raise ValueError("--eval_diversity reports at the --eval_ks cut-offs; give --eval_ks as well")
+    if args.eval_mmr_lambdas is not None:
+        args.eval_mmr_lambdas = parse_mmr_lambdas(args.eval_mmr_lambdas)
+        if not args.eval_ks:
+            raise ValueError("--eval_mmr_lambdas reports at the --eval_ks cut-offs; give --eval_ks as well")
     if args.parallel and args.embedSize != 64:
         raise ValueError("--parallel True is built for --embedSize 64 only; train --embedSize %d on one GPU (--parallel False)" % args.embedSize)
     return args

@@ -200,23 +200,25 @@ def eval_neg_all(model, batch_size, test_df, test_pos_neg, adj, itemNum, is_para
         return ev(Z)
 
 
-def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="auto", novelty_weight=0.0):
+def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="auto", novelty_weight=0.0, mmr_lambda=None):
     """Full-ranking metrics at the cut-offs `ks` (up to 8 of 1..100) with the standard definitions: precision, recall, NDCG with the
     ideal DCG of min(|test|, k) hits, hit ratio and MRR, averaged over the users with train and test items
     (ngacf_b200.cutoff_eval).  Returns FullRankingEvaluator.metrics()'s dict.  is_parallel under torchrun: the users are sharded over
     the ranks and the sums merged, as in eval_neg_all.  novelty_weight w != 0: the metrics of the novelty-weighted lists
-    (FullRankingEvaluator(novelty_weight=w)), from an evaluator cached per weight next to the plain one."""
-    from ngacf_b200.cutoff_eval import FullRankingEvaluator, check_ks, check_novelty_weight
+    (FullRankingEvaluator(novelty_weight=w)), from an evaluator cached per weight next to the plain one.  mmr_lambda lam: the metrics
+    of the MMR-diversified lists (FullRankingEvaluator(mmr_lambda=lam)), from an evaluator cached per (weight, lam)."""
+    from ngacf_b200.cutoff_eval import FullRankingEvaluator, check_ks, check_mmr_lambda, check_novelty_weight
     m = _unwrap(model)
     model.eval()
     _require_plain(m, "eval_full_ranking")
     ks = check_ks(ks)
     w = check_novelty_weight(novelty_weight)
+    lam = None if mmr_lambda is None else check_mmr_lambda(mmr_lambda)
     inter = _interactions(model, None, test_pos_neg, test_df)
     adj_t = _device_adj(model, adj)
     with torch.no_grad():
         Z = m.propagate(adj_t)
-        ev = _full_evaluator(m, w)
+        ev = _full_evaluator(m, w, lam)
         world = _world() if is_parallel else 1
         if ev is None or ev.inter is not inter or ev.mode != mode or ev.ks != ks or getattr(ev, "world", 1) != world:
             users = None
@@ -224,33 +226,52 @@ def eval_full_ranking(model, test_df, test_pos_neg, adj, ks, is_parallel, mode="
                 import torch.distributed as dist
                 from ngacf_b200.dist import shard_eval_users
                 users = shard_eval_users(inter.eval_users, dist.get_rank(), world)
-            ev = FullRankingEvaluator(inter, ks, mode, users=users, novelty_weight=w)
+            ev = FullRankingEvaluator(inter, ks, mode, users=users, novelty_weight=w, mmr_lambda=lam)
             ev.world = world
-            if w == 0.0:
+            if lam is not None:
+                m.__dict__.setdefault("_mmr_evaluators", {})[(w, lam)] = ev
+            elif w == 0.0:
                 m._full_evaluator = ev
             else:
                 m.__dict__.setdefault("_novelty_evaluators", {})[w] = ev
         return ev(Z)
 
 
-def _full_evaluator(m, w):
-    """the evaluator eval_full_ranking cached for novelty weight w (0: the plain one), or None"""
+def _full_evaluator(m, w, lam=None):
+    """the evaluator eval_full_ranking cached for novelty weight w (0: the plain one) and MMR lambda lam (None: no re-ranking), or
+    None"""
+    if lam is not None:
+        return m.__dict__.get("_mmr_evaluators", {}).get((w, lam))
     if w == 0.0:
         return getattr(m, "_full_evaluator", None)
     return m.__dict__.get("_novelty_evaluators", {}).get(w)
 
 
-def list_reports(model, beyond=True, groups=None, novelty_weight=0.0):
+def _cached_evaluator(model, novelty_weight, mmr_lambda, what):
+    from ngacf_b200.cutoff_eval import check_mmr_lambda, check_novelty_weight
+    lam = None if mmr_lambda is None else check_mmr_lambda(mmr_lambda)
+    ev = _full_evaluator(_unwrap(model), check_novelty_weight(novelty_weight), lam)
+    if ev is None or ev.source is None:
+        raise RuntimeError("%s: call eval_full_ranking first (with the same novelty_weight and mmr_lambda); it ranks the lists these "
+                           "reports read" % what)
+    return ev
+
+
+def diversity_report(model, novelty_weight=0.0, mmr_lambda=None):
+    """The intra-list diversity (FullRankingEvaluator.diversity_metrics()) of the lists the preceding eval_full_ranking call with the
+    same novelty_weight and mmr_lambda ranked, from the evaluator it cached: no second propagation or ranking.  Under torchrun every
+    rank calls it (the sums are all-reduced)."""
+    return _cached_evaluator(model, novelty_weight, mmr_lambda, "diversity_report").diversity_metrics()
+
+
+def list_reports(model, beyond=True, groups=None, novelty_weight=0.0, mmr_lambda=None):
     """The beyond-accuracy metrics (coverage, Gini of the item exposure, novelty, ARP) and the metrics per user-activity group
     (NGCF section 4.3.2) of the lists the preceding eval_full_ranking call ranked, from the evaluator it cached: no second
     propagation or ranking.  Returns {"beyond": FullRankingEvaluator.list_metrics() or None, "groups":
     FullRankingEvaluator.group_metrics(groups) or None}.  novelty_weight: read the lists of the eval_full_ranking call with that
-    weight.  Under torchrun every rank calls it (the counts and sums are all-reduced)."""
-    from ngacf_b200.cutoff_eval import check_novelty_weight
-    ev = _full_evaluator(_unwrap(model), check_novelty_weight(novelty_weight))
-    if ev is None or ev.source is None:
-        raise RuntimeError("list_reports: call eval_full_ranking first (with the same novelty_weight); it ranks the lists these "
-                           "reports read")
+    weight (and mmr_lambda: of the MMR-diversified lists).  Under torchrun every rank calls it (the counts and sums are
+    all-reduced)."""
+    ev = _cached_evaluator(model, novelty_weight, mmr_lambda, "list_reports")
     return {"beyond": ev.list_metrics() if beyond else None, "groups": ev.group_metrics(groups) if groups else None}
 
 
